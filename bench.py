@@ -2,6 +2,7 @@
 """Benchmark of the sampling hot path (BASELINE.json metric: leapfrog grad-evals/sec, min-ESS/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c2|c1|c5] [--scaling strong|weak] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json's Target configuration (configs[3], "C4"): Bayesian linear regression with 1000
 coefficients and 100,000 observations, NUTS, 4096 chains in lock-step (it fits one GPU: X is 400 MB).  With N GPUs the
@@ -250,7 +251,7 @@ def reference_arm(args, wl, config):
     cores = os.cpu_count() or 1
     if wl["kind"] == "pointwise":
         cores = min(cores, 32)
-    W_, K = max(args.warmup, 0), max(args.steps, 1)
+    W_, K = max(args.warmup, 0), args.steps
     # a step sized so that K of them end within a few minutes: C4 ~ 1 s (2 transitions), C3 / pointwise ~ 2-4 s
     scale = 0.2 if args.workload == "c4" else 0.3
     for _ in range(min(W_, 2)):
@@ -259,8 +260,6 @@ def reference_arm(args, wl, config):
     for _ in range(K):
         per = cpu_baseline(args.workload, cores, scale)
         vals.append(per["value"])
-        if time.perf_counter() - t0 > 240:      # safety only: never reached at the driver's K
-            break
     v = float(np.mean(vals))
     per["value"] = v
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": len(vals),
@@ -330,6 +329,31 @@ class Timed:
 
     def total_ms(self):
         return float(sum(a.elapsed_time(b) for a, b in self.ev))
+
+
+DUMP_BYTES = 48 << 20      # C4's draws are 131 MB a step: about 1500 of its 4096 chains fit
+
+
+def dump_outputs(out_dir, draws, depths=None):
+    """--dump-outputs: what the last timed step returned, as float32 .npy files -- the draws [iters, chains, D] of a
+    fixed sample of chains (numpy default_rng(0), as many as keep the whole dump within DUMP_BYTES; all of them when
+    they fit) and the NUTS tree depth [iters, chains] of every chain.  The inputs of a run depend only on the command
+    line, so two builds of the project can be compared file for file."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    if depths is not None:
+        out["tree_depth"] = depths.float().cpu().numpy()
+    iters, C, D = draws.shape
+    left = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 4096
+    keep = min(C, left // (4 * iters * D))
+    if keep < C:
+        import torch
+        idx = np.sort(np.random.default_rng(0).choice(C, keep, replace=False))
+        draws = draws.index_select(1, torch.from_numpy(idx).to(draws.device))
+    out["draws"] = draws.float().cpu().numpy()
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"outputs of the last timed step in {out_dir}: " + ", ".join(f"{k}{list(a.shape)}" for k, a in out.items()))
 
 
 # ----------------------------------------------------------------------------------------- GLM workloads (c4, c3)
@@ -462,6 +486,8 @@ def bench_glm(torch, dist, B, lib, args, wl, wl_name, rank, world, local_rank, f
     barrier()
     timed.run(one_step)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, draws, depths)
     lib.b2m_profile_read_ex(ten)
     lib.b2m_profile(0)
     four = list(ten)[:4]
@@ -627,6 +653,8 @@ def bench_glm_strong(torch, dist, B, lib, args, wl, wl_name, rank, world, local_
     barrier()
     timed.run(lambda: step(SLICE))
     barrier()
+    if args.dump_outputs and rank == 0:     # rank 0 advances (and writes the draws of) the first C / N chains
+        dump_outputs(args.dump_outputs, draws[:, :C // world], depths[:, :C // world])
     lib.b2m_profile_read_ex(ten)
     lib.b2m_profile(0)
     four = list(ten)[:4]
@@ -798,6 +826,8 @@ def bench_pointwise(torch, dist, B, lib, args, wl, wl_name, rank, world, local_r
     barrier()
     timed.run(one_step)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, draws)
     launches = lib.b2m_launch_count() - n0
     total_ms = timed.total_ms()
 
@@ -959,7 +989,14 @@ def main():
     ap.add_argument("--no-ess", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip the short runs of the other configurations")
     ap.add_argument("--no-jit", action="store_true", help="pointwise workloads: keep the generic interpreter kernels")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the draws (and NUTS tree depths) of the last timed step to DIR/<name>.npy, float32, "
+                         "at most 48 MiB in all (a fixed sample of the chains when the draws are larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the device path computed; the reference arm keeps no outputs")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -1016,7 +1053,7 @@ def main():
         if world == 1 and not args.no_others:
             others = {}
             small = argparse.Namespace(**vars(args))
-            small.steps, small.warmup, small.chains, small.no_ess = 5, 3, 0, True
+            small.steps, small.warmup, small.chains, small.no_ess, small.dump_outputs = 5, 3, 0, True, None
             for name in ("c3", "c2", "c1", "c5"):
                 if name == args.workload:
                     continue

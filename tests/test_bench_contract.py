@@ -1,9 +1,11 @@
 """CPU: the shape of bench.py's one JSON line -- the reference arm run for real on a small workload, and the last
-committed device line under profiles/ (the device arm itself needs a GPU)."""
+committed device line under profiles/ (the device arm itself needs a GPU) -- and its --dump-outputs files."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -93,3 +95,43 @@ def test_strong_scaling_is_refused_for_pointwise_workloads():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c2", "--scaling", "strong", "--impl", "reference"],
                          capture_output=True, text=True, timeout=120, env=dict(os.environ, PYTHONPATH=ROOT), cwd=ROOT)
     assert out.returncode != 0 and "observation sharding" in (out.stderr + out.stdout)
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_chains_within_the_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    draws = torch.arange(4 * 4096 * 32, dtype=torch.float32).reshape(4, 4096, 32)         # 2 MB: twice the budget
+    depths = torch.randint(0, 10, (4, 4096), dtype=torch.int32, generator=torch.Generator().manual_seed(0))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), draws, depths)
+    a = {f: np.load(tmp_path / "a" / f"{f}.npy") for f in ("draws", "tree_depth")}
+    assert sum(os.path.getsize(tmp_path / "a" / f"{f}.npy") for f in a) <= 1 << 20
+    assert a["draws"].dtype == a["tree_depth"].dtype == np.float32
+    assert np.array_equal(a["tree_depth"], depths.numpy())
+    kept = a["draws"][0, :, 0].astype(np.int64) // 32                                      # chain index of each kept row
+    assert 1000 < len(kept) < 4096 and np.all(np.diff(kept) > 0)
+    assert np.array_equal(a["draws"], draws.numpy()[:, kept])
+    for f, v in a.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f"{f}.npy"), v)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_identical_for_identical_arguments(cuda, tmp_path):
+    """--dump-outputs on a small regression run, twice: the timed path starts from the same inputs every time, so the
+    draws and tree depths of the last timed step agree bit for bit; --steps is the number of timed steps."""
+    import numpy as np
+    dumps = []
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c3", "--chains", "256",
+                              "--steps", "2", "--warmup", "0", "--no-others", "--no-cpu-baseline", "--no-ess",
+                              "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-3000:]
+        assert json.loads(out.stdout)["steps"] == 2
+        dumps.append({f: np.load(tmp_path / d / f"{f}.npy") for f in ("draws", "tree_depth")})
+    a, b = dumps
+    assert a["draws"].shape == (16, 256, 100) and a["tree_depth"].shape == (16, 256)
+    assert np.isfinite(a["draws"]).all()
+    for f in a:
+        assert np.array_equal(a[f], b[f]), f

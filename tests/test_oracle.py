@@ -1,5 +1,6 @@
 """CPU: the oracle restatement against the golden vectors produced from the unmodified reference
 (oracle/make_golden.py), plus the reference's own known-answer log_prob tests run on the oracle."""
+import json
 import math
 import os
 
@@ -42,19 +43,26 @@ def test_survey_golden_values():
 
 @pytest.mark.parametrize("name", RUN_FIXTURES)
 def test_port_reproduces_reference_draws(name):
-    """Same stand-in keys => the restatement's draws equal the reference's, bit for bit."""
+    """Same stand-in keys => the restatement's draws equal the reference's, bit for bit, and it ends on the committed
+    step size having consumed the committed random numbers (the slots the GPU parity tests inject)."""
     g = golden(name)
     fn, init, _ = W.ALL_SMALL[g["model"]](ns)
     kw = dict(g["kwargs"])
+    tape, eps = Tape(), None
     if g["method"] == "hmc":
-        s, a, _ = samplers.hmc_port(fn, init, key=mx.random.key(g["seed"]), **kw)
+        s, a, eps = samplers.hmc_port(fn, init, key=mx.random.key(g["seed"]), tape=tape, **kw)
     elif g["method"] == "nuts":
-        s, a, _ = samplers.nuts_port(fn, init, key=mx.random.key(g["seed"]), **kw)
+        s, a, eps = samplers.nuts_port(fn, init, key=mx.random.key(g["seed"]), tape=tape, **kw)
     else:
-        s, a = samplers.run_port(fn, init, method="metropolis", random_seed=g["seed"], **kw)
+        s, a = samplers.run_port(fn, init, method="metropolis", random_seed=g["seed"], tape=tape, **kw)
     assert a == g["accept_rate"]
     for k, v in g["draws"].items():
         assert np.array_equal(np.asarray(s[k], dtype=np.float32), np.asarray(v, dtype=np.float32))
+    assert json.loads(json.dumps(eps)) == g["final_step_size"]
+    normals = [{"it": k[0], "param": k[1], "z": np.asarray(v, dtype=np.float64).tolist()} for k, v in tape.normals.items()]
+    uniforms = [{"slot": list(k), "u": float(v)} for k, v in tape.uniforms.items()]
+    assert json.loads(json.dumps(normals)) == g["tape"]["normals"]
+    assert json.loads(json.dumps(uniforms)) == g["tape"]["uniforms"]
 
 
 # --- the reference's known-answer tests (tests/test_distributions.py, tests/test_new_distributions.py) ---
@@ -98,8 +106,8 @@ def test_diagnostics_restatement_matches_reference_fixture():
         assert abs(compute_ess(x) - row["ess06"]) <= 1e-4 * abs(row["ess06"])
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get("B2M_REFERENCE", "/root/reference")),
-                    reason="the upstream source tree is only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.environ.get("B2M_REFERENCE", "")),
+                    reason="set B2M_REFERENCE to a checkout of the upstream korentomas/mlx-mcmc source to run it")
 def test_committed_fixtures_reproduce_from_the_unmodified_reference():
     """The pin itself, re-checked where the reference is at hand: oracle/make_golden.py --check runs the UNMODIFIED
     reference samplers on the mlx.core stand-in and compares draws, acceptance rate and consumed random numbers with
