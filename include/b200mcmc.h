@@ -38,7 +38,7 @@ typedef unsigned long long uintptr_t;
 extern "C" {
 #endif
 
-#define B2M_ABI_VERSION 2
+#define B2M_ABI_VERSION 3
 #define B2M_MAX_TREE_DEPTH 12
 
 /* ---- model description (produced by the Python tracer from the user's log_prob) ---- */
@@ -337,13 +337,6 @@ int b2m_profile_read(double *out4);
 /* the same plus the per-chain kernels of the fused NUTS loop: {total ms, launches} x {K5, K6, state kernel, peer wait kernel
  * (includes waiting for the slowest rank's rows), peer signal kernel} */
 int b2m_profile_read_ex(double *out10);
-
-/* Experiments and tests only (no reference counterpart): set one launch-shape knob of the GLM contractions for this process,
- * e.g. ("fuse", 0) = the separate K5 / K6 launches (default), ("fuse", 1) = the concurrent K5 || K6 launch for large
- * problems, ("fuse", 2) = whenever the shape allows, ("fuse_slab", t), ("fuse_ring", r), ("l2_hints", 0|1), ("k6_order", 0|1:
- * pair row / column tile fastest in K6's persistent tile loop).  The same knobs are read once from B2M_TC_* environment
- * variables at load.  Returns non-zero for an unknown name.  Results never depend on a knob beyond float32 rounding. */
-int b2m_tuning_set(const char *name, int32_t value);
 
 /* number of kernel launches this library has issued since load (bench.py's gpu_launches) */
 int64_t b2m_launch_count(void);

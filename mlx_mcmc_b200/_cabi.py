@@ -74,14 +74,14 @@ GLM_AUTO, GLM_SIMT, GLM_TC, GLM_TC16 = 0, 1, 2, 3
 GLM_PATHS = {"auto": GLM_AUTO, "simt": GLM_SIMT, "tc": GLM_TC, "tc16": GLM_TC16}
 POINTWISE_AUTO, POINTWISE_GENERAL = 0, 1
 MAX_TREE_DEPTH = 12
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 EXPORTS = ["b2m_last_error", "b2m_abi_version", "b2m_struct_sizes", "b2m_model_create", "b2m_model_destroy",
            "b2m_model_dim", "b2m_model_class", "b2m_model_glm_path", "b2m_logp_grad", "b2m_hmc_run", "b2m_mh_run", "b2m_nuts_run",
            "b2m_launch_count", "b2m_comm_unique_id", "b2m_comm_init", "b2m_comm_destroy", "b2m_model_set_comm",
            "b2m_comm_allreduce_f32", "b2m_profile", "b2m_profile_read", "b2m_diag_series", "b2m_diag_params", "b2m_sample",
            "b2m_options_size", "b2m_peer_alloc", "b2m_peer_open", "b2m_peer_close", "b2m_peer_free", "b2m_model_peer_bytes",
-           "b2m_model_peer_attach", "b2m_mass_from_draws", "b2m_quantiles", "b2m_model_attach_module", "b2m_model_has_module", "b2m_profile_read_ex", "b2m_tuning_set"]
+           "b2m_model_peer_attach", "b2m_mass_from_draws", "b2m_quantiles", "b2m_model_attach_module", "b2m_model_has_module", "b2m_profile_read_ex"]
 
 _lib = None
 
@@ -147,7 +147,6 @@ def load(build_if_missing: bool = True):
     lib.b2m_profile.argtypes = [C.c_int32]
     lib.b2m_profile_read.argtypes = [C.POINTER(C.c_double)]
     lib.b2m_profile_read_ex.argtypes = [C.POINTER(C.c_double)]
-    lib.b2m_tuning_set.argtypes = [C.c_char_p, C.c_int32]
     lib.b2m_comm_unique_id.argtypes = [c_p]
     lib.b2m_comm_init.argtypes = [c_p, C.c_int32, C.c_int32, C.POINTER(c_p)]
     lib.b2m_comm_destroy.argtypes = [c_p]

@@ -208,8 +208,6 @@ int b2m_profile_read_ex(double *out10) {
   return b2m::tc_profile_read_n(out10, 5);
 }
 
-int b2m_tuning_set(const char *name, int32_t value) { return b2m::tuning_set(name, (int)value); }
-
 int b2m_struct_sizes(int32_t *out6) {
   out6[0] = (int32_t)sizeof(b2m_term);
   out6[1] = (int32_t)sizeof(b2m_operand);

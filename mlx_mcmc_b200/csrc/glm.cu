@@ -38,11 +38,6 @@ void glm_free(GlmModel &g) {
   g.h_flag = nullptr;
   if (g.h_prog) cudaFreeHost(const_cast<long long *>(g.h_prog));
   g.h_prog = nullptr;
-  if (g.fz_sync) cudaFree(g.fz_sync);
-  g.fz_sync = nullptr;
-  g.fz_sync_cap = 0;
-  if (g.h_fz_err) cudaFreeHost(const_cast<int *>(g.h_fz_err));
-  g.h_fz_err = nullptr;
 }
 
 int glm_reserve(GlmModel &g, int64_t n_chains) {
@@ -551,9 +546,8 @@ int glm_logp_grad(GlmModel &g, const float *theta, int64_t C, float *logp, float
   }
   ++g_launches;
   if (g.use_tc) {
-    if (grad) {
-      if (int rc = tc_gemm_resid_grad(g, Cp, st)) return rc;
-    } else if (int rc = tc_gemm_resid(g, Cp, st)) return rc;
+    if (int rc = tc_gemm_resid(g, Cp, st)) return rc;
+    if (grad) if (int rc = tc_gemm_grad(g, Cp, st)) return rc;
   } else {
     if (int rc = simt_gemm_resid(g, Cp, st)) return rc;
     if (grad) if (int rc = simt_gemm_grad(g, Cp, st)) return rc;

@@ -106,28 +106,7 @@ struct GlmModel {
   bool push_on = false;
   unsigned *blk_counter = nullptr;                           // device: "last block" counters of the signalling kernels
   volatile long long *h_prog = nullptr;                      // pinned + mapped: {ticks completed, finished chains} written by the device
-  // concurrent K5 || K6 launch (glm_tc.cu, tc_gemm_resid_grad): dependency counters [ready | turn] in device memory, zeroed
-  // before every launch, and a pinned + mapped flag a timed-out dependency wait raises (the next call then fails)
-  int *fz_sync = nullptr;
-  size_t fz_sync_cap = 0;
-  volatile int *h_fz_err = nullptr;
 };
-
-// knobs for experiments, read ONCE per process from the environment (never on the launch path):
-//   B2M_TC_GROUPS_RESID / B2M_TC_GROUPS_GRAD  persistent CTA groups, B2M_TC_CHUNK_RESID / B2M_TC_CHUNK_GRAD promotion
-//   interval in k-blocks, B2M_TC_PAIR=0 single-CTA kernels, B2M_TC_L2_HINTS=1 L2 eviction-policy hints on the TMA loads of
-//   the separate kernels (measured: no gain, off by default)
-//   B2M_TC_K6_ORDER=0 K6 tiles with the pair row fastest (round-1 order) instead of the column tile
-//   B2M_TC_FUSE=0 (default) separate K5 / K6 launches; 1 the concurrent launch for large fp16-encoded problems (a fifth
-//   of the DRAM traffic, ~10-20 % slower: DESIGN.md 4.2), 2 whenever the shape allows; B2M_TC_FUSE_SLAB 256-observation
-//   tiles per slab of the concurrent launch, B2M_TC_FUSE_RING slabs in the residual ring, B2M_TC_FUSE_GROUPS5 CTA pairs given to K5,
-//   B2M_TC_FUSE_HINTS5 / B2M_TC_FUSE_HINTS6 eviction-policy codes (A | B << 2; 0 none, 1 evict_first, 2 evict_last)
-struct Tuning {
-  int groups_resid = 0, groups_grad = 0, chunk_resid = 0, chunk_grad = 0, pair = 1, l2_hints = 0, k6_order = 1;
-  int fuse = 0, fuse_slab = 0, fuse_ring = 0, fuse_groups5 = 0, fuse_hints5 = -1, fuse_hints6 = -1;
-};
-const Tuning &tuning();
-int tuning_set(const char *name, int value);
 
 int glm_set_comm(GlmModel &g, Comm *c, cudaStream_t st);
 
@@ -148,12 +127,8 @@ int glm_recenter(GlmModel &g, const float *theta, int64_t C, cudaStream_t st);
 int simt_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st);   // B -> R, ss_part
 int simt_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);    // R -> G
 // tcgen05 implementation (glm_tc.cu)
-int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st);
-int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);
-// K5 then K6 of one evaluation: ONE launch in which half of the CTA pairs run K5 and the other half K6 a slab of
-// observations behind, the residual operand living in an L2-resident ring (large fp16-encoded problems), else the two
-// launches above
-int tc_gemm_resid_grad(GlmModel &g, int64_t Cp, cudaStream_t st);
+int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st);     // B -> R, ss_part
+int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);      // R -> G
 bool tc_available();
 void tc_profile(bool enable);
 int tc_profile_read(double *out4);

@@ -1433,10 +1433,10 @@ int glm_nuts_run_fused(GlmModel &gm, const b2m_nuts_args &a, cudaStream_t st) {
       prof_mark(3, st);
       ++g_launches;
     }
+    if ((rc = tc_gemm_resid(gm, Cp, st))) break;
     if (!peer) {
-      if ((rc = tc_gemm_resid_grad(gm, Cp, st))) break;
+      if ((rc = tc_gemm_grad(gm, Cp, st))) break;
     } else {
-      if ((rc = tc_gemm_resid(gm, Cp, st))) break;
       if ((rc = tc_gemm_grad_push(gm, Cp, st))) break;
       prof_mark(4, st);
       obs_signal_kernel<<<(unsigned)((Cp + 31) / 32), 256, 0, st>>>(gm.ss_part, gm.Np / 128, Cp, Q, seq, gm.blk_counter + 1);
@@ -1460,7 +1460,6 @@ int glm_nuts_run_fused(GlmModel &gm, const b2m_nuts_args &a, cudaStream_t st) {
     B2M_CHECK_CUDA(cudaMemcpy(&herr, pw.base[pw.rank] + pw.off_err, sizeof(int), cudaMemcpyDeviceToHost));
     B2M_REQUIRE(herr == 0, "NUTS peer exchange: a flag wait timed out");
   }
-  B2M_REQUIRE(!(gm.h_fz_err && *gm.h_fz_err), "concurrent K5 || K6 launch: a dependency wait timed out (results are invalid)");
   return 0;
 }
 

@@ -27,8 +27,6 @@
 //                 PLAIN: store the split-K partial of G                                              (K6)
 #include <cuda.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 
 #include <atomic>
 #include <vector>
@@ -99,48 +97,12 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
   // and was 7 % of the K5 stall samples
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-// L2 eviction policies for the TMA loads (opt-in, B2M_TC_L2_HINTS=1).  K6 streams the 1.6 GB residual operand past the 0.4 GB
-// transposed design matrix that sixteen row tiles re-read, and reads 3.1-4.0 GB from DRAM for 2.05 GB of operands.  Hints
-// (K6: A -> evict_first, B -> evict_last; K5: its small, re-read A operand -> evict_last) were measured and did not help
-// (K5 + K6 3.63 ms with, 3.42-3.51 ms without); what did was the tile order (column tile fastest, see the tile loop).
-// code: 1 = evict_first, 2 = evict_last (0 = no hint: the plain load is issued instead)
-__device__ __forceinline__ uint64_t l2_policy(int code) {
-  uint64_t p;
-  if (code == 2) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  else asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-// ---- dependency counters of the concurrent K5 || K6 launch (global memory, gpu scope)
-__device__ __forceinline__ int ld_acquire_gpu(const int *p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-// wait until *p >= need.  A wait that lasts ~1.5 s raises err[0] (device memory: every later wait returns at once) and the
-// pinned host flag err_host: a broken dependency makes the call fail, it cannot hang the GPU.
-__device__ __forceinline__ void spin_ge(const int *p, int need, volatile int *err, volatile int *err_host) {
-  if (ld_acquire_gpu(p) >= need) return;
-  const long long t0 = clock64();
-  while (ld_acquire_gpu(p) < need) {
-    __nanosleep(64);
-    if (*err) return;
-    if (clock64() - t0 > (1ll << 31)) { *err = 1; *err_host = 1; __threadfence_system(); return; }
-  }
-}
 // TMA load issued by one CTA of a pair; completion bytes are signalled on the LEADER's mbarrier (cluster address)
 __device__ __forceinline__ void tma_load_2d_pair(void *dst, const CUtensorMap *map, uint32_t leader_bar, int x, int y) {
   asm volatile(
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
           smem_u32(dst)),
       "l"(map), "r"(leader_bar), "r"(x), "r"(y)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_pair_hint(void *dst, const CUtensorMap *map, uint32_t leader_bar, int x, int y,
-                                                      uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-          smem_u32(dst)),
-      "l"(map), "r"(leader_bar), "r"(x), "r"(y), "l"(policy)
       : "memory");
 }
 __device__ __forceinline__ void umma_tf32_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -254,15 +216,6 @@ struct EpiParams {
   // it a few launches late because it reads the counter without draining the stream)
   const int *skip_flag;
   int skip_target;
-  int nt_fast;    // K6 tile order: column tile fastest (see the tile loop); 0 = pair row fastest (B2M_TC_K6_ORDER=0)
-  int l2_hints;   // CTA-pair kernels: L2 eviction-policy codes of the TMA loads, A | B << 2 (see l2_policy)
-  // FUSED (concurrent K5 || K6, tc_gemm_fused_kernel): the residual operand is a ring of `fz_ring` slabs of `fz_slab`
-  // 256-observation tiles, [Cp, fz_pitch] halves; fz_ready[pair row][slab] counts the epilogue warps of K5 tiles that
-  // have stored their part of the slab, fz_turn[pair row][K6 column tile] the epilogue warps of K6 tiles that have added
-  // their slab partial into G (slab order: the sum is deterministic)
-  int fz_slab, fz_ring, fz_pitch, fz_nslabs, fz_tn5, fz_tn6;
-  int *fz_ready, *fz_turn;
-  volatile int *fz_err, *fz_err_host;
   // PUSH (K6 of a peer-sliced observation shard): the finished tile goes, unscaled, straight into the window of the
   // rank that owns its chains -- slot `push_rank` of that rank's [nranks][own][Dp] gradient block -- over NVLink
   float *push_dst[kMaxPeers];
@@ -283,18 +236,16 @@ struct Cfg {
 };
 
 // MODE: 0 = PLAIN (split-K partial of G), 1 = RESID (K5 residual epilogue), 2 = PUSH (K6 tile -> owner's window)
-// FUSED: the body runs as one role of tc_gemm_fused_kernel (CTA pairs `group` of `n_groups` of that role); the residual
-// operand is the slab ring described at EpiParams and the two roles synchronise through its counters.
-template <int BLOCK_N, int MODE, int NCTA, bool F16, bool FUSED>
-__device__ __forceinline__ void
-tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap &tmBh, const CUtensorMap &tmBl,
-             const int k_blocks_total, const int k_blocks_per_split, const int CHUNK_KB, const int mma_mask, const int Tm,
-             const int Tn, const int n_tiles, const EpiParams &E, const int group, const int n_groups) {
+template <int BLOCK_N, int MODE, int NCTA, bool F16>
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
+               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl, int k_blocks_total,
+               int k_blocks_per_split, int CHUNK_KB, int mma_mask, int Tm, int Tn, int n_tiles, const __grid_constant__ EpiParams E) {
+  if (E.skip_flag && *reinterpret_cast<const volatile int *>(E.skip_flag) >= E.skip_target) return;   // uniform over the grid
   using C = Cfg<BLOCK_N, NCTA>;
   constexpr bool RESID = MODE == 1, PUSH = MODE == 2;
-  static_assert(!FUSED || (NCTA == 2 && F16 && !PUSH), "the concurrent launch exists for fp16 CTA-pair tiles");
   constexpr int BLOCK_K = Enc<F16>::BLOCK_K;   // K elements per k-block (shadows the tf32 constant)
-  constexpr int SCRATCH_BYTES = (RESID || PUSH || FUSED) ? NUM_EPI_WARPS * 32 * 33 * 4 : 0;   // per-warp transpose scratch of the epilogue
+  constexpr int SCRATCH_BYTES = (RESID || PUSH) ? NUM_EPI_WARPS * 32 * 33 * 4 : 0;   // per-warp transpose scratch of the epilogue
   extern __shared__ unsigned char smem_raw[];
   unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   float *scratch_base = reinterpret_cast<float *>(smem + C::STAGES * C::STAGE_BYTES);
@@ -306,6 +257,7 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t cta = NCTA == 2 ? cluster_ctarank() : 0u;   // rank inside the CTA pair; 0 = leader (issues the MMAs)
+  const int group = (int)blockIdx.x / NCTA, n_groups = (int)gridDim.x / NCTA;
   // Persistent tile loop: CTA group g (a CTA, or a pair) takes tiles g, g + G, g + 2G, ...  K5: tile t = (pair-row
   // t % Tm, observation tile t / Tm) -- the sixteen pairs on one observation tile share the B tile (design matrix rows),
   // the A operand (packed positions, 16 MB) lives in L2.  K6: tile t = (column tile t % Tn, pair-row (t / Tn) % Tm, K split
@@ -315,9 +267,8 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
   // are set up once; the producer and the MMA issuer run ahead into the next tile while the promotion warps are
   // still in the epilogue of the previous one (both TMEM chunk buffers are free by then).
 #define B2M_DECODE_TILE(t)                                                         \
-  const bool ntf_ = !RESID && E.nt_fast;                                           \
-  const int mp_ = ntf_ ? ((t) / Tn) % Tm : (t) % Tm;                               \
-  const int nt = ntf_ ? (t) % Tn : ((t) / Tm) % Tn;                                \
+  const int mp_ = RESID ? (t) % Tm : ((t) / Tn) % Tm;                              \
+  const int nt = RESID ? ((t) / Tm) % Tn : (t) % Tn;                               \
   const int zs = (t) / (Tm * Tn);                                                  \
   const int m0 = (mp_ * NCTA + (int)cta) * BLOCK_M, n0 = nt * BLOCK_N;             \
   const int kb0 = zs * k_blocks_per_split;                                         \
@@ -357,21 +308,8 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      // eviction-policy codes of the two operands (0 = plain load), set by the launcher
-      const int code_a = E.l2_hints & 3, code_b = (E.l2_hints >> 2) & 3;
-      const uint64_t pol_a = l2_policy(code_a), pol_b = l2_policy(code_b);
       for (int t = group; t < n_tiles; t += n_groups) {
       B2M_DECODE_TILE(t)
-      if (FUSED && !RESID) {
-        // K6 role: the slab's rows of this pair are complete once every epilogue warp (8 per CTA) of every K5 tile that
-        // covers them has arrived.  The residuals were written through the generic proxy and are read by TMA: acquire,
-        // then order the async proxy behind it.
-        const int tiles = min(E.fz_slab, E.fz_tn5 - zs * E.fz_slab);
-        spin_ge(E.fz_ready + mp_ * E.fz_nslabs + zs, tiles * NCTA * NUM_EPI_WARPS, E.fz_err, E.fz_err_host);
-        asm volatile("fence.proxy.async;" ::: "memory");
-      }
-      // column of the A operand: K6 of the concurrent launch reads slab zs from its slot of the ring
-      const int ka0 = (FUSED && !RESID) ? ((zs % E.fz_ring) * k_blocks_per_split - kb0) * BLOCK_K : 0;
       for (int kb = kb0; kb < kb1; ++kb) {
         mbar_wait(&empty[stage], phase ^ 1);
         unsigned char *st = smem + stage * C::STAGE_BYTES;
@@ -380,20 +318,10 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
           if (cta == 0) mbar_expect_tx(&full[stage], 2 * C::STAGE_BYTES);
           else mbar_arrive_cluster(lbar);
           const int nb = n0 + (int)cta * C::B_ROWS;               // this CTA's half of the B tile
-          if (code_a) {
-            tma_load_2d_pair_hint(st, &tmAh, lbar, kb * BLOCK_K + ka0, m0, pol_a);
-            tma_load_2d_pair_hint(st + A_TILE_BYTES, &tmAl, lbar, kb * BLOCK_K + ka0, m0, pol_a);
-          } else {
-            tma_load_2d_pair(st, &tmAh, lbar, kb * BLOCK_K + ka0, m0);
-            tma_load_2d_pair(st + A_TILE_BYTES, &tmAl, lbar, kb * BLOCK_K + ka0, m0);
-          }
-          if (code_b) {
-            tma_load_2d_pair_hint(st + 2 * A_TILE_BYTES, &tmBh, lbar, kb * BLOCK_K, nb, pol_b);
-            tma_load_2d_pair_hint(st + 2 * A_TILE_BYTES + C::B_TILE_BYTES, &tmBl, lbar, kb * BLOCK_K, nb, pol_b);
-          } else {
-            tma_load_2d_pair(st + 2 * A_TILE_BYTES, &tmBh, lbar, kb * BLOCK_K, nb);
-            tma_load_2d_pair(st + 2 * A_TILE_BYTES + C::B_TILE_BYTES, &tmBl, lbar, kb * BLOCK_K, nb);
-          }
+          tma_load_2d_pair(st, &tmAh, lbar, kb * BLOCK_K, m0);
+          tma_load_2d_pair(st + A_TILE_BYTES, &tmAl, lbar, kb * BLOCK_K, m0);
+          tma_load_2d_pair(st + 2 * A_TILE_BYTES, &tmBh, lbar, kb * BLOCK_K, nb);
+          tma_load_2d_pair(st + 2 * A_TILE_BYTES + C::B_TILE_BYTES, &tmBl, lbar, kb * BLOCK_K, nb);
         } else {
           mbar_expect_tx(&full[stage], C::STAGE_BYTES);
           tma_load_2d(st, &tmAh, &full[stage], kb * BLOCK_K, m0);
@@ -455,14 +383,6 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
     float acc[CW];
 #pragma unroll
     for (int j = 0; j < CW; ++j) acc[j] = 0.f;
-    bool turn_ok = true;
-    if (FUSED && !RESID && zs > 0) {
-      // K6 role: has the previous slab's partial of this output tile been added?  Sampled now, off the critical path
-      // (the tile that passes the turn on started a whole round of tiles earlier); the epilogue only waits if not.
-      int ok = 0;
-      if (lane == 0) ok = ld_acquire_gpu(E.fz_turn + mp_ * E.fz_tn6 + nt) >= zs * NCTA * NUM_EPI_WARPS;
-      turn_ok = __shfl_sync(0xffffffffu, ok, 0) != 0;
-    }
     for (int ch = 0; ch < n_chunks; ++ch, ++gch) {
       const int buf = gch & 1;
       mbar_wait(&tmem_full[buf], (gch >> 1) & 1);
@@ -497,16 +417,6 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
       const float rs_lane = F16 ? E.r_scale[m] : 1.0f;   // lane r holds the R scale of row r of this warp's 32 rows
       float *scratch = scratch_base + (warp - 2) * (32 * 33);
       const int64_t row0 = (int64_t)(m0 + q * 32);
-      // where the residuals go: [Cp, Np], or (concurrent launch) the slab's slot of the [Cp, fz_pitch] ring
-      const int r_pitch = FUSED ? E.fz_pitch : E.Np;
-      const int slab = FUSED ? nt / E.fz_slab : 0;
-      const int rcol = FUSED ? ((slab % E.fz_ring) * E.fz_slab + nt % E.fz_slab) * BLOCK_N + half * CW : nb;
-      if (FUSED && slab >= E.fz_ring) {
-        // the slot still holds slab - ring until every K6 tile of this pair row has consumed it (its turn counters are
-        // raised after the tile's last MMA has read the operand)
-        if (lane < E.fz_tn6) spin_ge(E.fz_turn + mp_ * E.fz_tn6 + lane, (slab - E.fz_ring + 1) * NCTA * NUM_EPI_WARPS, E.fz_err, E.fz_err_host);
-        __syncwarp();
-      }
       // the observations of this warp's columns: one coalesced load per 32-column block (lane = column), handed to
       // the row-owning threads by shuffle (a per-element __ldg serialised 128 L2 round trips per thread)
       float yv[CW / 32];
@@ -533,7 +443,7 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
           // (bank = 33 row + 2 col': even banks for one half-warp, odd for the other -- conflict free) packed into
           // one half2 store per array: half the conversions and half the store instructions of a per-element loop
           const int hrow = lane >> 4, cl = (lane & 15) * 2;
-          const int64_t off = (row0 + hrow) * r_pitch + rcol + b * 32 + cl;
+          const int64_t off = (row0 + hrow) * E.Np + nb + b * 32 + cl;
           __half2 *rh = reinterpret_cast<__half2 *>(static_cast<__half *>(E.Rh) + off);
           __half2 *rl = reinterpret_cast<__half2 *>(static_cast<__half *>(E.Rl) + off);
 #pragma unroll 8
@@ -541,8 +451,8 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
             const float v0 = scratch[(r + hrow) * 33 + cl], v1 = scratch[(r + hrow) * 33 + cl + 1];
             const __half2 hi = __floats2half2_rn(v0, v1);
             const float2 hf = __half22float2(hi);
-            rh[(int64_t)r * (r_pitch / 2)] = hi;
-            rl[(int64_t)r * (r_pitch / 2)] = __floats2half2_rn(v0 - hf.x, v1 - hf.y);
+            rh[(int64_t)r * (E.Np / 2)] = hi;
+            rl[(int64_t)r * (E.Np / 2)] = __floats2half2_rn(v0 - hf.x, v1 - hf.y);
           }
         } else {
           const int64_t off = row0 * E.Np + nb + b * 32 + lane;
@@ -558,17 +468,6 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
         __syncwarp();
       }
       E.ss_part[((int64_t)nt * 2 + half) * E.Cp + m] = ss;
-      if (FUSED) {
-        // publish this warp's part of the slab to the K6 role: every lane orders its own stores (gpu scope, and ahead of
-        // the async proxy that will read them), then one arrival per warp
-        __threadfence();
-        asm volatile("fence.proxy.async;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) {
-          __threadfence();   // cumulative: the warp's stores, observed through the barrier, precede the arrival
-          atomicAdd(E.fz_ready + mp_ * E.fz_nslabs + slab, 1);
-        }
-      }
     } else if (PUSH) {
       // The tile's 128 rows belong to one owner rank (own % 128 == 0).  Each warp transposes its 32 x 32 blocks through
       // the shared-memory scratch so that every store instruction writes one 128-byte row segment into the owner's
@@ -590,49 +489,6 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
         for (int r = 0; r < 32; ++r) dst[(int64_t)r * E.Dp + b * 32 + lane] = scratch[r * 33 + lane] * ics;
         __syncwarp();
       }
-    } else if (FUSED) {
-      // K6 role: the slab partial is added into the one [Cp, Dp] gradient buffer in slab order (turn counter of the output
-      // tile: 16 epilogue-warp arrivals per slab), so the sum is the same on every run.  The operand of this tile has
-      // been read completely by now (its last chunk was committed), which is what the K5 role waits for before it
-      // overwrites the ring slot.  Row segments of 128 bytes through the transposition scratch.  Every address receives
-      // its additions one slab after the other (the turn is passed on only after a gpu-scope fence), so the rounding is
-      // that of a sequential sum.
-      if (zs > 0 && !turn_ok) {   // (the counter was already sampled when the tile began: normally nothing to wait for)
-        if (lane == 0) spin_ge(E.fz_turn + mp_ * E.fz_tn6 + nt, zs * NCTA * NUM_EPI_WARPS, E.fz_err, E.fz_err_host);
-        __syncwarp();
-      }
-      float *g = E.Gpart + (int64_t)(m0 + q * 32) * E.Dp + nb;
-      float *scratch = scratch_base + (warp - 2) * (32 * 33);
-      // after the transposition a lane takes four adjacent columns of rows rr, rr + 4, ...: one 16-byte reduction (or store)
-      // per lane, four whole 128-byte row segments per warp instruction; scratch reads are conflict free (bank = rr + cc + k)
-      const int rr = lane >> 3, cc = (lane & 7) * 4;
-#pragma unroll
-      for (int b = 0; b < CW / 32; ++b) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) scratch[lane * 33 + j] = acc[b * 32 + j];
-        __syncwarp();
-        float *gp = g + b * 32 + cc;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int r = rr + 4 * i;
-          const float v0 = scratch[r * 33 + cc], v1 = scratch[r * 33 + cc + 1], v2 = scratch[r * 33 + cc + 2], v3 = scratch[r * 33 + cc + 3];
-          float *dst = gp + (int64_t)r * E.Dp;
-          if (zs > 0) {
-            // reductions performed at L2, no value returned: a load + add + store per row exposed one L2 / DRAM round trip
-            // per row to the promotion warps (measured: the K6 role ran 3.5x slower than its MMAs)
-            asm volatile("red.relaxed.gpu.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v0), "f"(v1), "f"(v2), "f"(v3) : "memory");
-          } else {
-            *reinterpret_cast<float4 *>(dst) = make_float4(v0, v1, v2, v3);
-          }
-        }
-        __syncwarp();
-      }
-      // one arrival per warp; lane 0's fence is cumulative over the warp's reductions (ordered before it by the barrier)
-      __syncwarp();
-      if (lane == 0) {
-        __threadfence();
-        atomicAdd(E.fz_turn + mp_ * E.fz_tn6 + nt, 1);
-      }
     } else {
       float *g = E.Gpart + ((int64_t)zs * E.Cp + m) * E.Dp + nb;
 #pragma unroll
@@ -653,39 +509,6 @@ tc_gemm_body(const CUtensorMap &tmAh, const CUtensorMap &tmAl, const CUtensorMap
     else
       asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS));
   }
-}
-
-template <int BLOCK_N, int MODE, int NCTA, bool F16>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
-               const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl, int k_blocks_total,
-               int k_blocks_per_split, int CHUNK_KB, int mma_mask, int Tm, int Tn, int n_tiles, const __grid_constant__ EpiParams E) {
-  if (E.skip_flag && *reinterpret_cast<const volatile int *>(E.skip_flag) >= E.skip_target) return;   // uniform over the grid
-  tc_gemm_body<BLOCK_N, MODE, NCTA, F16, false>(tmAh, tmAl, tmBh, tmBl, k_blocks_total, k_blocks_per_split, CHUNK_KB, mma_mask, Tm,
-                                                Tn, n_tiles, E, (int)blockIdx.x / NCTA, (int)gridDim.x / NCTA);
-}
-
-// K5 || K6 of one evaluation in ONE launch (fp16 encoding, CTA pairs, 256-column tiles).  The first `groups5` CTA pairs
-// run K5 over the observation tiles in order, the rest run K6 one slab of observations behind them; the residual operand
-// lives in a ring of a few slabs that stays in L2 (it never reaches HBM: two launches write and re-read 3.2 GB of it per
-// evaluation at C4), the transposed design matrix is read once per slab while the sixteen pair rows are on it, and the
-// slab partials of the gradient are added into one buffer in slab order.  Both roles are the bodies of the separate
-// kernels; only the dependency counters (EpiParams::fz_*) are new.  All CTAs of the launch are resident at once (one per
-// SM), so a role waiting for the other cannot starve it.
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-tc_gemm_fused_kernel(const __grid_constant__ CUtensorMap a5h, const __grid_constant__ CUtensorMap a5l,
-                     const __grid_constant__ CUtensorMap b5h, const __grid_constant__ CUtensorMap b5l,
-                     const __grid_constant__ CUtensorMap a6h, const __grid_constant__ CUtensorMap a6l,
-                     const __grid_constant__ CUtensorMap b6h, const __grid_constant__ CUtensorMap b6l, int kb5, int chunk5,
-                     int Tm, int kb6_total, int kb6_per, int chunk6, int groups5, const __grid_constant__ EpiParams E5,
-                     const __grid_constant__ EpiParams E6) {
-  if (E5.skip_flag && *reinterpret_cast<const volatile int *>(E5.skip_flag) >= E5.skip_target) return;   // uniform over the grid
-  const int group = (int)blockIdx.x / 2, n_groups = (int)gridDim.x / 2;
-  if (group < groups5)
-    tc_gemm_body<256, 1, 2, true, true>(a5h, a5l, b5h, b5l, kb5, kb5, chunk5, 7, Tm, E5.fz_tn5, Tm * E5.fz_tn5, E5, group, groups5);
-  else
-    tc_gemm_body<256, 0, 2, true, true>(a6h, a6l, b6h, b6l, kb6_total, kb6_per, chunk6, 7, Tm, E6.fz_tn6,
-                                        Tm * E6.fz_tn6 * E6.fz_nslabs, E6, group - groups5, n_groups - groups5);
 }
 
 // ---------------------------------------------------------------- tensor maps
@@ -781,11 +604,7 @@ int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap 
   }
   // `grid` arrives as (128-row tiles, column tiles, K splits); the launch is one persistent CTA group per SM (pair)
   const int Tm = (int)grid.x / NCTA, Tn = (int)grid.y, n_tiles = Tm * Tn * (int)grid.z;
-  int n_groups = n_tiles < 148 / NCTA ? n_tiles : 148 / NCTA;
-  {   // experiments: fewer persistent CTA groups (read once per process, glm.cuh)
-    const int want = RESID ? tuning().groups_resid : tuning().groups_grad;
-    if (want > 0 && want < n_groups) n_groups = want;
-  }
+  const int n_groups = n_tiles < 148 / NCTA ? n_tiles : 148 / NCTA;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (g_prof.on) {
     B2M_CHECK_CUDA(cudaEventCreate(&e0));
@@ -885,53 +704,10 @@ int tc_profile_read(double *out4) {
   return 0;
 }
 
-static Tuning &tuning_storage() {
-  static Tuning t = [] {   // C++11 magic static: initialised once, thread safe
-    Tuning x;
-    auto geti = [](const char *name, int dflt) {
-      const char *v = getenv(name);
-      return v ? atoi(v) : dflt;
-    };
-    x.groups_resid = geti("B2M_TC_GROUPS_RESID", 0);
-    x.groups_grad = geti("B2M_TC_GROUPS_GRAD", 0);
-    x.chunk_resid = geti("B2M_TC_CHUNK_RESID", 0);
-    x.chunk_grad = geti("B2M_TC_CHUNK_GRAD", 0);
-    x.pair = geti("B2M_TC_PAIR", 1);
-    x.l2_hints = geti("B2M_TC_L2_HINTS", 0);
-    x.k6_order = geti("B2M_TC_K6_ORDER", 1);
-    x.fuse = geti("B2M_TC_FUSE", 0);
-    x.fuse_slab = geti("B2M_TC_FUSE_SLAB", 0);
-    x.fuse_ring = geti("B2M_TC_FUSE_RING", 0);
-    x.fuse_groups5 = geti("B2M_TC_FUSE_GROUPS5", 0);
-    x.fuse_hints5 = geti("B2M_TC_FUSE_HINTS5", -1);
-    x.fuse_hints6 = geti("B2M_TC_FUSE_HINTS6", -1);
-    return x;
-  }();
-  return t;
-}
-const Tuning &tuning() { return tuning_storage(); }
-
-// tests / experiments: change one knob of the process (not thread safe against running launches; b2m_tuning_set)
-int tuning_set(const char *name, int value) {
-  Tuning &t = tuning_storage();
-  struct { const char *n; int *p; } tab[] = {
-      {"groups_resid", &t.groups_resid}, {"groups_grad", &t.groups_grad}, {"chunk_resid", &t.chunk_resid},
-      {"chunk_grad", &t.chunk_grad}, {"pair", &t.pair}, {"l2_hints", &t.l2_hints}, {"k6_order", &t.k6_order}, {"fuse", &t.fuse},
-      {"fuse_slab", &t.fuse_slab}, {"fuse_ring", &t.fuse_ring}, {"fuse_groups5", &t.fuse_groups5},
-      {"fuse_hints5", &t.fuse_hints5}, {"fuse_hints6", &t.fuse_hints6}};
-  for (auto &e : tab)
-    if (name && !strcmp(name, e.n)) { *e.p = value; return 0; }
-  set_error(std::string("b2m_tuning_set: unknown knob '") + (name ? name : "(null)") + "'");
-  return 2;
-}
-
 int grad_block_n(const GlmModel &g) { return g.Dp % 256 == 0 ? 256 : (g.Dp % 128 == 0 ? 128 : 64); }
 
-// CTA pairs need whole 256-row tiles of chains; B2M_TC_PAIR=0 forces the single-CTA kernel (experiments)
-static int pair_mode(int64_t Cp) {
-  if (tuning().pair == 0) return 1;
-  return (Cp % 256 == 0) ? 2 : 1;
-}
+// CTA pairs need whole 256-row tiles of chains
+static int pair_mode(int64_t Cp) { return (Cp % 256 == 0) ? 2 : 1; }
 
 // split-K factor of K6: enough CTAs to fill the 148 SMs in whole waves, each split at least 8 k-blocks deep
 int grad_splits(const GlmModel &g, int64_t Cp) {
@@ -964,7 +740,6 @@ int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   EpiParams E{};
   E.y = g.y0; E.inv_var = g.inv_var; E.ss_part = g.ss_part; E.Cp = Cp; E.Np = g.Np;
   E.skip_flag = g.skip_flag; E.skip_target = g.skip_target;
-  E.l2_hints = tuning().l2_hints ? 2 : 0;   // A (packed positions, re-read by every column tile): evict_last
   E.Rh = f16 ? (void *)g.R16h : (void *)g.Rh;
   E.Rl = f16 ? (void *)g.R16l : (void *)g.Rl;
   E.a_unscale = g.a_unscale; E.r_scale = g.r_scale;
@@ -976,7 +751,7 @@ int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   // fp16 encoding with K >= 512: two chunks of 8 k-blocks (512 values of K) per tile instead of four of 4 -- TMEM holds two
   // chunk accumulators, so the issuer can then run a WHOLE tile ahead of the residual epilogue instead of half a tile
   // (measured at C4: K5 1.94 -> 1.89 ms; gradient error vs float64 unchanged at 2e-6, full-size test green)
-  const int ck = tuning().chunk_resid > 0 ? tuning().chunk_resid : ((f16 && g.Dp / bk >= 8) ? 8 : DEFAULT_CHUNK_KB);
+  const int ck = (f16 && g.Dp / bk >= 8) ? 8 : DEFAULT_CHUNK_KB;
   return launch_tc<256, 1>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
 }
 
@@ -997,145 +772,12 @@ int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st) {
   EpiParams E{};
   E.Gpart = g.G; E.Cp = Cp; E.Dp = g.Dp;
   E.skip_flag = g.skip_flag; E.skip_target = g.skip_target;
-  E.l2_hints = tuning().l2_hints ? (1 | 2 << 2) : 0;   // A (residual stream): evict_first, B (transposed design matrix): evict_last
-  E.nt_fast = tuning().k6_order;
   dim3 grid((unsigned)(Cp / BLOCK_M), g.Dp / bn, (unsigned)((kb_total + kb_per - 1) / kb_per));
   g.g_splits = (int)grid.z;
-  const int ck = tuning().chunk_grad > 0 ? tuning().chunk_grad : (f16 ? DEFAULT_CHUNK_KB / 2 : DEFAULT_CHUNK_KB);
+  const int ck = f16 ? DEFAULT_CHUNK_KB / 2 : DEFAULT_CHUNK_KB;
   if (bn == 256) return launch_tc<256, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
   if (bn == 128) return launch_tc<128, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
   return launch_tc<64, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
-}
-
-// ---------------------------------------------------------------- K5 || K6 in one launch
-namespace {
-struct FusePlan {
-  bool on = false;
-  int slab = 0, ring = 0, n_slabs = 0, groups5 = 0, n_pairs = 0;
-};
-// The concurrent launch pays when the residual operand is far larger than L2 (it then costs two passes over HBM) and
-// there are enough slabs for the one-slab lag between the roles to be small against the whole evaluation.
-FusePlan fuse_plan(const GlmModel &g, int64_t Cp) {
-  FusePlan p;
-  const Tuning &T = tuning();
-  if (!T.fuse || g.use_tc != 2 || pair_mode(Cp) != 2 || g.Dp % 256 != 0) return p;
-  const int tn5 = g.Np / 256;
-  // slab: about 8 MB of residuals (hi + lo halves) for the batch, between 1 and 8 observation tiles, in a ring of two.
-  // Measured at C4 (profiles/r02_tc_gemm_fused_c4_ncu_summary.md): a 17 MB ring stays in L2 (DRAM traffic of the
-  // evaluation 6.3 -> 1.1 GB), 25 MB begins to spill (2.4 GB), 50 MB spills completely -- next to the 16 MB of packed
-  // positions and the 16 MB gradient buffer the two-die L2 keeps about half of its nominal 126 MB for this pattern.
-  int slab = T.fuse_slab > 0 ? T.fuse_slab : (int)((8ll << 20) / (Cp * 256 * 4));
-  if (slab < 1) slab = 1;
-  if (slab > 8 && T.fuse_slab <= 0) slab = 8;
-  const int ring = T.fuse_ring >= 2 ? T.fuse_ring : 2;
-  const int n_slabs = (tn5 + slab - 1) / slab;
-  const int64_t r_bytes = Cp * (int64_t)g.Np * 4;
-  if (n_slabs < 4 * ring || (r_bytes < (256ll << 20) && T.fuse < 2)) return p;   // B2M_TC_FUSE=2: whenever the shape allows
-  p.n_pairs = 148 / 2;
-  // the K6 role pays an epilogue (transposition + reductions at L2) per slab instead of per split: it gets the larger half
-  p.groups5 = T.fuse_groups5 > 0 && T.fuse_groups5 < p.n_pairs ? T.fuse_groups5 : p.n_pairs / 2 - 2;
-  p.slab = slab; p.ring = ring; p.n_slabs = n_slabs;
-  p.on = true;
-  return p;
-}
-}  // namespace
-
-static int tc_gemm_fused(GlmModel &g, int64_t Cp, const FusePlan &P, cudaStream_t st) {
-  if (g.h_fz_err && *g.h_fz_err) {
-    set_error("concurrent K5 || K6 launch: a dependency wait timed out in an earlier evaluation (results are invalid)");
-    return 2;
-  }
-  const int bk = 64, kb5 = g.Dp / bk, tn5 = g.Np / 256, tn6 = g.Dp / 256, Tm = (int)(Cp / 256);
-  const int pitch = P.ring * P.slab * 256;
-  // counters [ready: Tm x n_slabs | turn: Tm x tn6 | err]; the error word is cleared once, the counters before every launch
-  const size_t n_cnt = (size_t)Tm * P.n_slabs + (size_t)Tm * tn6;
-  if (g.fz_sync_cap < n_cnt + 1) {
-    if (g.fz_sync) { B2M_CHECK_CUDA(cudaStreamSynchronize(st)); cudaFree(g.fz_sync); g.fz_sync = nullptr; g.fz_sync_cap = 0; }
-    B2M_CHECK_CUDA(cudaMalloc(reinterpret_cast<void **>(&g.fz_sync), sizeof(int) * (n_cnt + 1 + 1024)));
-    g.fz_sync_cap = n_cnt + 1 + 1024;
-    B2M_CHECK_CUDA(cudaMemsetAsync(g.fz_sync, 0, sizeof(int) * g.fz_sync_cap, st));
-  }
-  if (!g.h_fz_err) {
-    int *hp = nullptr;
-    B2M_CHECK_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&hp), sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
-    *hp = 0;
-    g.h_fz_err = hp;
-  }
-  int *err_dev = g.fz_sync + g.fz_sync_cap - 1;
-  B2M_CHECK_CUDA(cudaMemsetAsync(g.fz_sync, 0, sizeof(int) * n_cnt, st));
-  CUtensorMap a5h, a5l, b5h, b5l, a6h, a6l, b6h, b6l;
-  if (make_map(&a5h, g.B16h, Cp, g.Dp, BLOCK_M, true) || make_map(&a5l, g.B16l, Cp, g.Dp, BLOCK_M, true) ||
-      make_map(&b5h, g.X16h, g.Np, g.Dp, 128, true) || make_map(&b5l, g.X16l, g.Np, g.Dp, 128, true) ||
-      make_map(&a6h, g.R16h, Cp, pitch, BLOCK_M, true) || make_map(&a6l, g.R16l, Cp, pitch, BLOCK_M, true) ||
-      make_map(&b6h, g.XT16h, g.Dp, g.Np, 128, true) || make_map(&b6l, g.XT16l, g.Dp, g.Np, 128, true))
-    return 2;
-  const Tuning &T = tuning();
-  EpiParams E5{};
-  E5.y = g.y0; E5.inv_var = g.inv_var; E5.ss_part = g.ss_part; E5.Cp = Cp; E5.Np = g.Np;
-  E5.skip_flag = g.skip_flag; E5.skip_target = g.skip_target;
-  E5.Rh = g.R16h; E5.Rl = g.R16l;
-  E5.a_unscale = g.a_unscale; E5.r_scale = g.r_scale;
-  E5.N_valid = g.N; E5.loc_const = 0.f; E5.weight = g.weight;
-  E5.fz_slab = P.slab; E5.fz_ring = P.ring; E5.fz_pitch = pitch; E5.fz_nslabs = P.n_slabs; E5.fz_tn5 = tn5; E5.fz_tn6 = tn6;
-  E5.fz_ready = g.fz_sync; E5.fz_turn = g.fz_sync + (size_t)Tm * P.n_slabs;
-  E5.fz_err = err_dev; E5.fz_err_host = g.h_fz_err;
-  EpiParams E6 = E5;
-  E6.Gpart = g.G; E6.Dp = g.Dp;
-  E6.nt_fast = T.k6_order;
-  // K5: A = packed positions (16 MB, re-read for every observation tile) -> evict_last, B = design matrix, read once while
-  // the sixteen pair rows are on the tile -> evict_first.  K6: no hints (the ring and the slab of the transposed matrix are
-  // re-read within a slab time and then dead).
-  E5.l2_hints = T.fuse_hints5 >= 0 ? T.fuse_hints5 : (2 | 1 << 2);
-  E6.l2_hints = T.fuse_hints6 >= 0 ? T.fuse_hints6 : 0;
-  g.g_splits = 1;
-  const int chunk5 = T.chunk_resid > 0 ? T.chunk_resid : (kb5 >= 8 ? 8 : DEFAULT_CHUNK_KB);
-  const int chunk6 = T.chunk_grad > 0 ? T.chunk_grad : DEFAULT_CHUNK_KB / 2;
-  const int kb6_total = g.Np / bk, kb6_per = P.slab * 4;
-  auto kernel = tc_gemm_fused_kernel;
-  using C = Cfg<256, 2>;
-  constexpr int SMEM = C::SMEM_BYTES + NUM_EPI_WARPS * 32 * 33 * 4;
-  static std::atomic<bool> configured[64];
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
-    B2M_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
-  }
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (g_prof.on) {
-    B2M_CHECK_CUDA(cudaEventCreate(&e0));
-    B2M_CHECK_CUDA(cudaEventCreate(&e1));
-    B2M_CHECK_CUDA(cudaEventRecord(e0, st));
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(P.n_pairs * 2), 1, 1);
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = SMEM;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  B2M_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, a5h, a5l, b5h, b5l, a6h, a6l, b6h, b6l, kb5, chunk5, Tm, kb6_total, kb6_per,
-                                    chunk6, P.groups5, E5, E6));
-  if (g_prof.on) {   // one launch covers both contractions: recorded under K5, no K6 entry (bench.py reads it that way)
-    B2M_CHECK_CUDA(cudaEventRecord(e1, st));
-    g_prof.ev[0].push_back(e0);
-    g_prof.ev[0].push_back(e1);
-  }
-  ++g_launches;
-  B2M_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
-int tc_gemm_resid_grad(GlmModel &g, int64_t Cp, cudaStream_t st) {
-  const FusePlan P = fuse_plan(g, Cp);
-  if (P.on) return tc_gemm_fused(g, Cp, P, st);
-  if (int rc = tc_gemm_resid(g, Cp, st)) return rc;
-  return tc_gemm_grad(g, Cp, st);
 }
 
 // K6 of a peer-sliced observation shard: one K pass over the rank's rows (no split-K: every output tile is produced
@@ -1152,14 +794,12 @@ int tc_gemm_grad_push(GlmModel &g, int64_t Cp, cudaStream_t st) {
     return 2;
   EpiParams E{};
   E.Cp = Cp; E.Dp = g.Dp;
-  E.l2_hints = tuning().l2_hints ? (1 | 2 << 2) : 0;
-  E.nt_fast = tuning().k6_order;
   E.push_own = (int)w.own; E.push_rank = w.rank;
   for (int s = 0; s < w.nranks; ++s) E.push_dst[s] = reinterpret_cast<float *>(w.base[s] + w.off_g);
   E.r_unscale = g.r_unscale; E.inv_col_scale = g.inv_col_scale;
   dim3 grid((unsigned)(Cp / BLOCK_M), g.Dp / bn, 1);
   g.g_splits = 1;
-  const int ck = tuning().chunk_grad > 0 ? tuning().chunk_grad : DEFAULT_CHUNK_KB / 2;
+  const int ck = DEFAULT_CHUNK_KB / 2;
   if (bn == 256) return launch_tc<256, 2>(2, Ah, Al, Bh, Bl, grid, kb_total, kb_total, E, st, ck, 7, true);
   if (bn == 128) return launch_tc<128, 2>(2, Ah, Al, Bh, Bl, grid, kb_total, kb_total, E, st, ck, 7, true);
   return launch_tc<64, 2>(2, Ah, Al, Bh, Bl, grid, kb_total, kb_total, E, st, ck, 7, true);

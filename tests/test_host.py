@@ -32,18 +32,6 @@ def test_library_loads_and_exports_every_declared_symbol():
                                                         _cabi.MhArgs, _cabi.NutsArgs)]
 
 
-def test_tuning_knobs_are_named_and_unknown_names_are_errors():
-    """b2m_tuning_set (launch-shape experiments; host-only state, no CUDA call): every knob the header names exists, the
-    defaults are the measured ones (two launches, column-tile-fastest K6 order, no L2 hints) and a typo is an error."""
-    lib = _cabi.load()
-    for knob, default in (("fuse", 0), ("fuse_slab", 0), ("fuse_ring", 0), ("fuse_groups5", 0), ("l2_hints", 0),
-                          ("k6_order", 1), ("pair", 1)):
-        assert lib.b2m_tuning_set(knob.encode(), default) == 0, knob
-    assert lib.b2m_tuning_set(b"no_such_knob", 1) != 0
-    assert b"no_such_knob" in lib.b2m_last_error()
-    assert lib.b2m_tuning_set(None, 1) != 0
-
-
 def test_library_is_sm100a_only():
     import subprocess
     out = subprocess.run(["cuobjdump", "--list-elf", _cabi.lib_path()], capture_output=True, text=True).stdout

@@ -52,8 +52,7 @@ for _ in range(args.reps):
     torch.cuda.synchronize()
     times.append(a.elapsed_time(b))
 ms = float(np.median(times))
-# GEMM-only time of the same calls: CUDA events inside the library around every K5 / K6 launch (one entry when the two run
-# as the concurrent launch)
+# GEMM-only time of the same calls: CUDA events inside the library around every K5 / K6 launch
 import ctypes
 from mlx_mcmc_b200 import _cabi
 lib = _cabi.load()
@@ -66,8 +65,8 @@ lib.b2m_profile(0)
 k5 = four[0] / max(four[1], 1)
 k6 = four[2] / max(four[3], 1)
 flops = 4.0 * args.n * args.d * args.chains
-out = {"glm_path": model.glm_path, "gemm_ms": {"K5": k5, "K6": k6, "both": k5 + k6, "fused": four[3] == 0},
-       "knobs": {k: v for k, v in os.environ.items() if k.startswith("B2M_TC_")}, "where": args.where, "n": args.n, "d": args.d, "chains": args.chains, "path": args.path, "ms_per_eval": ms, "all_ms": times,
+out = {"glm_path": model.glm_path, "gemm_ms": {"K5": k5, "K6": k6, "both": k5 + k6},
+       "where": args.where, "n": args.n, "d": args.d, "chains": args.chains, "path": args.path, "ms_per_eval": ms, "all_ms": times,
        "useful_tflops": flops / ms / 1e9, "grad_evals_per_s": args.chains / ms * 1e3,
        "logical_GBps": 4.0 * args.n * args.d * args.chains / ms / 1e6}
 if args.check:
