@@ -38,20 +38,22 @@ typedef unsigned long long uintptr_t;
 extern "C" {
 #endif
 
-#define B2M_ABI_VERSION 3
+#define B2M_ABI_VERSION 4
 #define B2M_MAX_TREE_DEPTH 12
 
 /* ---- model description (produced by the Python tracer from the user's log_prob) ---- */
 
-/* distribution tags: the reference's six classes (mlx_mcmc/distributions/<name>.py) */
+/* distribution tags: the reference's six classes (mlx_mcmc/distributions/<name>.py), plus Bernoulli (ABI 4) */
 enum {
   B2M_NORMAL = 0,      /* normal.py:49-56      p0=loc  p1=scale               */
   B2M_HALFNORMAL = 1,  /* halfnormal.py:55-63  p0=scale           mask x>=0   */
   B2M_EXPONENTIAL = 2, /* exponential.py:61-71 p0=rate            mask x>=0   */
   B2M_GAMMA = 3,       /* gamma.py:53-88       p0=rate(beta) k0=alpha k1=lgamma(alpha)  mask x>0 */
   B2M_BETA = 4,        /* beta.py:53-91        k0=a k1=b k2=logB(a,b)         mask 0<x<1 */
-  B2M_CONSTANT = 5     /* a term with no traced operand: value k0 (Categorical with concrete
+  B2M_CONSTANT = 5,    /* a term with no traced operand: value k0 (Categorical with concrete
                           probs/index, categorical.py:69-93, folds to this)   */
+  B2M_BERNOULLI = 7    /* x=label p0=logit: x p0 - softplus(p0), mask x in {0, 1}; p1 unused.  Not 6: that value is
+                          B2M_SAMPLE_CATEGORICAL of b2m_sample, and 6 stays an unknown term tag */
 };
 
 /* operand kinds: value[n] of one slot of a term, n = element index inside the term */
@@ -310,8 +312,8 @@ int b2m_quantiles(const float *x, int64_t n, const double *q, int32_t n_q, doubl
 /* ---- forward sampling on the device (SURVEY.md 8f row 4) ----
  * n draws from one library distribution into out[n] (device).  Replaces Distribution.sample (distributions/<name>.py; the
  * reference's Gamma / Beta fall back to numpy, gamma.py:107-117, beta.py:110-119).  dist = B2M_NORMAL (p0 loc, p1 scale),
- * B2M_HALFNORMAL (p0 scale), B2M_EXPONENTIAL (p0 rate), B2M_GAMMA (p0 alpha, p1 rate), B2M_BETA (p0 a, p1 b) or
- * B2M_SAMPLE_CATEGORICAL (cdf = device array of n_cat cumulative probabilities, last = 1; draws are indices as floats).
+ * B2M_HALFNORMAL (p0 scale), B2M_EXPONENTIAL (p0 rate), B2M_GAMMA (p0 alpha, p1 rate), B2M_BETA (p0 a, p1 b),
+ * B2M_BERNOULLI (p0 = probability of 1; draws are 0 / 1 as floats) or B2M_SAMPLE_CATEGORICAL (cdf = device array of n_cat cumulative probabilities, last = 1; draws are indices as floats).
  * Output i depends only on (seed, i). */
 #define B2M_SAMPLE_CATEGORICAL 6
 int b2m_sample(int32_t dist, float p0, float p1, const float *cdf, int32_t n_cat, uint64_t seed, int64_t n, float *out,

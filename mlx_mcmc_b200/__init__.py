@@ -18,7 +18,7 @@ from types import SimpleNamespace as _NS
 __version__ = "0.1.0"
 
 from . import core
-from .distributions import Beta, Categorical, Distribution, Exponential, Gamma, HalfNormal, Normal
+from .distributions import Bernoulli, Beta, Categorical, Distribution, Exponential, Gamma, HalfNormal, Normal
 from .inference.mcmc import MCMC
 from .kernels.hmc import hmc
 from .kernels.metropolis import metropolis_hastings
@@ -27,7 +27,7 @@ from .tracer import UnsupportedOpError, trace
 
 # namespace object accepted by the model factories in mlx_mcmc_b200.workloads
 ns = _NS(mx=core, Normal=Normal, HalfNormal=HalfNormal, Beta=Beta, Gamma=Gamma, Exponential=Exponential,
-         Categorical=Categorical)
+         Categorical=Categorical, Bernoulli=Bernoulli)
 
-__all__ = ["Normal", "HalfNormal", "Beta", "Gamma", "Exponential", "Categorical", "metropolis_hastings", "hmc",
+__all__ = ["Normal", "HalfNormal", "Beta", "Gamma", "Exponential", "Categorical", "Bernoulli", "metropolis_hastings", "hmc",
            "nuts", "MCMC", "core", "trace", "UnsupportedOpError", "ns"]

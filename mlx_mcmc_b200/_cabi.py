@@ -74,7 +74,7 @@ GLM_AUTO, GLM_SIMT, GLM_TC, GLM_TC16 = 0, 1, 2, 3
 GLM_PATHS = {"auto": GLM_AUTO, "simt": GLM_SIMT, "tc": GLM_TC, "tc16": GLM_TC16}
 POINTWISE_AUTO, POINTWISE_GENERAL = 0, 1
 MAX_TREE_DEPTH = 12
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 EXPORTS = ["b2m_last_error", "b2m_abi_version", "b2m_struct_sizes", "b2m_model_create", "b2m_model_destroy",
            "b2m_model_dim", "b2m_model_class", "b2m_model_glm_path", "b2m_logp_grad", "b2m_hmc_run", "b2m_mh_run", "b2m_nuts_run",

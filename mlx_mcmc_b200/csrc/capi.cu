@@ -24,6 +24,7 @@ int launch_hmc(const KModel &km, b2m_hmc_args a, cudaStream_t st, JitModule *jit
 int launch_mh(const KModel &km, b2m_mh_args a, cudaStream_t st, JitModule *jit);
 int launch_nuts(const KModel &km, b2m_nuts_args a, cudaStream_t st, JitModule *jit);
 int glm_build(GlmModel &g, const float *X, const float *y, int N, int D, bool force_tc16);
+int glm_check_labels(const float *y, int N);
 int mass_from_draws(const float *draws, int64_t S, int64_t C, int64_t D, float *inv_mass, cudaStream_t st);
 int quantiles(const float *x, int64_t n, const double *q, int n_q, double *out, cudaStream_t st);
 int peer_alloc(int64_t bytes, void **ptr, uint8_t *handle64);
@@ -96,8 +97,9 @@ static int check_operand(const b2m_operand &o, int length, int D, int n_lin, con
   }
 }
 
-// GLM class: exactly one Normal likelihood whose location is X @ beta (+ const), observed y, scale constant or
-// a scalar parameter; every other term is a pointwise prior.
+// GLM class: exactly one likelihood over X @ beta (+ const) and an observed vector y -- a Normal with X @ beta as its
+// location and a constant or scalar-parameter scale, or a Bernoulli with X @ beta as its logits and labels y in {0, 1};
+// every other term is a pointwise prior.
 static int setup_glm(b2m_model *m, int D, int glm_path, const int32_t *tf) {
   int lik = -1;
   for (size_t t = 0; t < m->terms.size(); ++t) {
@@ -105,10 +107,10 @@ static int setup_glm(b2m_model *m, int D, int glm_path, const int32_t *tf) {
     const bool has_mv = T.x.kind == B2M_OP_MATVEC || T.p0.kind == B2M_OP_MATVEC || T.p1.kind == B2M_OP_MATVEC;
     if (!has_mv) continue;
     B2M_REQUIRE(lik < 0, "GLM class: only one X @ beta term is supported");
-    B2M_REQUIRE(T.dist == B2M_NORMAL && T.p0.kind == B2M_OP_MATVEC && T.x.kind == B2M_OP_DATA &&
-                    (T.p1.kind == B2M_OP_CONST || T.p1.kind == B2M_OP_PARAM),
+    const bool normal = T.dist == B2M_NORMAL && (T.p1.kind == B2M_OP_CONST || T.p1.kind == B2M_OP_PARAM);
+    B2M_REQUIRE((normal || T.dist == B2M_BERNOULLI) && T.p0.kind == B2M_OP_MATVEC && T.x.kind == B2M_OP_DATA,
                 "GLM class: X @ beta must be the location of a Normal likelihood over an observed vector, with a "
-                "constant or scalar-parameter scale");
+                "constant or scalar-parameter scale, or the logits of a Bernoulli likelihood over observed labels");
     lik = (int)t;
   }
   B2M_REQUIRE(lik >= 0, "GLM class: no X @ beta term found");
@@ -121,8 +123,11 @@ static int setup_glm(b2m_model *m, int D, int glm_path, const int32_t *tf) {
   g.beta_off = L.p0.b;
   g.loc_const = L.p0.c;
   g.weight = L.weight;
-  g.sigma_param = L.p1.kind == B2M_OP_PARAM ? L.p1.a : -1;
-  g.sigma_const = L.p1.kind == B2M_OP_CONST ? L.p1.c : 1.f;
+  g.lik = L.dist == B2M_BERNOULLI ? b2m::kLikLogit : b2m::kLikNormal;
+  g.sigma_param = (g.lik == b2m::kLikNormal && L.p1.kind == B2M_OP_PARAM) ? L.p1.a : -1;
+  g.sigma_const = (g.lik == b2m::kLikNormal && L.p1.kind == B2M_OP_CONST) ? L.p1.c : 1.f;
+  if (g.lik == b2m::kLikLogit)
+    if (int rc = b2m::glm_check_labels(Y.data, (int)L.length)) return rc;
   // b2m_model_options.glm_path: SIMT (fp32 FMA tiles) | TC (tcgen05 3xTF32) | TC16 (tcgen05 3xFP16 with scaled operands);
   // AUTO: the fp16 encoding when the data's dynamic range allows it (checked in glm_build), else tf32
   g.use_tc = (!b2m::tc_available() || glm_path == B2M_GLM_SIMT) ? 0 : (glm_path == B2M_GLM_TC ? 1 : 2);
@@ -172,7 +177,9 @@ int b2m_debug_tc_gemm(const float *A, const float *Bm, int M, int N, int K, floa
 int b2m_sample(int32_t dist, float p0, float p1, const float *cdf, int32_t n_cat, uint64_t seed, int64_t n, float *out,
                void *stream) {
   B2M_REQUIRE(n >= 0 && (out || n == 0), "b2m_sample: bad output");
-  B2M_REQUIRE((dist >= B2M_NORMAL && dist <= B2M_BETA) || dist == B2M_SAMPLE_CATEGORICAL, "b2m_sample: unknown distribution tag");
+  B2M_REQUIRE((dist >= B2M_NORMAL && dist <= B2M_BETA) || dist == B2M_SAMPLE_CATEGORICAL || dist == B2M_BERNOULLI,
+              "b2m_sample: unknown distribution tag");
+  if (dist == B2M_BERNOULLI) B2M_REQUIRE(p0 >= 0.f && p0 <= 1.f, "b2m_sample: a Bernoulli probability must lie in [0, 1]");
   B2M_REQUIRE(dist != B2M_SAMPLE_CATEGORICAL || (cdf && n_cat > 0), "b2m_sample: categorical needs a cdf");
   if (dist == B2M_GAMMA || dist == B2M_BETA) B2M_REQUIRE(p0 > 0.f && p1 > 0.f, "b2m_sample: shape / rate parameters must be positive");
   return b2m::sample(dist, p0, p1, cdf, n_cat, seed, n, out, static_cast<cudaStream_t>(stream));
@@ -243,7 +250,7 @@ int b2m_model_create(const b2m_term *terms, int32_t n_terms, const b2m_lin_entry
   }
   for (int t = 0; t < n_terms; ++t) {
     const b2m_term &T = terms[t];
-    if (T.dist < B2M_NORMAL || T.dist > B2M_CONSTANT) {
+    if ((T.dist < B2M_NORMAL || T.dist > B2M_CONSTANT) && T.dist != B2M_BERNOULLI) {
       set_error("term " + std::to_string(t) + ": unknown distribution tag " + std::to_string(T.dist));
       return 1;
     }
@@ -422,6 +429,7 @@ int b2m_model_peer_bytes(b2m_model *m, int64_t n_chains, int32_t n_ranks, int64_
 int b2m_model_peer_attach(b2m_model *m, void *const *windows, int32_t n_ranks, int32_t rank, int64_t n_chains, int64_t bytes) {
   B2M_REQUIRE(m && windows, "b2m_model_peer_attach: NULL argument");
   B2M_REQUIRE(m->model_class == 1, "b2m_model_peer_attach: the peer window is defined for GLM-class models only");
+  B2M_REQUIRE(m->glm.lik == b2m::kLikNormal, "b2m_model_peer_attach: observation sharding is defined for the Normal likelihood only");
   B2M_REQUIRE(m->glm.use_tc == 2, "b2m_model_peer_attach: the peer exchange is built on the fp16-encoded tcgen05 path");
   B2M_REQUIRE(m->glm.tf == nullptr, "b2m_model_peer_attach: constraint transforms are not supported with the peer exchange");
   B2M_REQUIRE(n_ranks >= 2 && n_ranks <= b2m::kMaxPeers && rank >= 0 && rank < n_ranks, "b2m_model_peer_attach: 2..8 ranks");

@@ -151,6 +151,31 @@ __global__ void split_f16_kernel(const float *__restrict__ Xp, int Np, int Dp, c
   XTh[(int64_t)d * Np + n] = hi; XTl[(int64_t)d * Np + n] = lo;
 }
 
+// labels of a Bernoulli likelihood: count the entries of y[0, N) that are neither 0 nor 1 (NaN included)
+__global__ void count_bad_labels_kernel(const float *__restrict__ y, int N, unsigned *bad) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool b = i < N && !(y[i] == 0.f || y[i] == 1.f);
+  const unsigned n = __popc(__ballot_sync(0xffffffffu, b));
+  if ((threadIdx.x & 31) == 0 && n) atomicAdd(bad, n);
+}
+
+int glm_check_labels(const float *y, int N) {
+  unsigned *d = nullptr, h = 0;
+  B2M_CHECK_CUDA(cudaMalloc(&d, sizeof(unsigned)));
+  B2M_CHECK_CUDA(cudaMemset(d, 0, sizeof(unsigned)));
+  if (N > 0) count_bad_labels_kernel<<<(N + 255) / 256, 256>>>(y, N, d);
+  ++g_launches;
+  const cudaError_t e = cudaMemcpy(&h, d, sizeof(unsigned), cudaMemcpyDeviceToHost);
+  cudaFree(d);
+  B2M_CHECK_CUDA(e);
+  if (h) {
+    set_error("GLM class: Bernoulli labels must all be 0 or 1 (" + std::to_string(h) + " of " + std::to_string(N) +
+              " are not)");
+    return 1;
+  }
+  return 0;
+}
+
 int glm_build(GlmModel &g, const float *X, const float *y, int N, int D, bool force_tc16) {
   g.N = N; g.D = D;
   g.N_total = N;
@@ -246,11 +271,12 @@ __global__ void glm_center_final_kernel(const double *__restrict__ part, int Dp,
   beta0[d] = (float)(s / (double)C);
 }
 
-// y0[n] = (y[n] - c) - sum_d X[n, d] beta0[d], float64 accumulation, one warp per observation row
+// y0[n] = (y[n] - c) - sum_d X[n, d] beta0[d], float64 accumulation, one warp per observation row.
+// logit: y0[n] = eta0[n] = c + sum_d X[n, d] beta0[d] instead (padding rows: -inf, see GlmModel::y0).
 __global__ void __launch_bounds__(256) glm_y0_kernel(const float *__restrict__ X, const float *__restrict__ y,
                                                      const float *__restrict__ beta0, int N, int Np, int Dp,
                                                      float loc_const, float *__restrict__ y0,
-                                                     unsigned *__restrict__ y0max_bits) {
+                                                     unsigned *__restrict__ y0max_bits, bool logit) {
   extern __shared__ float sb[];
   for (int d = threadIdx.x; d < Dp; d += blockDim.x) sb[d] = beta0[d];
   __syncthreads();
@@ -268,9 +294,13 @@ __global__ void __launch_bounds__(256) glm_y0_kernel(const float *__restrict__ X
   }
   for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) {
-    const float v = n < N ? (float)(((double)y[n] - (double)loc_const) - acc) : 0.f;
-    y0[n] = v;
-    if (v == v) atomicMax(y0max_bits, __float_as_uint(fabsf(v)));
+    if (logit) {
+      y0[n] = n < N ? (float)((double)loc_const + acc) : -INFINITY;
+    } else {
+      const float v = n < N ? (float)(((double)y[n] - (double)loc_const) - acc) : 0.f;
+      y0[n] = v;
+      if (v == v) atomicMax(y0max_bits, __float_as_uint(fabsf(v)));
+    }
   }
 }
 
@@ -280,7 +310,7 @@ int glm_recenter(GlmModel &g, const float *theta, int64_t C, cudaStream_t st) {
   glm_center_final_kernel<<<(g.Dp + 127) / 128, 128, 0, st>>>(g.center_part, g.Dp, C, g.beta0);
   cudaMemsetAsync(g.y0max_bits, 0, sizeof(unsigned), st);
   glm_y0_kernel<<<(g.Np + 7) / 8, 256, sizeof(float) * g.Dp, st>>>(g.X, g.y, g.beta0, g.N, g.Np, g.Dp, g.loc_const, g.y0,
-                                                                   g.y0max_bits);
+                                                                   g.y0max_bits, g.lik == kLikLogit);
   g_launches += 3;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -337,6 +367,7 @@ PackP make_pack(const GlmModel &g) {
   P.Dtot = g.Dtot; P.beta_off = g.beta_off; P.D = g.D; P.Dp = g.Dp; P.sigma_param = g.sigma_param;
   P.sigma_const = g.sigma_const; P.weight = g.weight;
   P.inv_col_scale = g.inv_col_scale; P.y0max_bits = g.y0max_bits; P.x_rownorm_max = g.x_rownorm_max;
+  P.logit = g.lik == kLikLogit ? 1 : 0;
   P.Bh = g.B16h; P.Bl = g.B16l;
   P.inv_var = g.inv_var; P.a_unscale = g.a_unscale; P.r_scale = g.r_scale; P.r_unscale = g.r_unscale;
   P.n_peers = 0;
@@ -347,12 +378,14 @@ PackP make_pack(const GlmModel &g) {
 // C[m, n] = sum_k A[m, k] * Bm[n, k]; both operands K-major; all dimensions padded to the tile.
 constexpr int TM = 64, TN = 64, TK = 16;
 
-template <bool RESID>
+// RESID && LOGIT: the Bernoulli-logit epilogue; y = labels, eta0 = c + X beta0 (GlmModel::y0)
+template <bool RESID, bool LOGIT = false>
 __global__ void __launch_bounds__(256) simt_gemm_kernel(const float *__restrict__ A, const float *__restrict__ Bm,
                                                         int K, int lda, int ldb, float *__restrict__ Cout, int ldc,
                                                         const float *__restrict__ y, const float *__restrict__ inv_var,
                                                         float *__restrict__ ss_part, int64_t Cp, int N_valid,
-                                                        float loc_const, float weight) {
+                                                        float loc_const, float weight,
+                                                        const float *__restrict__ eta0 = nullptr) {
   __shared__ float sA[TK][TM + 4], sB[TK][TN + 4];
   const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
   const int m0 = blockIdx.y * TM, n0 = blockIdx.x * TN;
@@ -378,18 +411,26 @@ __global__ void __launch_bounds__(256) simt_gemm_kernel(const float *__restrict_
   }
   if (RESID) {
     // epilogue: z = y - c - M ; R = w z / sigma^2 ; per-row partial sum of z^2 over this column tile
+    // logit:    eta = eta0 + M ; R = w (y - sigmoid(eta)) ; partial sum of y eta - softplus(eta) (padding adds 0)
     __shared__ float red[TM][17];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int m = m0 + ty * 4 + i;
-      const float iv = inv_var[m] * weight;
+      const float iv = LOGIT ? weight : inv_var[m] * weight;
       float s = 0.f;
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int n = n0 + tx * 4 + j;
-        const float z = (n < N_valid) ? (y[n] - loc_const) - acc[i][j] : 0.f;
-        s = fmaf(z, z, s);
-        acc[i][j] = z * iv;
+        if (LOGIT) {
+          float lp, dt;
+          bernoulli_logit(y[n] != 0.f, eta0[n] + acc[i][j], lp, dt);
+          s += lp;
+          acc[i][j] = dt * iv;
+        } else {
+          const float z = (n < N_valid) ? (y[n] - loc_const) - acc[i][j] : 0.f;
+          s = fmaf(z, z, s);
+          acc[i][j] = z * iv;
+        }
       }
       *reinterpret_cast<float4 *>(Cout + (int64_t)m * ldc + n0 + tx * 4) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
       red[ty * 4 + i][tx] = s;
@@ -411,8 +452,12 @@ __global__ void __launch_bounds__(256) simt_gemm_kernel(const float *__restrict_
 
 int simt_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   dim3 grid(g.Np / TN, (unsigned)(Cp / TM));
-  simt_gemm_kernel<true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, g.R, g.Np, g.y0, g.inv_var, g.ss_part, Cp,
-                                                g.N, 0.f, g.weight);
+  if (g.lik == kLikLogit)
+    simt_gemm_kernel<true, true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, g.R, g.Np, g.y, g.inv_var, g.ss_part,
+                                                       Cp, g.N, 0.f, g.weight, g.y0);
+  else
+    simt_gemm_kernel<true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, g.R, g.Np, g.y0, g.inv_var, g.ss_part, Cp,
+                                                  g.N, 0.f, g.weight);
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -449,6 +494,8 @@ __global__ void __launch_bounds__(256) glm_reduce_kernel(const float *__restrict
 }
 
 int glm_set_comm(GlmModel &g, Comm *c, cudaStream_t st) {
+  B2M_REQUIRE(!c || g.lik == kLikNormal,
+              "observation sharding is defined for the Normal likelihood of the GLM class only (use chain sharding)");
   g.comm = c;
   g.N_total = g.N;
   if (!c) return 0;
@@ -498,6 +545,7 @@ FinishP make_finish(const GlmModel &g, int64_t Cp, bool with_grad) {
   F.has_prior = g.has_prior ? 1 : 0;
   F.Dtot = g.Dtot; F.beta_off = g.beta_off; F.D = g.D; F.Dp = g.Dp; F.sigma_param = g.sigma_param;
   F.sigma_const = g.sigma_const; F.weight = g.weight; F.N = (int)g.N_total;
+  F.logit = g.lik == kLikLogit ? 1 : 0;
   F.n_tiles = g.use_tc ? g.Np / 128 : g.Np / TN;   // tcgen05: 256-wide tiles, two column halves each
   F.ss_part = g.ss_part; F.G = g.G; F.g_splits = with_grad ? (g.use_tc ? g.g_splits : 1) : 0; F.Cp = Cp;
   F.r_unscale = g.use_tc == 2 ? g.r_unscale : nullptr;

@@ -1,8 +1,12 @@
-// GLM-class models: log p(theta) = priors(theta) + w * sum_n Normal(y_n | c + (X @ beta)_n, sigma)
-// with beta a slice of theta and sigma a constant or a scalar parameter.
+// GLM-class models: log p(theta) = priors(theta) + w * sum_n L(y_n | eta_n = c + (X @ beta)_n) with beta a slice of theta
+// and one of two likelihood kinds (GlmModel::lik):
+//     kLikNormal  Normal(y_n | eta_n, sigma), sigma a constant or a scalar parameter
+//     kLikLogit   Bernoulli(y_n | logits = eta_n), labels y_n in {0, 1}
 //
 // The gradient of the likelihood is two dense contractions shared by all chains of a lock-step batch:
-//     M = B X^T     [C, D] x [D, N]   -> residual epilogue  R = w (y - c - M) / sigma_c^2,  ss_c = sum_n (y - c - M)^2
+//     M = B X^T     [C, D] x [D, N]   -> residual epilogue, per element
+//                                        Normal: R = w (y - c - M) / sigma_c^2,  ss_c += (y - c - M)^2
+//                                        logit:  R = w (y - sigmoid(c + M)),     ss_c += y eta - softplus(eta)
 //     G = R X       [C, N] x [N, D]
 // (K5 / K6 of SURVEY.md 2b).  Two implementations sit behind the same interface:
 //   * fp32 SIMT tiles (glm_simt.cu)    -- any shape, the validation path
@@ -27,6 +31,7 @@ int comm_allreduce_i64(Comm *c, int64_t *buf, int64_t n, cudaStream_t st);
 int comm_allreduce_f32_max(Comm *c, float *buf, int64_t n, cudaStream_t st);
 
 constexpr int kCenterSlices = 32;  // chain slices of the deterministic two-stage mean (glm.cu, centring)
+constexpr int kLikNormal = 0, kLikLogit = 1;   // GlmModel::lik
 constexpr int kMaxPeers = 8;       // ranks of one NVSwitch box
 
 // The peer window of observation sharding with sliced state (include/b200mcmc.h, B2M_SLICE_PEER).  Every rank owns one
@@ -56,20 +61,23 @@ struct GlmModel {
   int Np = 0, Dp = 0;      // padded: Np % 256 == 0, Dp % 64 == 0 (zero padded)
   int Dtot = 0;            // full parameter count
   int beta_off = 0;        // beta = theta[beta_off : beta_off + D]
-  int sigma_param = -1;    // index of sigma in theta, or -1 when constant
+  int sigma_param = -1;    // index of sigma in theta, or -1 when constant (always -1 for kLikLogit)
   float sigma_const = 1.f, loc_const = 0.f, weight = 1.f;
+  int lik = kLikNormal;    // likelihood kind
   // observed data in HBM (owned by the handle)
   float *X = nullptr, *XT = nullptr;                         // [Np, Dp], [Dp, Np] fp32
   float *Xh = nullptr, *Xl = nullptr, *XTh = nullptr, *XTl = nullptr;  // tf32 hi / lo splits
-  float *y = nullptr;                                        // [Np]
+  float *y = nullptr;                                        // [Np] observations / labels (padding: 0)
   // fp16 hi/lo encoding (use_tc == 2): X' = X * col_scale[d] (power of two, column maximum just below 2^14) split
   // into two halves, hi = fp16(x'), lo = fp16(x' - hi); same for the transposed copy
   __half *X16h = nullptr, *X16l = nullptr, *XT16h = nullptr, *XT16l = nullptr;
   float *col_scale = nullptr, *inv_col_scale = nullptr;      // [Dp]
   float *colmax = nullptr;                                   // [Dp] column maxima of |X| the scales were derived from
   float x_rownorm_max = 0.f;                                 // max_n ||X_n||_2: Cauchy-Schwarz bound of |(X delta)_n|
-  unsigned *y0max_bits = nullptr;                            // device scalar: max_n |y0_n| as float bits (per recentre)
-  // centring (glm.cu): beta0 = mean current position of the batch, y0 = y - c - X beta0 (float64 accumulation)
+  unsigned *y0max_bits = nullptr;                            // device scalar: max_n |y0_n| as float bits (per recentre, Normal)
+  // centring (glm.cu): beta0 = mean current position of the batch, float64 accumulation of
+  //   Normal: y0 = y - c - X beta0        logit: y0 = eta0 = c + X beta0 (padding columns: -inf, which makes their
+  //   log-likelihood and residual exactly zero in the epilogues without a per-element test)
   float *y0 = nullptr, *beta0 = nullptr;                     // [Np], [Dp]
   double *center_part = nullptr;                             // [32, Dp]
   // prior terms (everything except the matvec likelihood) as a pointwise term table
@@ -84,7 +92,8 @@ struct GlmModel {
   float *a_unscale = nullptr, *r_scale = nullptr, *r_unscale = nullptr;   // [cap] per-row scales of the two A operands
   float *G = nullptr;                                        // [g_splits_cap, cap, Dp] split-K partials of the gradient
   int g_splits = 1, g_splits_cap = 1;
-  float *ss_part = nullptr;                                  // [Np / 64, cap] per-column-tile partial sum of squares
+  float *ss_part = nullptr;                                  // [Np / 64, cap] per-column-tile partial sum of squares (Normal)
+                                                             // or of the Bernoulli log-likelihood terms (logit)
   float *inv_var = nullptr;                                  // [cap]
   int use_tc = 0;                                            // 0: SIMT fp32 tiles, 1: tcgen05 3xTF32, 2: tcgen05 3xFP16
   // sampler workspace (glm_samplers.cu): one arena reused across calls, plus a pinned host flag

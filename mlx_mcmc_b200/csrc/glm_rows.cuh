@@ -32,6 +32,7 @@ struct PackP {
   const float *inv_col_scale;
   const unsigned *y0max_bits;
   float x_rownorm_max;
+  int logit;              // GlmModel::lik == kLikLogit: |R| <= |w|, the row scale of R needs no data bound
   __half *Bh, *Bl;        // [Cp, Dp]
   float *inv_var, *a_unscale, *r_scale, *r_unscale;   // [Cp]
   // peer window (sliced observation sharding): the row is written into every rank's window instead, with the row
@@ -45,7 +46,8 @@ struct PackP {
 //   delta'_d = (beta_d - beta0_d) / col_scale_d          (X' = X col_scale, so delta' . X' = delta . X exactly)
 //   row scale s_a = 2^k putting max_d |delta'_d| just below 2^14; hi / lo halves of delta' s_a
 // and the row scale of the residual operand of K6 from a bound that is known before K5 runs:
-//   |z_n| = |y0_n - (X delta)_n| <= max|y0| + ||delta||_2 max_n ||X_n||_2      (Cauchy-Schwarz)
+//   Normal: |z_n| = |y0_n - (X delta)_n| <= max|y0| + ||delta||_2 max_n ||X_n||_2      (Cauchy-Schwarz)
+//   logit:  |R_n| = |w| |y_n - sigmoid(eta_n)| <= |w|
 __device__ __forceinline__ void pack16_row(const PackP &P, const float *__restrict__ th, int64_t row, int lane) {
   const bool live = th != nullptr;
   B2M_ASSERT(row >= 0 && P.Dp % 64 == 0 && P.D <= P.Dp && P.beta_off + P.D <= P.Dtot);
@@ -82,7 +84,8 @@ __device__ __forceinline__ void pack16_row(const PackP &P, const float *__restri
     }
     if (lane == 0) {
       P.inv_var[row] = iv;
-      const float bound = (__uint_as_float(*P.y0max_bits) + sqrtf(n2) * P.x_rownorm_max) * fabsf(iv * P.weight);
+      const float bound = P.logit ? fabsf(P.weight)
+                                  : (__uint_as_float(*P.y0max_bits) + sqrtf(n2) * P.x_rownorm_max) * fabsf(iv * P.weight);
       const float sr = pow2_scale(bound);
       P.a_unscale[row] = 1.0f / sa;
       P.r_scale[row] = sr;
@@ -114,7 +117,8 @@ struct FinishP {
   int Dtot, beta_off, D, Dp, sigma_param;
   float sigma_const, weight;
   int N;                 // observations of the whole model (all shards)
-  int n_tiles;           // partial sums of z^2 per row
+  int logit;             // GlmModel::lik == kLikLogit: the partial sums are the log-likelihood itself, no sigma
+  int n_tiles;           // partial sums of z^2 (or of the Bernoulli terms) per row
   const float *ss_part;  // [n_tiles, Cp]
   const float *G;        // [g_splits, Cp, Dp]
   int g_splits;
@@ -143,7 +147,7 @@ __device__ __forceinline__ void finish_row(const FinishP &F, const SModel &sm, c
   const float sg = sigma_param >= 0 ? th[sigma_param] : F.sigma_const;
   const float iv = 1.0f / (sg * sg);
   const float weight = F.weight;
-  float lp = weight * ((float)F.N * (-kHalfLog2Pi - logf(sg)) - 0.5f * ss * iv);
+  float lp = F.logit ? weight * ss : weight * ((float)F.N * (-kHalfLog2Pi - logf(sg)) - 0.5f * ss * iv);
   // One warp per chain: with a scalar loop over d the warp walks D / 32 dependent iterations (80-120 us at D = 1000
   // whatever the number of chains: latency bound).  When the layout allows, each lane takes four consecutive
   // coefficients and all split-K partials of an iteration are independent 16-byte loads.

@@ -24,6 +24,8 @@
 //               fp32 master accumulators in registers (lane = output row, 8 warps = 4 lane quarters x 2 column
 //               halves).  At the end:
 //                 RESID: z = y - c - acc, per-row sum z^2, R = w z / sigma^2 split into tf32 hi/lo   (K5)
+//                 LOGIT: eta = eta0 + acc, per-row sum of y eta - softplus(eta), R = w (y - sigmoid(eta))
+//                        (K5 of the Bernoulli-logit likelihood, same transposition and stores as RESID)
 //                 PLAIN: store the split-K partial of G                                              (K6)
 #include <cuda.h>
 #include <cuda_fp16.h>
@@ -222,6 +224,8 @@ struct EpiParams {
   int push_own, push_rank;
   const float *r_unscale;       // [Cp]
   const float *inv_col_scale;   // [Dp]
+  // LOGIT (last, so that the parameter offsets of the other modes stay where they were)
+  const float *eta0;      // [Np] c + X beta0 (float64-accumulated centring, padding -inf); `y` holds the labels
 };
 
 template <int BLOCK_N, int NCTA>
@@ -235,7 +239,8 @@ struct Cfg {
   static constexpr int COLS_PER_WARP = BLOCK_N / 2;    // each promotion warp owns 32 rows x half of the columns
 };
 
-// MODE: 0 = PLAIN (split-K partial of G), 1 = RESID (K5 residual epilogue), 2 = PUSH (K6 tile -> owner's window)
+// MODE: 0 = PLAIN (split-K partial of G), 1 = RESID (K5 residual epilogue), 2 = PUSH (K6 tile -> owner's window),
+//       3 = LOGIT (K5 with the Bernoulli-logit residual epilogue)
 template <int BLOCK_N, int MODE, int NCTA, bool F16>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
@@ -243,7 +248,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
                int k_blocks_per_split, int CHUNK_KB, int mma_mask, int Tm, int Tn, int n_tiles, const __grid_constant__ EpiParams E) {
   if (E.skip_flag && *reinterpret_cast<const volatile int *>(E.skip_flag) >= E.skip_target) return;   // uniform over the grid
   using C = Cfg<BLOCK_N, NCTA>;
-  constexpr bool RESID = MODE == 1, PUSH = MODE == 2;
+  constexpr bool LOGIT = MODE == 3, RESID = MODE == 1 || LOGIT, PUSH = MODE == 2;
   constexpr int BLOCK_K = Enc<F16>::BLOCK_K;   // K elements per k-block (shadows the tf32 constant)
   constexpr int SCRATCH_BYTES = (RESID || PUSH) ? NUM_EPI_WARPS * 32 * 33 * 4 : 0;   // per-warp transpose scratch of the epilogue
   extern __shared__ unsigned char smem_raw[];
@@ -410,8 +415,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
       // partial-sector writes -- the first version spent more time here than in the MMAs).  Each warp therefore
       // transposes 32x32 blocks through a private shared-memory scratch (33-float pitch: conflict-free both ways)
       // and stores whole 128-byte row segments.
-      float ss = 0.f;
-      const float ivw = E.inv_var[m] * E.weight;
+      float ss = 0.f;   // Normal: sum z^2; LOGIT: sum of the Bernoulli log-likelihood terms
+      const float ivw = LOGIT ? E.weight : E.inv_var[m] * E.weight;
       // F16: the accumulators carry the row scale of the A operand (delta); R gets its own row scale before the split
       const float a_un = F16 ? E.a_unscale[m] : 1.0f;
       const float rs_lane = F16 ? E.r_scale[m] : 1.0f;   // lane r holds the R scale of row r of this warp's 32 rows
@@ -419,23 +424,40 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
       const int64_t row0 = (int64_t)(m0 + q * 32);
       // the observations of this warp's columns: one coalesced load per 32-column block (lane = column), handed to
       // the row-owning threads by shuffle (a per-element __ldg serialised 128 L2 round trips per thread)
-      float yv[CW / 32];
+      float yv[CW / 32], ev[LOGIT ? CW / 32 : 1];
 #pragma unroll
       for (int b = 0; b < CW / 32; ++b) {
         const int n = nb + b * 32 + lane;
-        yv[b] = (n < E.N_valid) ? __ldg(E.y + n) - E.loc_const : 0.f;
+        if (LOGIT) {   // labels and eta0: both arrays are Np long, the padding needs no test (eta0 = -inf there)
+          yv[b] = __ldg(E.y + n);
+          ev[b] = __ldg(E.eta0 + n);
+        } else {
+          yv[b] = (n < E.N_valid) ? __ldg(E.y + n) - E.loc_const : 0.f;
+        }
       }
-      // (columns n >= N_valid need no test below: the padded rows of X are zero, so acc = 0 there, and yv = 0)
+      // (columns n >= N_valid need no test below: the padded rows of X are zero, so acc = 0 there, and yv = 0; LOGIT:
+      // label 0 and eta = -inf give a zero term and a zero residual)
 #pragma unroll
       for (int b = 0; b < CW / 32; ++b) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const float yj = __shfl_sync(0xffffffffu, yv[b], j);
-          const float z = yj - (F16 ? acc[b * 32 + j] * a_un : acc[b * 32 + j]);
-          ss = fmaf(z, z, ss);
+          const float xd = F16 ? acc[b * 32 + j] * a_un : acc[b * 32 + j];
+          float r;
+          if (LOGIT) {
+            // one exp(-|eta|) feeds softplus and sigmoid (bernoulli_logit, model.cuh)
+            float lp, dt;
+            bernoulli_logit(yj != 0.f, __shfl_sync(0xffffffffu, ev[b], j) + xd, lp, dt);
+            ss += lp;
+            r = dt * ivw;
+          } else {
+            const float z = yj - xd;
+            ss = fmaf(z, z, ss);
+            r = z * ivw;
+          }
           // F16: the row scale of R is applied here, by the thread that owns the row (same two multiplications, in the
           // same order, as scaling after the transposition -- without a shuffle and two multiplies per stored pair)
-          scratch[lane * 33 + j] = F16 ? (z * ivw) * rs_lane : z * ivw;
+          scratch[lane * 33 + j] = F16 ? r * rs_lane : r;
         }
         __syncwarp();
         if (F16) {
@@ -590,7 +612,7 @@ template <int BLOCK_N, int MODE, int NCTA, bool F16>
 int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap &Bh, const CUtensorMap &Bl, dim3 grid,
                 int kb_total, int kb_per_split, const EpiParams &E, cudaStream_t st, int chunk_kb, int mma_mask) {
   using C = Cfg<BLOCK_N, NCTA>;
-  constexpr bool RESID = MODE == 1;
+  constexpr bool RESID = MODE == 1 || MODE == 3;
   auto kernel = tc_gemm_kernel<BLOCK_N, MODE, NCTA, F16>;
   constexpr int SMEM = C::SMEM_BYTES + (MODE != 0 ? NUM_EPI_WARPS * 32 * 33 * 4 : 0);
   // per device: the attribute belongs to the function on the current device.  Setting it again is harmless, so a plain
@@ -744,6 +766,8 @@ int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   E.Rl = f16 ? (void *)g.R16l : (void *)g.Rl;
   E.a_unscale = g.a_unscale; E.r_scale = g.r_scale;
   E.N_valid = g.N; E.loc_const = 0.f; E.weight = g.weight;   // y0 is already centred and shifted (glm.cu)
+  const bool logit = g.lik == kLikLogit;
+  if (logit) { E.y = g.y; E.eta0 = g.y0; }   // labels, and the centring c + X beta0
   dim3 grid((unsigned)(Cp / BLOCK_M), g.Np / 256, 1);
   // promotion interval: 128 values of K for tf32; 256 for fp16 -- the MMAs of a tile take half as long there, and the
   // longer chunk lets the issuer run far enough into the next tile to cover the epilogue (measured at C4: 4.28 ->
@@ -752,6 +776,7 @@ int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   // chunk accumulators, so the issuer can then run a WHOLE tile ahead of the residual epilogue instead of half a tile
   // (measured at C4: K5 1.94 -> 1.89 ms; gradient error vs float64 unchanged at 2e-6, full-size test green)
   const int ck = (f16 && g.Dp / bk >= 8) ? 8 : DEFAULT_CHUNK_KB;
+  if (logit) return launch_tc<256, 3>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
   return launch_tc<256, 1>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
 }
 

@@ -197,6 +197,19 @@ struct Elem {
   float lp, dx, d0, d1;
 };
 
+// Bernoulli with logit t and label y (one = y is 1): lp = y t - softplus(t), dt = d lp / dt = y - sigmoid(t), both from one
+// e = exp(-|t|) in (0, 1].  y t - max(t, 0) is 0 when the label agrees with the sign of t and -|t| otherwise, and
+// y - sigmoid(t) is +-sigmoid(-|t|) or +-sigmoid(|t|): no cancellation and no overflow at any |t| (inf included).
+// Shared by the pointwise density below and the residual epilogues of the GLM contractions (glm.cu, glm_tc.cu).
+__device__ __forceinline__ void bernoulli_logit(bool one, float t, float &lp, float &dt) {
+  const float e = expf(-fabsf(t));
+  const float r = 1.0f / (1.0f + e);   // sigmoid(|t|)
+  const bool match = one == (t >= 0.f);
+  lp = (match ? 0.f : -fabsf(t)) - log1pf(e);
+  const float m = match ? e * r : r;
+  dt = one ? m : -m;
+}
+
 template <bool GRAD>
 __device__ __forceinline__ Elem dist_eval(int dist, float x, float p0, float p1, float k0, float k1, float k2) {
   Elem e;
@@ -243,6 +256,16 @@ __device__ __forceinline__ Elem dist_eval(int dist, float x, float p0, float p1,
       if (x > 0.f && x < 1.f) {
         e.lp = (k0 - 1.0f) * logf(x) + (k1 - 1.0f) * logf(1.0f - x) - k2;
         if (GRAD) e.dx = (k0 - 1.0f) / x - (k1 - 1.0f) / (1.0f - x);
+      } else {
+        e.lp = ninf;
+      }
+    } break;
+    case B2M_BERNOULLI: {  // x = label, p0 = logit
+      if (x == 0.f || x == 1.f) {
+        float lp, dt;
+        bernoulli_logit(x == 1.f, p0, lp, dt);
+        e.lp = lp;
+        if (GRAD) e.d0 = dt;
       } else {
         e.lp = ninf;
       }

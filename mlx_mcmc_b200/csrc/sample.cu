@@ -6,6 +6,7 @@
 //   Gamma        gamma.py:90-117        (the reference falls back to numpy's generator; here Marsaglia-Tsang)
 //   Beta         beta.py:93-119         (numpy fallback there; here Ga / (Ga + Gb))
 //   Categorical  categorical.py:95-113  inverse CDF over the normalised probabilities
+//   Bernoulli    (no reference class)   U < p
 // Philox4x32-10, counter = (output index, attempt, slot), key = seed: the i-th output depends only on (seed, i).
 #include <math.h>
 
@@ -57,6 +58,7 @@ __global__ void __launch_bounds__(256) sample_kernel(int dist, float p0, float p
       const float ga = gamma_unit_rate(p0, seed, (uint64_t)i, 0u), gb = gamma_unit_rate(p1, seed, (uint64_t)i, 1u);
       r = ga / (ga + gb);
     } break;
+    case B2M_BERNOULLI: r = u01(Philox::draw(seed, (uint64_t)i, 0u, 0u).x) < p0 ? 1.f : 0.f; break;   // p0 = P(1)
     case SAMPLE_CATEGORICAL: {
       const float u = u01(Philox::draw(seed, (uint64_t)i, 0u, 0u).x);
       int lo = 0, hi = n_cat - 1;   // first k with cdf[k] > u

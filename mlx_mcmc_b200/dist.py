@@ -27,7 +27,7 @@ import numpy as np
 import torch
 import torch.distributed as td
 
-from .tracer import OP_DATA, OP_MATVEC, TracedModel
+from .tracer import NORMAL, OP_DATA, OP_MATVEC, TracedModel
 
 
 # ------------------------------------------------------------------------------------------ partitions
@@ -76,6 +76,9 @@ def shard_observations(traced: TracedModel, rank: int, world: int) -> TracedMode
     if len(lik) != 1:
         raise ValueError("observation sharding supports exactly one X @ beta term")
     t = out.terms[lik[0]]
+    if t.dist != NORMAL:
+        raise ValueError("observation sharding supports the Normal likelihood of the GLM class only; shard the chains "
+                         "(shard='chains') of a Bernoulli (logistic) model instead")
     if t.p0.kind != OP_MATVEC or t.x.kind != OP_DATA:
         raise ValueError("observation sharding needs the form Normal(X @ beta, sigma).log_prob(y)")
     xi, yi = t.p0.a, t.x.a

@@ -35,9 +35,10 @@ class UnsupportedOpError(TypeError):
 
 # distribution / operand tags: keep in sync with include/b200mcmc.h
 NORMAL, HALFNORMAL, EXPONENTIAL, GAMMA, BETA, CONSTANT = range(6)
+BERNOULLI = 7   # not 6: b2m_sample's B2M_SAMPLE_CATEGORICAL is 6, and 6 stays an unknown term tag
 OP_CONST, OP_PARAM, OP_DATA, OP_PARAMVEC, OP_LIN, OP_MATVEC = range(6)
 DIST_NAMES = {NORMAL: "Normal", HALFNORMAL: "HalfNormal", EXPONENTIAL: "Exponential", GAMMA: "Gamma",
-              BETA: "Beta", CONSTANT: "const"}
+              BETA: "Beta", CONSTANT: "const", BERNOULLI: "Bernoulli"}
 
 
 def _is_number(x) -> bool:

@@ -132,6 +132,32 @@ def regression_posterior(meta):
     return m, V
 
 
+def data_logistic(n, d, seed=0):
+    """X ~ N(0, 1) [n, d], beta* ~ N(0, 1/d) (logits of order 1), y ~ Bernoulli(sigmoid(X beta*)) as float32 0 / 1."""
+    rng = np.random.default_rng(seed)
+    X = rng.standard_normal((n, d), dtype=np.float32)
+    beta = (rng.standard_normal(d) / np.sqrt(d)).astype(np.float32)
+    eta = X.astype(np.float64) @ beta.astype(np.float64)
+    y = (rng.uniform(size=n) < 1.0 / (1.0 + np.exp(-eta))).astype(np.float32)
+    return X, y, beta
+
+
+def logistic_regression(ns, n, d, seed=0, prior_scale=10.0):
+    """Bayesian logistic regression: log p = sum Normal(0, prior_scale)(beta) + sum Bernoulli(logits = X @ beta)(y).
+    Same design-matrix shape as `regression`, so it runs on the same GLM contractions with the Bernoulli-logit
+    epilogue."""
+    mx, Normal, Bernoulli = ns.mx, ns.Normal, ns.Bernoulli
+    X, y, beta_true = data_logistic(n, d, seed)
+    Xa, ya = mx.array(X), mx.array(y)
+
+    def log_prob(params):
+        beta = params["beta"]
+        return mx.sum(Normal(0, prior_scale).log_prob(beta)) + mx.sum(Bernoulli(logits=Xa @ beta).log_prob(ya))
+
+    meta = SimpleNamespace(name=f"logistic_{d}x{n}", D=d, N=n, X=X, y=y, beta_true=beta_true, prior_scale=prior_scale)
+    return log_prob, {"beta": np.zeros(d, dtype=np.float32)}, meta
+
+
 # small models taken from the reference's own sampler tests -------------------------------
 def t_normal_1d(ns, loc=5.0, scale=2.0):
     """tests/test_nuts.py:13-17, tests/test_hmc.py:13-20."""
