@@ -108,12 +108,19 @@ enum { B2M_TF_NONE = 0, B2M_TF_LOG = 1, B2M_TF_LOGIT = 2 };
 /* arithmetic of the two GLM contractions / evaluation path of pointwise models (were environment variables in ABI 1) */
 enum { B2M_GLM_AUTO = 0, B2M_GLM_SIMT = 1, B2M_GLM_TC = 2, B2M_GLM_TC16 = 3 };
 enum { B2M_POINTWISE_AUTO = 0, B2M_POINTWISE_GENERAL = 1 };
+/* evaluation form of the GLM likelihood (DESIGN.md 4.2).  STREAM: two contractions over X per evaluation (B X^T with
+ * the residual epilogue, then R X).  GRAM: one [C, D] x [D, D] contraction against X^T X, precomputed in float64 when
+ * the model is created -- the Normal likelihood on the tensor-core paths only.  AUTO picks GRAM for a Normal likelihood
+ * on a tensor-core path with N >= 2 D and D <= 4096 (padded), else STREAM.  Observation sharding (b2m_model_set_comm)
+ * switches an AUTO model to STREAM; forcing GRAM where it cannot run is an error. */
+enum { B2M_FORM_AUTO = 0, B2M_FORM_STREAM = 1, B2M_FORM_GRAM = 2 };
 
 typedef struct {
   int32_t glm_path;          /* B2M_GLM_*: AUTO = tcgen05 3xFP16 when the data's dynamic range allows, else 3xTF32 */
   int32_t pointwise_path;    /* B2M_POINTWISE_*: AUTO = compact (registers + constant bank) when the model allows */
   const int32_t *transforms; /* HOST array [D] of B2M_TF_*, or NULL (= the reference: no transforms) */
-  int32_t reserved[4];       /* must be zero */
+  int32_t glm_form;          /* B2M_FORM_*: evaluation form of a GLM-class model with a Normal likelihood, see below */
+  int32_t reserved[3];       /* must be zero */
 } b2m_model_options;
 
 /* ---- sampler arguments ---- */
@@ -260,6 +267,8 @@ int b2m_model_class(const b2m_model *m);
  * by powers of two into fp16's range, chosen automatically unless the data's dynamic range is too wide); -1 otherwise.
  * b2m_model_options.glm_path forces one. */
 int b2m_model_glm_path(const b2m_model *m);
+/* GLM class: evaluation form in use -- 1 streaming, 2 Gram (B2M_FORM_*); -1 otherwise */
+int b2m_model_glm_form(const b2m_model *m);
 
 /* log p(theta_c) and d/dtheta for C chains.  Replaces mx.grad(log_prob_flat)(*params) plus the
  * separate value call in hamiltonian() (kernels/hmc.py:53-67,102-111).  grad may be NULL. */

@@ -33,7 +33,7 @@ class Array(C.Structure):
 
 class ModelOptions(C.Structure):
     _fields_ = [("glm_path", C.c_int32), ("pointwise_path", C.c_int32), ("transforms", C.POINTER(C.c_int32)),
-                ("reserved", C.c_int32 * 4)]
+                ("glm_form", C.c_int32), ("reserved", C.c_int32 * 3)]
 
 
 class HmcArgs(C.Structure):
@@ -73,11 +73,13 @@ TF_NONE, TF_LOG, TF_LOGIT = 0, 1, 2
 GLM_AUTO, GLM_SIMT, GLM_TC, GLM_TC16 = 0, 1, 2, 3
 GLM_PATHS = {"auto": GLM_AUTO, "simt": GLM_SIMT, "tc": GLM_TC, "tc16": GLM_TC16}
 POINTWISE_AUTO, POINTWISE_GENERAL = 0, 1
+FORM_AUTO, FORM_STREAM, FORM_GRAM = 0, 1, 2
+GLM_FORMS = {"auto": FORM_AUTO, "stream": FORM_STREAM, "gram": FORM_GRAM}
 MAX_TREE_DEPTH = 12
 ABI_VERSION = 4
 
 EXPORTS = ["b2m_last_error", "b2m_abi_version", "b2m_struct_sizes", "b2m_model_create", "b2m_model_destroy",
-           "b2m_model_dim", "b2m_model_class", "b2m_model_glm_path", "b2m_logp_grad", "b2m_hmc_run", "b2m_mh_run", "b2m_nuts_run",
+           "b2m_model_dim", "b2m_model_class", "b2m_model_glm_path", "b2m_model_glm_form", "b2m_logp_grad", "b2m_hmc_run", "b2m_mh_run", "b2m_nuts_run",
            "b2m_launch_count", "b2m_comm_unique_id", "b2m_comm_init", "b2m_comm_destroy", "b2m_model_set_comm",
            "b2m_comm_allreduce_f32", "b2m_profile", "b2m_profile_read", "b2m_diag_series", "b2m_diag_params", "b2m_sample",
            "b2m_options_size", "b2m_peer_alloc", "b2m_peer_open", "b2m_peer_close", "b2m_peer_free", "b2m_model_peer_bytes",
@@ -137,6 +139,7 @@ def load(build_if_missing: bool = True):
     lib.b2m_model_dim.argtypes = [c_p]
     lib.b2m_model_class.argtypes = [c_p]
     lib.b2m_model_glm_path.argtypes = [c_p]
+    lib.b2m_model_glm_form.argtypes = [c_p]
     lib.b2m_logp_grad.argtypes = [c_p, c_p, C.c_int64, c_p, c_p, C.c_int32, c_p]
     lib.b2m_hmc_run.argtypes = [c_p, C.POINTER(HmcArgs), c_p]
     lib.b2m_mh_run.argtypes = [c_p, C.POINTER(MhArgs), c_p]

@@ -100,7 +100,7 @@ static int check_operand(const b2m_operand &o, int length, int D, int n_lin, con
 // GLM class: exactly one likelihood over X @ beta (+ const) and an observed vector y -- a Normal with X @ beta as its
 // location and a constant or scalar-parameter scale, or a Bernoulli with X @ beta as its logits and labels y in {0, 1};
 // every other term is a pointwise prior.
-static int setup_glm(b2m_model *m, int D, int glm_path, const int32_t *tf) {
+static int setup_glm(b2m_model *m, int D, int glm_path, int glm_form, const int32_t *tf) {
   int lik = -1;
   for (size_t t = 0; t < m->terms.size(); ++t) {
     const b2m_term &T = m->terms[t];
@@ -131,6 +131,7 @@ static int setup_glm(b2m_model *m, int D, int glm_path, const int32_t *tf) {
   // b2m_model_options.glm_path: SIMT (fp32 FMA tiles) | TC (tcgen05 3xTF32) | TC16 (tcgen05 3xFP16 with scaled operands);
   // AUTO: the fp16 encoding when the data's dynamic range allows it (checked in glm_build), else tf32
   g.use_tc = (!b2m::tc_available() || glm_path == B2M_GLM_SIMT) ? 0 : (glm_path == B2M_GLM_TC ? 1 : 2);
+  g.form_req = glm_form;   // resolved in glm_build once the encoding is known
   if (tf) {   // constraint transforms: device copy of the per-parameter codes (before any workspace is reserved)
     bool any = false;
     for (int d = 0; d < D; ++d) any = any || tf[d] != B2M_TF_NONE;
@@ -236,7 +237,8 @@ int b2m_model_create(const b2m_term *terms, int32_t n_terms, const b2m_lin_entry
   B2M_REQUIRE(o.glm_path >= B2M_GLM_AUTO && o.glm_path <= B2M_GLM_TC16, "b2m_model_create: unknown glm_path");
   B2M_REQUIRE(o.pointwise_path == B2M_POINTWISE_AUTO || o.pointwise_path == B2M_POINTWISE_GENERAL,
               "b2m_model_create: unknown pointwise_path");
-  for (int i = 0; i < 4; ++i) B2M_REQUIRE(o.reserved[i] == 0, "b2m_model_create: reserved option fields must be zero");
+  B2M_REQUIRE(o.glm_form >= B2M_FORM_AUTO && o.glm_form <= B2M_FORM_GRAM, "b2m_model_create: unknown glm_form");
+  for (int i = 0; i < 3; ++i) B2M_REQUIRE(o.reserved[i] == 0, "b2m_model_create: reserved option fields must be zero");
   if (o.transforms)
     for (int d = 0; d < D; ++d)
       B2M_REQUIRE(o.transforms[d] >= B2M_TF_NONE && o.transforms[d] <= B2M_TF_LOGIT, "b2m_model_create: unknown transform code");
@@ -320,7 +322,7 @@ int b2m_model_create(const b2m_term *terms, int32_t n_terms, const b2m_lin_entry
   // observation vectors are staged in shared memory when they fit beside the mailboxes
   m->km.stage_floats = (stage * 4 <= 96 * 1024) ? (int32_t)stage : 0;
   if (m->model_class == 1) {
-    if (int rc = setup_glm(m, D, o.glm_path, o.transforms)) {
+    if (int rc = setup_glm(m, D, o.glm_path, o.glm_form, o.transforms)) {
       b2m_model_destroy(m);
       return rc;
     }
@@ -356,6 +358,7 @@ int b2m_model_has_module(const b2m_model *m) { return (m && m->jit) ? 1 : 0; }
 int b2m_model_dim(const b2m_model *m) { return m ? m->km.D : -1; }
 int b2m_model_class(const b2m_model *m) { return m ? m->model_class : -1; }
 int b2m_model_glm_path(const b2m_model *m) { return (m && m->model_class == 1) ? m->glm.use_tc : -1; }
+int b2m_model_glm_form(const b2m_model *m) { return (m && m->model_class == 1) ? m->glm.form : -1; }
 
 int b2m_logp_grad(b2m_model *m, const float *theta, int64_t n_chains, float *logp, float *grad, int32_t lanes,
                   void *stream) {
@@ -436,6 +439,7 @@ int b2m_model_peer_attach(b2m_model *m, void *const *windows, int32_t n_ranks, i
   B2M_REQUIRE(n_chains > 0 && n_chains % (128 * (int64_t)n_ranks) == 0 && n_chains % 256 == 0,
               "b2m_model_peer_attach: n_chains must be a multiple of 256 and of 128 x the number of ranks");
   for (int s = 0; s < n_ranks; ++s) B2M_REQUIRE(windows[s] != nullptr, "b2m_model_peer_attach: NULL window");
+  if (int rc = b2m::glm_use_streaming(m->glm, "the peer exchange of observation sharding")) return rc;
   return b2m::glm_peer_attach(m->glm, windows, n_ranks, rank, n_chains, bytes);
 }
 

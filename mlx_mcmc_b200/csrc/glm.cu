@@ -31,6 +31,7 @@ void glm_free(GlmModel &g) {
   FREE(g.y0); FREE(g.beta0); FREE(g.center_part);
   FREE(g.X16h); FREE(g.X16l); FREE(g.XT16h); FREE(g.XT16l); FREE(g.col_scale); FREE(g.inv_col_scale); FREE(g.y0max_bits);
   FREE(g.colmax);
+  FREE(g.G64); FREE(g.gvec); FREE(g.gb); FREE(g.gterm); FREE(g.Gmh); FREE(g.Gml); FREE(g.g_unscale);
   FREE(g.ws);
   FREE(g.tf); FREE(g.blk_counter);
   g.ws_cap = 0;
@@ -48,24 +49,26 @@ int glm_reserve(GlmModel &g, int64_t n_chains) {
   size_t g_rows = (size_t)cp;
   if (g.use_tc)
     for (int64_t c = 128; c <= cp; c += 128) {
-      const size_t need = (size_t)grad_splits(g, c) * (size_t)c;
+      const size_t need = (size_t)contraction_splits(g, c) * (size_t)c;
       if (need > g_rows) g_rows = need;
     }
   g.g_splits_cap = (int)((g_rows + cp - 1) / cp);
-  if (dev_alloc(&g.B, cp * g.Dp) || dev_alloc(&g.G, g_rows * g.Dp) || dev_alloc(&g.ss_part, (size_t)(g.Np / 64) * cp) ||
-      dev_alloc(&g.inv_var, cp) || dev_alloc(&g.red, (size_t)cp * g.Dp + cp))
+  if (dev_alloc(&g.B, cp * g.Dp) || dev_alloc(&g.G, g_rows * g.Dp) || dev_alloc(&g.inv_var, cp) ||
+      dev_alloc(&g.red, (size_t)cp * g.Dp + cp))
     return 2;
   if (g.tf && dev_alloc(&g.thc, (size_t)cp * g.Dtot)) return 2;
+  // the residual operand R [cap, Np] and the per-tile sums exist only in the streaming form (2 x 1.6 GB at C4 in fp16)
+  const bool stream = g.form == kFormStream;
+  if (stream && dev_alloc(&g.ss_part, (size_t)(g.Np / 64) * cp)) return 2;
   if (g.use_tc == 0 && dev_alloc(&g.R, cp * (size_t)g.Np)) return 2;
   if (g.use_tc == 1) {
-    if (dev_alloc(&g.Bh, cp * g.Dp) || dev_alloc(&g.Bl, cp * g.Dp) || dev_alloc(&g.Rh, cp * (size_t)g.Np) ||
-        dev_alloc(&g.Rl, cp * (size_t)g.Np))
-      return 2;
+    if (dev_alloc(&g.Bh, cp * g.Dp) || dev_alloc(&g.Bl, cp * g.Dp)) return 2;
+    if (stream && (dev_alloc(&g.Rh, cp * (size_t)g.Np) || dev_alloc(&g.Rl, cp * (size_t)g.Np))) return 2;
   }
   if (g.use_tc == 2) {
-    if (dev_alloc(&g.B16h, cp * g.Dp) || dev_alloc(&g.B16l, cp * g.Dp) || dev_alloc(&g.R16h, cp * (size_t)g.Np) ||
-        dev_alloc(&g.R16l, cp * (size_t)g.Np) || dev_alloc(&g.a_unscale, cp) || dev_alloc(&g.r_scale, cp) ||
-        dev_alloc(&g.r_unscale, cp))
+    if (dev_alloc(&g.B16h, cp * g.Dp) || dev_alloc(&g.B16l, cp * g.Dp) || dev_alloc(&g.a_unscale, cp)) return 2;
+    if (stream && (dev_alloc(&g.R16h, cp * (size_t)g.Np) || dev_alloc(&g.R16l, cp * (size_t)g.Np) ||
+                   dev_alloc(&g.r_scale, cp) || dev_alloc(&g.r_unscale, cp)))
       return 2;
   }
   g.cap = cp;
@@ -176,6 +179,175 @@ int glm_check_labels(const float *y, int N) {
   return 0;
 }
 
+// ---------------------------------------------------------------- Gram form: statistics (once per model)
+// Gram matrix of the augmented matrix A = [X | y | 1 | 0 ...] ([Np, Da], Da = Dp + 64): column Dp is y, column Dp + 1
+// the indicator of the N real rows, so one pass yields X^T X, X^T y, X^T 1, ||y||^2 and sum y.  Products of fp32 values
+// are exact in float64; only the sums round.  Upper-triangle 64 x 64 tiles (blockIdx.x), each over one slice of the
+// rows (blockIdx.y); the slices are added in a fixed order afterwards.
+constexpr int GT = 64, GK = 16;
+
+__device__ __forceinline__ double aug_at(const float *__restrict__ X, const float *__restrict__ y, int N, int Dp, int n, int d) {
+  if (d < Dp) return (double)X[(int64_t)n * Dp + d];
+  if (d == Dp) return (double)y[n];   // padding rows of y are 0
+  return (d == Dp + 1 && n < N) ? 1.0 : 0.0;
+}
+
+__global__ void __launch_bounds__(256) gram_partial_kernel(const float *__restrict__ X, const float *__restrict__ y, int N,
+                                                           int Np, int Dp, int Da, int rows_per_slice, double *__restrict__ part) {
+  __shared__ double sA[GK][GT], sB[GK][GT];
+  const int nt = Da / GT;
+  int t = blockIdx.x, ti = 0;
+  while (t >= nt - ti) { t -= nt - ti; ++ti; }
+  const int i0 = ti * GT, j0 = (ti + t) * GT;
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  const int n_begin = blockIdx.y * rows_per_slice, n_end = min(n_begin + rows_per_slice, Np);
+  double acc[4][4] = {};
+  for (int n0 = n_begin; n0 < n_end; n0 += GK) {
+    for (int e = threadIdx.x; e < GK * GT; e += 256) {
+      const int r = e / GT, col = e % GT, n = n0 + r;
+      sA[r][col] = n < n_end ? aug_at(X, y, N, Dp, n, i0 + col) : 0.0;
+      sB[r][col] = n < n_end ? aug_at(X, y, N, Dp, n, j0 + col) : 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < GK; ++k) {
+      double a[4], b[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) { a[i] = sA[k][ty + 16 * i]; b[i] = sB[k][tx + 16 * i]; }
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      part[((size_t)blockIdx.y * Da + i0 + ty + 16 * i) * Da + j0 + tx + 16 * j] = acc[i][j];
+}
+
+// G64 (mirrored from the upper tiles: a diagonal tile computes (i, j) and (j, i) from the same products in the same
+// order, so G64 is exactly symmetric) and gvec = X^T y || X^T 1 || ||y||^2 || sum y
+__global__ void gram_final_kernel(const double *__restrict__ part, int S, int Da, int Dp, double *__restrict__ G64,
+                                  double *__restrict__ gvec) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t nG = (int64_t)Dp * Dp;
+  if (i >= nG + 2 * Dp + 2) return;
+  int r, c;
+  if (i < nG) { r = int(i / Dp); c = int(i % Dp); }
+  else {
+    const int k = int(i - nG);
+    if (k < Dp) { r = k; c = Dp; }
+    else if (k < 2 * Dp) { r = k - Dp; c = Dp + 1; }
+    else { r = Dp; c = k == 2 * Dp ? Dp : Dp + 1; }
+  }
+  if (r / GT > c / GT) { const int tmp = r; r = c; c = tmp; }
+  double s = 0.0;
+  for (int z = 0; z < S; ++z) s += part[((size_t)z * Da + r) * Da + c];
+  if (i < nG) G64[i] = s; else gvec[i - nG] = s;
+}
+
+// B operand of the per-leaf contraction, one block per column j of G~ = diag(cs) G diag(cs) (cs = col_scale of the fp16
+// encoding, 1 for tf32).  fp16: column j is scaled by the power of two t_j that puts its maximum just below 2^14 (the
+// entries reach N max|x|^2 otherwise), then split into hi / lo halves; row j of the stored operand = column j (K-major).
+__global__ void __launch_bounds__(256) gram_operand_kernel(const double *__restrict__ G64, int Dp,
+                                                           const float *__restrict__ col_scale, void *Gh, void *Gl,
+                                                           float *__restrict__ g_unscale) {
+  __shared__ double red[256];
+  const int j = blockIdx.x;
+  const double csj = col_scale ? (double)col_scale[j] : 1.0;
+  double m = 0.0;
+  for (int k = threadIdx.x; k < Dp; k += 256) {
+    const double ck = col_scale ? (double)col_scale[k] : 1.0;
+    m = fmax(m, fabs(ck * G64[(int64_t)k * Dp + j] * csj));
+  }
+  red[threadIdx.x] = m;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] = fmax(red[threadIdx.x], red[threadIdx.x + o]);
+    __syncthreads();
+  }
+  const double t = col_scale ? (double)pow2_scale((float)red[0]) : 1.0;
+  for (int k = threadIdx.x; k < Dp; k += 256) {
+    const double ck = col_scale ? (double)col_scale[k] : 1.0;
+    const double v = ck * G64[(int64_t)k * Dp + j] * csj * t;   // powers of two: exact
+    const int64_t o = (int64_t)j * Dp + k;
+    if (col_scale) {
+      const __half hi = __double2half(v);
+      static_cast<__half *>(Gh)[o] = hi;
+      static_cast<__half *>(Gl)[o] = __double2half(v - (double)__half2float(hi));
+    } else {
+      float hi, lo;
+      split_tf32((float)v, hi, lo);
+      static_cast<float *>(Gh)[o] = hi;
+      static_cast<float *>(Gl)[o] = lo;
+    }
+  }
+  if (threadIdx.x == 0 && g_unscale) g_unscale[j] = (float)(1.0 / (csj * t));
+}
+
+static int gram_build(GlmModel &g) {
+  const int Dp = g.Dp, Da = Dp + GT;
+  const size_t dd = (size_t)Dp * Dp;
+  const bool f16 = g.use_tc == 2;
+  if (dev_alloc(&g.G64, dd) || dev_alloc(&g.gvec, 2 * (size_t)Dp + 2) || dev_alloc(&g.gb, (size_t)Dp + 1) ||
+      dev_alloc(&g.gterm, Dp))
+    return 2;
+  B2M_CHECK_CUDA(cudaMalloc(&g.Gmh, dd * (f16 ? 2 : 4)));
+  B2M_CHECK_CUDA(cudaMalloc(&g.Gml, dd * (f16 ? 2 : 4)));
+  if (f16 && dev_alloc(&g.g_unscale, Dp)) return 2;
+  // row slices: about two blocks per SM in all, each slice a whole number of 256-row blocks
+  const int nt = Da / GT, tiles = nt * (nt + 1) / 2;
+  int S = (296 + tiles - 1) / tiles;
+  if (S > g.Np / 256) S = g.Np / 256;
+  if (S < 1) S = 1;
+  const int rows_per_slice = (g.Np / 256 + S - 1) / S * 256;
+  S = (g.Np + rows_per_slice - 1) / rows_per_slice;
+  double *part = nullptr;
+  if (dev_alloc(&part, (size_t)S * Da * Da)) return 2;
+  gram_partial_kernel<<<dim3((unsigned)tiles, (unsigned)S), 256>>>(g.X, g.y, g.N, g.Np, Dp, Da, rows_per_slice, part);
+  const int64_t nf = (int64_t)dd + 2 * Dp + 2;
+  gram_final_kernel<<<(unsigned)((nf + 255) / 256), 256>>>(part, S, Da, Dp, g.G64, g.gvec);
+  gram_operand_kernel<<<Dp, 256>>>(g.G64, Dp, f16 ? g.col_scale : nullptr, g.Gmh, g.Gml, g.g_unscale);
+  g_launches += 3;
+  B2M_CHECK_CUDA(cudaGetLastError());
+  const cudaError_t e = cudaDeviceSynchronize();
+  cudaFree(part);
+  B2M_CHECK_CUDA(e);
+  return 0;
+}
+
+// b2m_model_options.glm_form -> GlmModel::form.  Auto: the Gram form for the Normal likelihood on a tensor-core path when
+// N >= 2 Dp (the per-leaf contraction is then at most a quarter of the streaming form's flops) and Dp <= kGramMaxDp
+// (the Gram arrays stay small).  Observation sharding switches back later (glm_use_streaming).
+static int resolve_form(GlmModel &g) {
+  if (g.form_req == kFormStream) { g.form = kFormStream; return 0; }
+  const bool possible = g.lik == kLikNormal && g.use_tc != 0;
+  if (g.form_req == kFormGram) {
+    B2M_REQUIRE(g.lik == kLikNormal, "glm_form = gram: the Gram form is defined for the Normal likelihood only (the "
+                                     "Bernoulli-logit likelihood has no closed form in X^T X); use 'auto' or 'stream'");
+    B2M_REQUIRE(g.use_tc != 0, "glm_form = gram: the Gram form runs on the tensor-core paths (glm_path 'tc' / 'tc16'), "
+                               "the SIMT path keeps the streaming form");
+    g.form = kFormGram;
+    return 0;
+  }
+  g.form = (possible && (int64_t)g.N >= 2 * (int64_t)g.Dp && g.Dp <= kGramMaxDp) ? kFormGram : kFormStream;
+  return 0;
+}
+
+int glm_use_streaming(GlmModel &g, const char *why) {
+  if (g.form == kFormStream) return 0;
+  if (g.form_req == kFormGram) {
+    set_error(std::string("glm_form = gram: ") + why + " needs the streaming form (create the model with glm_form 'auto' or 'stream')");
+    return 1;
+  }
+  g.form = kFormStream;
+  free_workspace(g);   // the next reservation allocates the residual operand of the streaming form
+  return 0;
+}
+
 int glm_build(GlmModel &g, const float *X, const float *y, int N, int D, bool force_tc16) {
   g.N = N; g.D = D;
   g.N_total = N;
@@ -228,6 +400,8 @@ int glm_build(GlmModel &g, const float *X, const float *y, int N, int D, bool fo
   }
   B2M_CHECK_CUDA(cudaGetLastError());
   B2M_CHECK_CUDA(cudaDeviceSynchronize());
+  if (int rc = resolve_form(g)) return rc;   // after the encoding is final (the Gram operand uses its column scales)
+  if (g.form == kFormGram) return gram_build(g);
   return 0;
 }
 
@@ -304,10 +478,56 @@ __global__ void __launch_bounds__(256) glm_y0_kernel(const float *__restrict__ X
   }
 }
 
+// Gram form: the same centring from the build-time statistics, without reading X (O(Dp^2), float64):
+//     b = X^T y0 = (v - c s1) - G beta0                                 v = X^T y, s1 = X^T 1
+//     q = ||y0||^2 = ||y||^2 - 2 c sum y + N c^2 - beta0 . (2 (v - c s1) - G beta0)
+// q is a difference of large numbers (||y||^2 ~ 1e8 against q ~ 1e5 at C4): harmless in float64, not in float32.
+// One warp per coefficient d: b_d and the term beta0_d (2 (v_d - c s1_d) - (G beta0)_d) of q.
+__global__ void __launch_bounds__(256) gram_center_kernel(const double *__restrict__ G64, const double *__restrict__ gvec,
+                                                          const float *__restrict__ beta0, int Dp, float loc_const,
+                                                          double *__restrict__ gb, double *__restrict__ gterm) {
+  const int lane = threadIdx.x & 31;
+  const int d = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (d >= Dp) return;
+  double u = 0.0;
+  for (int k = lane; k < Dp; k += 32) u = fma(G64[(int64_t)d * Dp + k], (double)beta0[k], u);
+  for (int o = 16; o > 0; o >>= 1) u += __shfl_xor_sync(0xffffffffu, u, o);
+  if (lane == 0) {
+    const double w = gvec[d] - (double)loc_const * gvec[Dp + d];
+    gb[d] = w - u;
+    gterm[d] = (double)beta0[d] * (2.0 * w - u);
+  }
+}
+
+// q = gb[Dp], one block, fixed summation order
+__global__ void __launch_bounds__(256) gram_q_kernel(const double *__restrict__ gvec, const double *__restrict__ gterm,
+                                                     int Dp, int N, float loc_const, double *__restrict__ gb) {
+  __shared__ double sh[256];
+  double s = 0.0;
+  for (int d = threadIdx.x; d < Dp; d += 256) s += gterm[d];
+  sh[threadIdx.x] = s;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const double c = (double)loc_const;
+    gb[Dp] = (gvec[2 * Dp] - 2.0 * c * gvec[2 * Dp + 1] + (double)N * c * c) - sh[0];
+  }
+}
+
 int glm_recenter(GlmModel &g, const float *theta, int64_t C, cudaStream_t st) {
   dim3 gp(g.Dp / 32, kCenterSlices), bp(32, 8);
   glm_center_partial_kernel<<<gp, bp, 0, st>>>(theta, C, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
   glm_center_final_kernel<<<(g.Dp + 127) / 128, 128, 0, st>>>(g.center_part, g.Dp, C, g.beta0);
+  if (g.form == kFormGram) {
+    gram_center_kernel<<<(g.Dp + 7) / 8, 256, 0, st>>>(g.G64, g.gvec, g.beta0, g.Dp, g.loc_const, g.gb, g.gterm);
+    gram_q_kernel<<<1, 256, 0, st>>>(g.gvec, g.gterm, g.Dp, g.N, g.loc_const, g.gb);
+    g_launches += 4;
+    B2M_CHECK_CUDA(cudaGetLastError());
+    return 0;
+  }
   cudaMemsetAsync(g.y0max_bits, 0, sizeof(unsigned), st);
   glm_y0_kernel<<<(g.Np + 7) / 8, 256, sizeof(float) * g.Dp, st>>>(g.X, g.y, g.beta0, g.N, g.Np, g.Dp, g.loc_const, g.y0,
                                                                    g.y0max_bits, g.lik == kLikLogit);
@@ -370,6 +590,7 @@ PackP make_pack(const GlmModel &g) {
   P.logit = g.lik == kLikLogit ? 1 : 0;
   P.Bh = g.B16h; P.Bl = g.B16l;
   P.inv_var = g.inv_var; P.a_unscale = g.a_unscale; P.r_scale = g.r_scale; P.r_unscale = g.r_unscale;
+  if (g.form == kFormGram) { P.y0max_bits = nullptr; P.r_scale = nullptr; P.r_unscale = nullptr; }   // there is no R
   P.n_peers = 0;
   return P;
 }
@@ -496,6 +717,8 @@ __global__ void __launch_bounds__(256) glm_reduce_kernel(const float *__restrict
 int glm_set_comm(GlmModel &g, Comm *c, cudaStream_t st) {
   B2M_REQUIRE(!c || g.lik == kLikNormal,
               "observation sharding is defined for the Normal likelihood of the GLM class only (use chain sharding)");
+  if (c)
+    if (int rc = glm_use_streaming(g, "observation sharding")) return rc;
   g.comm = c;
   g.N_total = g.N;
   if (!c) return 0;
@@ -551,6 +774,14 @@ FinishP make_finish(const GlmModel &g, int64_t Cp, bool with_grad) {
   F.r_unscale = g.use_tc == 2 ? g.r_unscale : nullptr;
   F.inv_col_scale = g.use_tc == 2 ? g.inv_col_scale : nullptr;
   F.tf = g.tf; F.thc = g.thc;
+  if (g.form == kFormGram) {   // the contraction runs for value-only calls too: log p needs delta . (G delta)
+    F.gram = 1;
+    F.g_splits = g.g_splits;
+    F.gb = g.gb; F.beta0 = g.beta0;
+    F.a_unscale = g.use_tc == 2 ? g.a_unscale : nullptr;
+    F.g_unscale = g.use_tc == 2 ? g.g_unscale : nullptr;
+    F.r_unscale = nullptr; F.inv_col_scale = nullptr;
+  }
   return F;
 }
 
@@ -593,7 +824,9 @@ int glm_logp_grad(GlmModel &g, const float *theta, int64_t C, float *logp, float
                                                                     g.sigma_param, g.sigma_const, g.B, g.Bh, g.Bl, g.inv_var);
   }
   ++g_launches;
-  if (g.use_tc) {
+  if (g.use_tc && g.form == kFormGram) {
+    if (int rc = tc_gemm_gram(g, Cp, st)) return rc;   // value-only too (log p needs it)
+  } else if (g.use_tc) {
     if (int rc = tc_gemm_resid(g, Cp, st)) return rc;
     if (grad) if (int rc = tc_gemm_grad(g, Cp, st)) return rc;
   } else {

@@ -32,6 +32,8 @@ int comm_allreduce_f32_max(Comm *c, float *buf, int64_t n, cudaStream_t st);
 
 constexpr int kCenterSlices = 32;  // chain slices of the deterministic two-stage mean (glm.cu, centring)
 constexpr int kLikNormal = 0, kLikLogit = 1;   // GlmModel::lik
+constexpr int kFormStream = 1, kFormGram = 2;   // GlmModel::form (b2m_model_options.glm_form: 0 = auto, 1, 2)
+constexpr int kGramMaxDp = 4096;                // auto picks the Gram form up to this padded width (f64 G: 128 MB)
 constexpr int kMaxPeers = 8;       // ranks of one NVSwitch box
 
 // The peer window of observation sharding with sliced state (include/b200mcmc.h, B2M_SLICE_PEER).  Every rank owns one
@@ -80,6 +82,19 @@ struct GlmModel {
   //   log-likelihood and residual exactly zero in the epilogues without a per-element test)
   float *y0 = nullptr, *beta0 = nullptr;                     // [Np], [Dp]
   double *center_part = nullptr;                             // [32, Dp]
+  // evaluation form (DESIGN.md 4.2).  Streaming: K5 (B X^T + residual epilogue) then K6 (R X), X read twice per leaf.
+  // Gram (Normal likelihood, tensor-core paths, unsharded): with G = X^T X, b = X^T y0, q = ||y0||^2 precomputed,
+  //     X^T (y0 - X delta) = b - G delta,   ||y0 - X delta||^2 = q - 2 delta.b + delta.(G delta)
+  // so one [C, Dp] x [Dp, Dp] contraction per leaf replaces both passes over X.
+  int form = kFormStream;
+  int form_req = 0;                                          // the option as given (0 auto, 1 streaming, 2 Gram)
+  double *G64 = nullptr;                                     // [Dp, Dp] X^T X, float64 sums of exact products
+  double *gvec = nullptr;                                    // [2 Dp + 2] X^T y || X^T 1 || ||y||^2, sum y
+  double *gb = nullptr;                                      // [Dp + 1] b = X^T y0 || q = ||y0||^2 (per recentre)
+  double *gterm = nullptr;                                   // [Dp] per-coefficient terms of q (fixed-order sum)
+  void *Gmh = nullptr, *Gml = nullptr;                       // [Dp, Dp] hi / lo halves of the B operand, row j = column j
+                                                             // of diag(cs) G diag(cs) times t_j (fp16 or tf32 values)
+  float *g_unscale = nullptr;                                // [Dp] 1 / (cs_j t_j)  (fp16 encoding; nullptr for tf32)
   // prior terms (everything except the matvec likelihood) as a pointwise term table
   KModel prior{};
   bool has_prior = false;
@@ -118,6 +133,7 @@ struct GlmModel {
 };
 
 int glm_set_comm(GlmModel &g, Comm *c, cudaStream_t st);
+int glm_use_streaming(GlmModel &g, const char *why);   // observation sharding: back to the streaming form (or refuse)
 
 int glm_reserve(GlmModel &g, int64_t n_chains);
 void glm_free(GlmModel &g);
@@ -138,12 +154,14 @@ int simt_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);    // R -> G
 // tcgen05 implementation (glm_tc.cu)
 int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st);     // B -> R, ss_part
 int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);      // R -> G
+int tc_gemm_gram(GlmModel &g, int64_t Cp, cudaStream_t st);      // B -> G = (beta - beta0) G~  (Gram form)
 bool tc_available();
 void tc_profile(bool enable);
 int tc_profile_read(double *out4);
 int tc_profile_read_n(double *out, int n_kinds);
 void prof_mark(int kind, cudaStream_t st);   // kinds 2 state, 3 peer wait, 4 peer signal: call before and after the launch
-int grad_splits(const GlmModel &g, int64_t Cp);
+int grad_splits(const GlmModel &g, int64_t Cp, int k_blocks);
+int contraction_splits(const GlmModel &g, int64_t Cp);   // split-K of the gradient contraction of the model's form
 
 int tc_gemm_grad_push(GlmModel &g, int64_t Cp, cudaStream_t st);   // K6 whose epilogue stores into the owners' windows
 int glm_finish_launch(GlmModel &g, const float *theta, int64_t C, float *logp, float *grad, cudaStream_t st,

@@ -84,12 +84,14 @@ __device__ __forceinline__ void pack16_row(const PackP &P, const float *__restri
     }
     if (lane == 0) {
       P.inv_var[row] = iv;
-      const float bound = P.logit ? fabsf(P.weight)
-                                  : (__uint_as_float(*P.y0max_bits) + sqrtf(n2) * P.x_rownorm_max) * fabsf(iv * P.weight);
-      const float sr = pow2_scale(bound);
       P.a_unscale[row] = 1.0f / sa;
-      P.r_scale[row] = sr;
-      P.r_unscale[row] = 1.0f / sr;
+      if (P.r_scale) {   // streaming form only: the Gram form has no residual operand
+        const float bound = P.logit ? fabsf(P.weight)
+                                    : (__uint_as_float(*P.y0max_bits) + sqrtf(n2) * P.x_rownorm_max) * fabsf(iv * P.weight);
+        const float sr = pow2_scale(bound);
+        P.r_scale[row] = sr;
+        P.r_unscale[row] = 1.0f / sr;
+      }
     }
   } else {
     // two coefficients per lane and store: 128-byte segments per warp instruction towards every peer over NVLink
@@ -127,7 +129,52 @@ struct FinishP {
   const float *inv_col_scale;  // [Dp] or nullptr
   const int *tf;         // transforms or nullptr
   const float *thc;      // [Cp, Dtot] constrained rows written by pack (tf != nullptr)
+  // Gram form (GlmModel::form): G holds the split-K partials of P = delta G~ instead, ss_part is unused
+  int gram;
+  const double *gb;          // [Dp + 1] b = X^T y0 || q = ||y0||^2 of the current centring
+  const float *beta0;        // [Dp]
+  const float *a_unscale;    // [Cp] 1 / row scale of the packed delta (fp16 encoding) or nullptr
+  const float *g_unscale;    // [Dp] 1 / (cs_j t_j) (fp16 encoding) or nullptr
 };
+
+// Gram form, likelihood part of one row: P = sum of the split-K partials (fixed order), unscaled;
+//     grad_beta = w iv (b - P),   ss = q - 2 delta.b + delta.P   (float64 across the warp, fixed order)
+// with delta = theta_beta - beta0 exactly as pack computed it.  The lane <-> coefficient mapping depends on D only,
+// never on whether a gradient is wanted: a value-only call gets the bit-identical ss.  Returns ss (every lane).
+__device__ __forceinline__ float gram_row(const FinishP &F, const float *__restrict__ th, int64_t c, float ivw,
+                                          float *__restrict__ gr, int lane) {
+  const int D = F.D, Dp = F.Dp, beta_off = F.beta_off;
+  const int64_t stride = F.Cp * (int64_t)Dp;
+  const float *__restrict__ Gr = F.G + c * Dp;
+  const float au = F.a_unscale ? F.a_unscale[c] : 1.0f;
+  const int step = (D & 3) == 0 ? 4 : 1;   // four consecutive coefficients per lane: independent 16-byte loads
+  double acc = 0.0;
+  for (int j0 = step * lane; j0 < D; j0 += 32 * step) {
+    float p[4] = {0.f, 0.f, 0.f, 0.f};
+    if (step == 4) {
+#pragma unroll 4
+      for (int s = 0; s < F.g_splits; ++s) {
+        const float4 t = *reinterpret_cast<const float4 *>(Gr + s * stride + j0);
+        p[0] += t.x; p[1] += t.y; p[2] += t.z; p[3] += t.w;
+      }
+    } else {
+#pragma unroll 4
+      for (int s = 0; s < F.g_splits; ++s) p[0] += Gr[s * stride + j0];
+    }
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      if (e >= step) break;
+      const int j = j0 + e;
+      const float pj = F.g_unscale ? p[e] * (au * F.g_unscale[j]) : p[e];
+      const double bj = F.gb[j];
+      const float dl = __fsub_rn(th[beta_off + j], F.beta0[j]);
+      acc += (double)dl * ((double)pj - 2.0 * bj);
+      if (gr) gr[beta_off + j] = (float)(bj - (double)pj) * ivw;
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  return (float)(F.gb[Dp] + acc);
+}
 
 // Assemble log p and the full gradient of one chain from the contraction outputs.  `c` = row of ss_part / G (and of
 // thc); `th` = the chain's parameter row as the samplers hold it (unconstrained when tf is set); logp / gr = outputs.
@@ -141,17 +188,26 @@ __device__ __forceinline__ void finish_row(const FinishP &F, const SModel &sm, c
   const int Dtot = F.Dtot, D = F.D, Dp = F.Dp, beta_off = F.beta_off, sigma_param = F.sigma_param;
   const int64_t Cp = F.Cp;
   const float *__restrict__ G = F.G;
-  float ss = 0.f;
-  for (int t = lane; t < F.n_tiles; t += 32) ss += F.ss_part[(int64_t)t * Cp + c];
-  for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
   const float sg = sigma_param >= 0 ? th[sigma_param] : F.sigma_const;
   const float iv = 1.0f / (sg * sg);
   const float weight = F.weight;
+  float ss = 0.f;
+  if (F.gram) {
+    ss = gram_row(F, th, c, iv * weight, gr, lane);
+    if (gr) {   // the coordinates outside beta: zero, or the analytic sigma gradient
+      for (int d = lane; d < Dtot; d += 32)
+        if (d < beta_off || d >= beta_off + D) gr[d] = d == sigma_param ? weight * (ss * iv - (float)F.N) / sg : 0.f;
+    }
+    __syncwarp();
+  } else {
+    for (int t = lane; t < F.n_tiles; t += 32) ss += F.ss_part[(int64_t)t * Cp + c];
+    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+  }
   float lp = F.logit ? weight * ss : weight * ((float)F.N * (-kHalfLog2Pi - logf(sg)) - 0.5f * ss * iv);
   // One warp per chain: with a scalar loop over d the warp walks D / 32 dependent iterations (80-120 us at D = 1000
   // whatever the number of chains: latency bound).  When the layout allows, each lane takes four consecutive
   // coefficients and all split-K partials of an iteration are independent 16-byte loads.
-  const bool vec4 = gr && sigma_param < 0 && (Dtot & 3) == 0 && (beta_off & 3) == 0 && (D & 3) == 0 &&
+  const bool vec4 = !F.gram && gr && sigma_param < 0 && (Dtot & 3) == 0 && (beta_off & 3) == 0 && (D & 3) == 0 &&
                     ((reinterpret_cast<uintptr_t>(gr) | reinterpret_cast<uintptr_t>(G)) & 15) == 0;
   if (vec4) {
     const float ru = F.r_unscale ? F.r_unscale[c] : 1.0f;
@@ -173,7 +229,7 @@ __device__ __forceinline__ void finish_row(const FinishP &F, const SModel &sm, c
       *reinterpret_cast<float4 *>(gr + d) = v;
     }
     __syncwarp();
-  } else if (gr) {
+  } else if (gr && !F.gram) {
 #pragma unroll 2
     for (int d = lane; d < Dtot; d += 32) {
       float v = 0.f;

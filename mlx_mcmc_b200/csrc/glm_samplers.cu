@@ -1433,10 +1433,13 @@ int glm_nuts_run_fused(GlmModel &gm, const b2m_nuts_args &a, cudaStream_t st) {
       prof_mark(3, st);
       ++g_launches;
     }
-    if ((rc = tc_gemm_resid(gm, Cp, st))) break;
-    if (!peer) {
+    if (gm.form == kFormGram) {   // one contraction against the Gram operand (never sharded)
+      if ((rc = tc_gemm_gram(gm, Cp, st))) break;
+    } else if (!peer) {
+      if ((rc = tc_gemm_resid(gm, Cp, st))) break;
       if ((rc = tc_gemm_grad(gm, Cp, st))) break;
     } else {
+      if ((rc = tc_gemm_resid(gm, Cp, st))) break;
       if ((rc = tc_gemm_grad_push(gm, Cp, st))) break;
       prof_mark(4, st);
       obs_signal_kernel<<<(unsigned)((Cp + 31) / 32), 256, 0, st>>>(gm.ss_part, gm.Np / 128, Cp, Q, seq, gm.blk_counter + 1);

@@ -610,7 +610,8 @@ struct Prof {
 
 template <int BLOCK_N, int MODE, int NCTA, bool F16>
 int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap &Bh, const CUtensorMap &Bl, dim3 grid,
-                int kb_total, int kb_per_split, const EpiParams &E, cudaStream_t st, int chunk_kb, int mma_mask) {
+                int kb_total, int kb_per_split, const EpiParams &E, cudaStream_t st, int chunk_kb, int mma_mask,
+                int prof_kind) {
   using C = Cfg<BLOCK_N, NCTA>;
   constexpr bool RESID = MODE == 1 || MODE == 3;
   auto kernel = tc_gemm_kernel<BLOCK_N, MODE, NCTA, F16>;
@@ -648,8 +649,9 @@ int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap 
   B2M_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, Ah, Al, Bh, Bl, kb_total, kb_per_split, chunk_kb, mma_mask, Tm, Tn, n_tiles, E));
   if (g_prof.on) {
     B2M_CHECK_CUDA(cudaEventRecord(e1, st));
-    g_prof.ev[RESID ? 0 : 1].push_back(e0);
-    g_prof.ev[RESID ? 0 : 1].push_back(e1);
+    const int k = prof_kind >= 0 ? prof_kind : (RESID ? 0 : 1);
+    g_prof.ev[k].push_back(e0);
+    g_prof.ev[k].push_back(e1);
   }
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
@@ -659,17 +661,17 @@ int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap 
 template <int BLOCK_N, int MODE>
 int launch_tc(int ncta, const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap &Bh, const CUtensorMap &Bl,
               dim3 grid, int kb_total, int kb_per_split, const EpiParams &E, cudaStream_t st,
-              int chunk_kb = DEFAULT_CHUNK_KB, int mma_mask = 7, bool f16 = false) {
+              int chunk_kb = DEFAULT_CHUNK_KB, int mma_mask = 7, bool f16 = false, int prof_kind = -1) {
   if constexpr (MODE == 2) {   // the push epilogue exists for the shape it is used with: fp16 encoding, CTA pairs
     B2M_REQUIRE(f16 && ncta == 2, "K6 push epilogue: needs the fp16 encoding and whole 256-row tiles");
-    return launch_tc_n<BLOCK_N, 2, 2, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask);
+    return launch_tc_n<BLOCK_N, 2, 2, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask, prof_kind);
   } else {
     if (f16) {
-      if (ncta == 2) return launch_tc_n<BLOCK_N, MODE, 2, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask);
-      return launch_tc_n<BLOCK_N, MODE, 1, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask);
+      if (ncta == 2) return launch_tc_n<BLOCK_N, MODE, 2, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask, prof_kind);
+      return launch_tc_n<BLOCK_N, MODE, 1, true>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask, prof_kind);
     }
-    if (ncta == 2) return launch_tc_n<BLOCK_N, MODE, 2, false>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask);
-    return launch_tc_n<BLOCK_N, MODE, 1, false>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask);
+    if (ncta == 2) return launch_tc_n<BLOCK_N, MODE, 2, false>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask, prof_kind);
+    return launch_tc_n<BLOCK_N, MODE, 1, false>(Ah, Al, Bh, Bl, grid, kb_total, kb_per_split, E, st, chunk_kb, mma_mask, prof_kind);
   }
 }
 
@@ -731,10 +733,10 @@ int grad_block_n(const GlmModel &g) { return g.Dp % 256 == 0 ? 256 : (g.Dp % 128
 // CTA pairs need whole 256-row tiles of chains
 static int pair_mode(int64_t Cp) { return (Cp % 256 == 0) ? 2 : 1; }
 
-// split-K factor of K6: enough CTAs to fill the 148 SMs in whole waves, each split at least 8 k-blocks deep
-int grad_splits(const GlmModel &g, int64_t Cp) {
+// split-K factor of the gradient contraction over `kb` k-blocks (K6: K = Np; Gram form: K = Dp): enough CTAs to fill
+// the 148 SMs in whole waves, each split at least 8 k-blocks deep
+int grad_splits(const GlmModel &g, int64_t Cp, int kb) {
   const int64_t tiles = (Cp / BLOCK_M) * (g.Dp / grad_block_n(g));   // CTAs per split
-  const int kb = g.Np / (g.use_tc == 2 ? 64 : 32);
   int max_s = kb / 8 > 0 ? kb / 8 : 1;
   if (max_s > 32) max_s = 32;
   int best = 1;
@@ -747,6 +749,10 @@ int grad_splits(const GlmModel &g, int64_t Cp) {
     if (eff > best_eff + 1e-9) { best_eff = eff; best = s; }
   }
   return best;
+}
+
+int contraction_splits(const GlmModel &g, int64_t Cp) {
+  return grad_splits(g, Cp, (g.form == kFormGram ? g.Dp : g.Np) / (g.use_tc == 2 ? 64 : 32));
 }
 
 int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
@@ -785,8 +791,8 @@ int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st) {
   const bool f16 = g.use_tc == 2;
   const int bk = f16 ? 64 : 32;
   const int bn = grad_block_n(g);
-  const int splits = grad_splits(g, Cp);
   const int kb_total = g.Np / bk;
+  const int splits = grad_splits(g, Cp, kb_total);
   const int kb_per = (kb_total + splits - 1) / splits;
   const void *A_h = f16 ? (const void *)g.R16h : (const void *)g.Rh, *A_l = f16 ? (const void *)g.R16l : (const void *)g.Rl;
   const void *B_h = f16 ? (const void *)g.XT16h : (const void *)g.XTh, *B_l = f16 ? (const void *)g.XT16l : (const void *)g.XTl;
@@ -803,6 +809,35 @@ int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st) {
   if (bn == 256) return launch_tc<256, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
   if (bn == 128) return launch_tc<128, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
   return launch_tc<64, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16);
+}
+
+// Gram form: P = (packed delta rows) G~, [Cp, Dp] x [Dp, Dp] -- the K6 kernel body with the packed rows of K5 as the A
+// operand and the Gram halves as the B operand (K = Dp).  Its launch is the only contraction of an evaluation and is timed
+// in the K5 slot of the profile (b2m_profile_read): readers that sum K5 + K6 get the contraction time of one evaluation
+// and, with no K6 entries, count one launch per evaluation.
+int tc_gemm_gram(GlmModel &g, int64_t Cp, cudaStream_t st) {
+  B2M_REQUIRE(g.form == kFormGram && g.Gmh && g.Gml, "tc_gemm_gram: the model has no Gram operand");
+  const int ncta = pair_mode(Cp);
+  const bool f16 = g.use_tc == 2;
+  const int bk = f16 ? 64 : 32;
+  const int bn = grad_block_n(g);
+  const int kb_total = g.Dp / bk;
+  const int splits = grad_splits(g, Cp, kb_total);
+  const int kb_per = (kb_total + splits - 1) / splits;
+  const void *A_h = f16 ? (const void *)g.B16h : (const void *)g.Bh, *A_l = f16 ? (const void *)g.B16l : (const void *)g.Bl;
+  CUtensorMap Ah, Al, Bh, Bl;
+  if (make_map(&Ah, A_h, Cp, g.Dp, BLOCK_M, f16) || make_map(&Al, A_l, Cp, g.Dp, BLOCK_M, f16) ||
+      make_map(&Bh, g.Gmh, g.Dp, g.Dp, bn / ncta, f16) || make_map(&Bl, g.Gml, g.Dp, g.Dp, bn / ncta, f16))
+    return 2;
+  EpiParams E{};
+  E.Gpart = g.G; E.Cp = Cp; E.Dp = g.Dp;
+  E.skip_flag = g.skip_flag; E.skip_target = g.skip_target;
+  dim3 grid((unsigned)(Cp / BLOCK_M), g.Dp / bn, (unsigned)((kb_total + kb_per - 1) / kb_per));
+  g.g_splits = (int)grid.z;
+  const int ck = f16 ? DEFAULT_CHUNK_KB / 2 : DEFAULT_CHUNK_KB;
+  if (bn == 256) return launch_tc<256, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16, 0);
+  if (bn == 128) return launch_tc<128, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16, 0);
+  return launch_tc<64, 0>(ncta, Ah, Al, Bh, Bl, grid, kb_total, kb_per, E, st, ck, 7, f16, 0);
 }
 
 // K6 of a peer-sliced observation shard: one K pass over the rank's rows (no split-K: every output tile is produced

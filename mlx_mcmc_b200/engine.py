@@ -36,10 +36,13 @@ class DeviceModel:
     ``glm_path`` ('auto' | 'simt' | 'tc' | 'tc16') and ``pointwise_path`` ('auto' | 'general') choose the arithmetic /
     evaluation path (b2m_model_options; they were environment variables in ABI 1).  ``transforms``: None (the
     reference: the sampler moves in the model's own coordinates) or 'auto' -- positive / unit-interval parameters,
-    recognised from the support of the distribution they are the value of, are sampled in log / logit coordinates."""
+    recognised from the support of the distribution they are the value of, are sampled in log / logit coordinates.
+    ``glm_form`` ('auto' | 'stream' | 'gram') chooses how a GLM-class Normal likelihood is evaluated: two contractions
+    over X per evaluation, or one against X^T X precomputed in float64 (DESIGN.md 4.2); ``self.glm_form`` is the form
+    in use ('stream' | 'gram', None for pointwise models)."""
 
     def __init__(self, traced: TracedModel, device: Optional[torch.device] = None, glm_path: str = "auto",
-                 pointwise_path: str = "auto", transforms=None):
+                 pointwise_path: str = "auto", transforms=None, glm_form: str = "auto"):
         self.lib = _cabi.load()
         self.device = device or _require_cuda()
         self.traced = traced
@@ -47,6 +50,8 @@ class DeviceModel:
         self.layout = traced.layout
         if glm_path not in _cabi.GLM_PATHS:
             raise ValueError(f"Unknown glm_path: {glm_path}")
+        if glm_form not in _cabi.GLM_FORMS:
+            raise ValueError(f"Unknown glm_form: {glm_form}")
         if pointwise_path not in ("auto", "general"):
             raise ValueError(f"Unknown pointwise_path: {pointwise_path}")
         if transforms not in (None, "auto"):
@@ -74,6 +79,7 @@ class DeviceModel:
         handle = C.c_void_p()
         opt = _cabi.ModelOptions()
         opt.glm_path = _cabi.GLM_PATHS[glm_path]
+        opt.glm_form = _cabi.GLM_FORMS[glm_form]
         opt.pointwise_path = _cabi.POINTWISE_GENERAL if pointwise_path == "general" else _cabi.POINTWISE_AUTO
         tf_arr = (C.c_int32 * self.D)(*[int(v) for v in self.tf_codes])
         opt.transforms = tf_arr if self.has_transforms else None
@@ -83,6 +89,7 @@ class DeviceModel:
         self.jit = False            # set by jit.specialize once a specialised module is attached
         self.model_class = self.lib.b2m_model_class(handle)
         self.glm_path = {0: "simt", 1: "tc", 2: "tc16"}.get(self.lib.b2m_model_glm_path(handle))
+        self.glm_form = {1: "stream", 2: "gram"}.get(self.lib.b2m_model_glm_form(handle))
 
     def __del__(self):
         h, self.handle = getattr(self, "handle", None), None
@@ -298,7 +305,7 @@ def clear_model_cache() -> None:
 
 
 def compile_model(log_prob_fn, initial_params, cache: bool = True, glm_path: str = "auto", pointwise_path: str = "auto",
-                  transforms=None) -> DeviceModel:
+                  transforms=None, glm_form: str = "auto") -> DeviceModel:
     """Trace `log_prob_fn` (always) and return its device model: a cached one when the trace -- terms, layout and the
     contents of the observed arrays -- is identical to one already resident on this device, else a new one.
     ``cache=False`` neither looks up nor stores."""
@@ -306,12 +313,13 @@ def compile_model(log_prob_fn, initial_params, cache: bool = True, glm_path: str
     traced = trace(log_prob_fn, initial_params)
     key = None
     if cache:
-        key = _trace_fingerprint(traced, (dev.index, glm_path, pointwise_path, transforms))
+        key = _trace_fingerprint(traced, (dev.index, glm_path, pointwise_path, transforms, glm_form))
         hit = _MODEL_CACHE.pop(key, None)
         if hit is not None:
             _MODEL_CACHE[key] = hit          # most recently used goes last
             return hit
-    model = DeviceModel(traced, dev, glm_path=glm_path, pointwise_path=pointwise_path, transforms=transforms)
+    model = DeviceModel(traced, dev, glm_path=glm_path, pointwise_path=pointwise_path, transforms=transforms,
+                        glm_form=glm_form)
     model._fn = log_prob_fn
     if cache:
         _MODEL_CACHE[key] = model

@@ -64,7 +64,8 @@ def setup(kind, seed=1234):
     else:
         fn, init, meta = W.regression(B.ns, n, d, seed=0)
         curv, eps0 = float(n), 8e-4
-    model = compile_model(fn, init, cache=False, glm_path=args.path)
+    # the Normal reference runs the streaming form: the comparison is of the two kinds' K5 epilogues over the same K6
+    model = compile_model(fn, init, cache=False, glm_path=args.path, glm_form="stream")
     th = torch.zeros(128, d, device="cuda")
     for _ in range(30):                    # gradient ascent with a step below 1 / (largest curvature): the mode
         _, g = model.logp_grad(th)
@@ -136,7 +137,8 @@ res["k6_logistic_over_normal"] = res["logistic"]["k6_ms_per_eval_median"] / res[
 def probe(kind, d):
     """K5 / K6 ms of one value+gradient at [chains, d] x [d, n], median of 5 (b2m_profile events)"""
     fn, init, _ = (W.logistic_regression if kind == "logistic" else W.regression)(B.ns, args.n, d, seed=0)
-    model = compile_model(fn, init, cache=False, glm_path=args.path)
+    # the Normal reference runs the streaming form: the comparison is of the two kinds' K5 epilogues over the same K6
+    model = compile_model(fn, init, cache=False, glm_path=args.path, glm_form="stream")
     gen = torch.Generator(device="cuda")
     gen.manual_seed(3)
     theta = (0.05 * torch.randn(args.chains, d, device="cuda", generator=gen)).contiguous()
