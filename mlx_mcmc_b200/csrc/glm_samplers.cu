@@ -317,9 +317,17 @@ int glm_mh_run(GlmModel &gm, const b2m_mh_args &a, cudaStream_t st) {
 
 // ================================================================= NUTS
 struct NutsBufs {
-  // [C, D] vectors
-  float *g, *p0, *q_lo, *p_lo, *g_lo, *q_hi, *p_hi, *g_hi, *cq, *cg, *fq, *fp, *fg, *sfq, *sfp, *scq, *scg;
-  float *st_fq, *st_fp, *st_cq, *st_cg;  // [MD, C, D] stack of parked left subtrees
+  // [C, D] vectors: gradient at the starting points of the call, and the working leaf (position, momentum, gradient)
+  float *g, *fq, *fp, *fg;
+  // Saved tree states: n_slots slots per chain, [C, n_slots, 3, D]; slot s of chain c holds q, p, g as three [D] rows.
+  // The tree refers to them by per-chain slot numbers, so a merge, a push or a candidate choice moves an index, not a
+  // vector.  Live at once: lo, hi, cand and st_f / st_c of every parked level (at most 2 MD + 1), plus the new leaf.
+  float *slots;
+  int n_slots;
+  int *lo, *hi, *cand;   // [C] trajectory edges and the candidate
+  int *leaf_slot;        // [C] the last completed leaf (the start of the next leaf; the new edge at a doubling's end)
+  int *sub_c;            // [C] candidate of the completed subtree of the current doubling
+  int *st_f, *st_c;      // [MD, C] first edge and candidate of the parked left subtrees
   // [C] scalars
   float *lp, *clp, *h0, *log_slice, *flp, *sclp, *feps, *heps;
   int *n, *s, *v, *leaf, *building, *sub_n, *sub_na, *sub_s, *alpha_cnt, *depth;
@@ -391,21 +399,32 @@ __device__ __noinline__ bool straight_w(const float *q_lo, const float *q_hi, co
   return a >= 0.f && b >= 0.f;
 }
 
+// row r (0 = q, 1 = p, 2 = g) of slot s of chain c
+__device__ __forceinline__ float *slot_row(const NutsBufs &W, int D, int64_t c, int s, int r) {
+  return W.slots + (((size_t)c * W.n_slots + s) * 3 + r) * D;
+}
+
 __device__ __forceinline__ void nuts_begin_dev(const b2m_nuts_args &A, const NutsBufs &W, int D, int64_t c, int lane, int it) {
   const uint64_t gchain = (uint64_t)(A.chain_offset + c);
   const uint32_t giter = (uint32_t)(A.iter_offset + it);
   const size_t row = (size_t)it * A.n_chains + c;
   const size_t o = (size_t)c * D;
   const uint4 w0 = Philox::draw(A.seed, gchain, giter, 0u);
-  fill_momentum(W.p0 + o, D, A.inj_normal ? A.inj_normal + row * D : nullptr, A.seed, gchain, giter, w0, lane, A.inv_mass);
+  // the start slot: the previous transition's candidate already holds theta and its gradient; the first transition
+  // of a call takes them from the caller's theta and the gradient evaluated at the start of the call
+  int s0 = 0;
+  if (it == 0) {
+    vcopy(slot_row(W, D, c, 0, 0), A.theta + o, D, lane);
+    vcopy(slot_row(W, D, c, 0, 2), W.g + o, D, lane);
+  } else {
+    s0 = W.cand[c];
+  }
+  float *p = slot_row(W, D, c, s0, 1);
+  fill_momentum(p, D, A.inj_normal ? A.inj_normal + row * D : nullptr, A.seed, gchain, giter, w0, lane, A.inv_mass);
   __syncwarp();
-  const float kin = kinetic_w(W.p0 + o, D, lane, A.inv_mass);
-  const float *q = A.theta + o;
-  vcopy(W.q_lo + o, q, D, lane); vcopy(W.q_hi + o, q, D, lane);
-  vcopy(W.p_lo + o, W.p0 + o, D, lane); vcopy(W.p_hi + o, W.p0 + o, D, lane);
-  vcopy(W.g_lo + o, W.g + o, D, lane); vcopy(W.g_hi + o, W.g + o, D, lane);
-  vcopy(W.cq + o, q, D, lane); vcopy(W.cg + o, W.g + o, D, lane);
+  const float kin = kinetic_w(p, D, lane, A.inv_mass);
   if (lane == 0) {
+    W.lo[c] = s0; W.hi[c] = s0; W.cand[c] = s0;
     const float h0 = -W.lp[c] + kin;
     const float us = A.inj_slice ? A.inj_slice[row] : u01(w0.z);
     const double log_u64 = (double)(-h0) + (double)logf(us);
@@ -429,15 +448,13 @@ __device__ __forceinline__ void nuts_doubling_begin_dev(const b2m_nuts_args &A, 
   const uint64_t gchain = (uint64_t)(A.chain_offset + c);
   const uint32_t giter = (uint32_t)(A.iter_offset + it);
   const size_t row = (size_t)it * A.n_chains + c;
-  const size_t o = (size_t)c * D;
   float ud;
   if (A.inj_dir) ud = A.inj_dir[row * A.max_tree_depth + j];
   else ud = u01(Philox::draw(A.seed, gchain, giter, SLOT_NUTS_DOUBLING + j).x);
   const int v = ud < 0.5f ? 1 : -1;
-  if (v == 1) { vcopy(W.fq + o, W.q_hi + o, D, lane); vcopy(W.fp + o, W.p_hi + o, D, lane); vcopy(W.fg + o, W.g_hi + o, D, lane); }
-  else        { vcopy(W.fq + o, W.q_lo + o, D, lane); vcopy(W.fp + o, W.p_lo + o, D, lane); vcopy(W.fg + o, W.g_lo + o, D, lane); }
   if (lane == 0) {
     const double eps = W.eps_it[c];
+    W.leaf_slot[c] = v == 1 ? W.hi[c] : W.lo[c];   // the first leaf steps off the edge in direction v
     W.v[c] = v;
     W.feps[c] = (float)((double)v * eps);
     W.heps[c] = (float)(0.5 * ((double)v * eps));
@@ -456,20 +473,24 @@ __device__ __forceinline__ void nuts_leaf_pre_dev(const b2m_nuts_args &A, const 
   const size_t o = (size_t)c * D;
   const float he = W.heps[c], fe = W.feps[c];
   float *__restrict__ fq = W.fq + o, *__restrict__ fp = W.fp + o;
-  const float *__restrict__ fg = W.fg + o;
+  // start state: the last leaf, or the edge the doubling extends
+  const int s = W.leaf_slot[c];
+  const float *__restrict__ sq = slot_row(W, D, c, s, 0), *__restrict__ sp = slot_row(W, D, c, s, 1),
+                            *__restrict__ sg = slot_row(W, D, c, s, 2);
   if (const float *__restrict__ im = A.inv_mass) {   // diagonal mass matrix: drift by eps M^-1 p
 #pragma unroll 4
     for (int d = lane; d < D; d += 32) {
-      const float pv = __fadd_rn(fp[d], __fmul_rn(he, fg[d]));
+      const float pv = __fadd_rn(sp[d], __fmul_rn(he, sg[d]));
       fp[d] = pv;
-      fq[d] = __fadd_rn(fq[d], __fmul_rn(fe, im[d] * pv));
+      fq[d] = __fadd_rn(sq[d], __fmul_rn(fe, im[d] * pv));
     }
     return;
   }
-  if ((D & 3) == 0 && ((reinterpret_cast<uintptr_t>(fq) | reinterpret_cast<uintptr_t>(fp) | reinterpret_cast<uintptr_t>(fg)) & 15) == 0) {
+  if ((D & 3) == 0 && ((reinterpret_cast<uintptr_t>(fq) | reinterpret_cast<uintptr_t>(fp) | reinterpret_cast<uintptr_t>(sq) |
+                        reinterpret_cast<uintptr_t>(sp) | reinterpret_cast<uintptr_t>(sg)) & 15) == 0) {
     for (int d = 4 * lane; d < D; d += 128) {   // four coefficients per lane: same per-element arithmetic
-      const float4 g4 = *reinterpret_cast<const float4 *>(fg + d);
-      float4 p4 = *reinterpret_cast<float4 *>(fp + d), q4 = *reinterpret_cast<float4 *>(fq + d);
+      const float4 g4 = *reinterpret_cast<const float4 *>(sg + d);
+      float4 p4 = *reinterpret_cast<const float4 *>(sp + d), q4 = *reinterpret_cast<const float4 *>(sq + d);
       p4.x = __fadd_rn(p4.x, __fmul_rn(he, g4.x)); p4.y = __fadd_rn(p4.y, __fmul_rn(he, g4.y));
       p4.z = __fadd_rn(p4.z, __fmul_rn(he, g4.z)); p4.w = __fadd_rn(p4.w, __fmul_rn(he, g4.w));
       q4.x = __fadd_rn(q4.x, __fmul_rn(fe, p4.x)); q4.y = __fadd_rn(q4.y, __fmul_rn(fe, p4.y));
@@ -481,9 +502,9 @@ __device__ __forceinline__ void nuts_leaf_pre_dev(const b2m_nuts_args &A, const 
   }
 #pragma unroll 4
   for (int d = lane; d < D; d += 32) {
-    const float pv = __fadd_rn(fp[d], __fmul_rn(he, fg[d]));
+    const float pv = __fadd_rn(sp[d], __fmul_rn(he, sg[d]));
     fp[d] = pv;
-    fq[d] = __fadd_rn(fq[d], __fmul_rn(fe, pv));
+    fq[d] = __fadd_rn(sq[d], __fmul_rn(fe, pv));
   }
 }
 
@@ -501,27 +522,31 @@ __device__ __forceinline__ void nuts_leaf_post_dev(const b2m_nuts_args &A, const
   const size_t o = (size_t)c * D;
   const int MD = A.max_tree_depth;
   const bool ref_compat = A.compat == B2M_COMPAT_REFERENCE;
-  float *fq = W.fq + o, *fp = W.fp + o;
-  const float *fg = W.fg + o;
+  const float *fq = W.fq + o, *fp = W.fp + o, *fg = W.fg + o;
   const float he = W.heps[c];
-  // one pass: second half kick, kinetic energy, and the four copies that make "the subtree being assembled = this
-  // leaf" (first edge = candidate = this state) -- three loads and five stores per element instead of six passes
+  const int i = W.leaf[c];
+  // a free slot for this leaf: one that is not an edge, not the candidate and not a parked subtree (the parked levels
+  // are the set bits of the leaf index)
+  unsigned live = (1u << W.lo[c]) | (1u << W.hi[c]) | (1u << W.cand[c]);
+  for (int k = 0; k < j; ++k)
+    if ((i >> k) & 1) live |= (1u << W.st_f[(size_t)k * C + c]) | (1u << W.st_c[(size_t)k * C + c]);
+  const int L = __ffs(~live) - 1;
+  B2M_ASSERT(L >= 0 && L < W.n_slots);
+  float *__restrict__ lq = slot_row(W, D, c, L, 0), *__restrict__ lp = slot_row(W, D, c, L, 1), *__restrict__ lg = slot_row(W, D, c, L, 2);
+  // one pass: second half kick, kinetic energy, and the completed leaf stored into its slot -- three loads and three
+  // stores per element.  The leaf is then both the first edge and the candidate of the subtree being assembled.
   float k0 = 0.f, k1 = 0.f;
   {
-    float *__restrict__ sfq = W.sfq + o, *__restrict__ sfp = W.sfp + o, *__restrict__ scq = W.scq + o, *__restrict__ scg = W.scg + o;
     int d = lane;
     if ((D & 3) == 0 && ((reinterpret_cast<uintptr_t>(fq) | reinterpret_cast<uintptr_t>(fp) | reinterpret_cast<uintptr_t>(fg) |
-                          reinterpret_cast<uintptr_t>(sfq) | reinterpret_cast<uintptr_t>(sfp) | reinterpret_cast<uintptr_t>(scq) |
-                          reinterpret_cast<uintptr_t>(scg)) & 15) == 0) {
+                          reinterpret_cast<uintptr_t>(lq) | reinterpret_cast<uintptr_t>(lp) | reinterpret_cast<uintptr_t>(lg)) & 15) == 0) {
       for (int e = 4 * lane; e < D; e += 128) {   // four coefficients per lane
         const float4 q4 = *reinterpret_cast<const float4 *>(fq + e), g4 = *reinterpret_cast<const float4 *>(fg + e);
-        float4 p4 = *reinterpret_cast<float4 *>(fp + e);
+        float4 p4 = *reinterpret_cast<const float4 *>(fp + e);
         p4.x = __fadd_rn(p4.x, __fmul_rn(he, g4.x)); p4.y = __fadd_rn(p4.y, __fmul_rn(he, g4.y));
         p4.z = __fadd_rn(p4.z, __fmul_rn(he, g4.z)); p4.w = __fadd_rn(p4.w, __fmul_rn(he, g4.w));
         k0 = fmaf(p4.x, p4.x, k0); k1 = fmaf(p4.y, p4.y, k1); k0 = fmaf(p4.z, p4.z, k0); k1 = fmaf(p4.w, p4.w, k1);
-        *reinterpret_cast<float4 *>(fp + e) = p4;
-        *reinterpret_cast<float4 *>(sfq + e) = q4; *reinterpret_cast<float4 *>(scq + e) = q4;
-        *reinterpret_cast<float4 *>(sfp + e) = p4; *reinterpret_cast<float4 *>(scg + e) = g4;
+        *reinterpret_cast<float4 *>(lq + e) = q4; *reinterpret_cast<float4 *>(lp + e) = p4; *reinterpret_cast<float4 *>(lg + e) = g4;
       }
       d = D;   // nothing left for the scalar loops
     }
@@ -529,20 +554,18 @@ __device__ __forceinline__ void nuts_leaf_post_dev(const b2m_nuts_args &A, const
       const float q0 = fq[d], q1 = fq[d + 32], g0 = fg[d], g1 = fg[d + 32];
       const float p0 = __fadd_rn(fp[d], __fmul_rn(he, g0)), p1 = __fadd_rn(fp[d + 32], __fmul_rn(he, g1));
       k0 = fmaf(p0, p0, k0); k1 = fmaf(p1, p1, k1);
-      fp[d] = p0; fp[d + 32] = p1;
-      sfq[d] = q0; sfq[d + 32] = q1; scq[d] = q0; scq[d + 32] = q1;
-      sfp[d] = p0; sfp[d + 32] = p1; scg[d] = g0; scg[d + 32] = g1;
+      lq[d] = q0; lq[d + 32] = q1; lp[d] = p0; lp[d + 32] = p1; lg[d] = g0; lg[d + 32] = g1;
     }
     for (; d < D; d += 32) {
       const float q0 = fq[d], g0 = fg[d];
       const float p0 = __fadd_rn(fp[d], __fmul_rn(he, g0));
       k0 = fmaf(p0, p0, k0);
-      fp[d] = p0; sfq[d] = q0; scq[d] = q0; sfp[d] = p0; scg[d] = g0;
+      lq[d] = q0; lp[d] = p0; lg[d] = g0;
     }
   }
   float kin = 0.5f * warp_sum(k0 + k1);
   __syncwarp();
-  if (A.inv_mass) kin = kinetic_w(fp, D, lane, A.inv_mass);   // 0.5 sum p^2 / m (fp holds the completed step's momentum)
+  if (A.inv_mass) kin = kinetic_w(lp, D, lane, A.inv_mass);   // 0.5 sum p^2 / m (lp holds the completed step's momentum)
   const float flp = W.flp[c], h0 = W.h0[c], log_slice = W.log_slice[c];
   const float h1 = -flp + kin;
   const int n1 = (log_slice <= -h1) ? 1 : 0;
@@ -550,7 +573,7 @@ __device__ __forceinline__ void nuts_leaf_post_dev(const b2m_nuts_args &A, const
   float a1 = expf(-h1 + h0);
   if (a1 != a1) a1 = ref_compat ? 1.0f : 0.0f;
   a1 = fminf(a1, 1.0f);
-  const int v = W.v[c], i = W.leaf[c];
+  const int v = W.v[c];
   B2M_ASSERT(j >= 0 && j < A.max_tree_depth && i >= 0 && i < (1 << j) && (v == 1 || v == -1));
   if (lane == 0) {
     A.n_leaves[c] += 1;
@@ -560,11 +583,12 @@ __device__ __forceinline__ void nuts_leaf_post_dev(const b2m_nuts_args &A, const
   int sub_n = n1, sub_na = 1;
   bool sub_s = s1;
   double sub_alpha = (double)a1;
+  int sf = L, sc = L;   // first edge and candidate of the subtree being assembled
   int k = 0;
   bool finished = false;
   while (true) {
     if (k == j) { finished = true; break; }
-    const size_t so = ((size_t)k * C + c) * D, ss = (size_t)k * C + c;
+    const size_t ss = (size_t)k * C + c;
     if ((i >> k) & 1) {
       const int m = i - __popc(i) + k;
       float um;
@@ -578,32 +602,37 @@ __device__ __forceinline__ void nuts_leaf_post_dev(const b2m_nuts_args &A, const
       const int n_tot = W.st_n[ss] + sub_n;
       const double ratio = (double)sub_n / fmax((double)n_tot, 1.0);
       if (!((double)um < ratio)) {
-        vcopy(W.scq + o, W.st_cq + so, D, lane); vcopy(W.scg + o, W.st_cg + so, D, lane);
+        sc = W.st_c[ss];
         sub_clp = W.st_clp[ss];
       }
+      // the parked subtree's first edge against the far edge of this one (the leaf just stored)
+      const int pf = W.st_f[ss];
+      const float *fq_k = slot_row(W, D, c, pf, 0), *fp_k = slot_row(W, D, c, pf, 1);
       bool st;
-      if (v == 1) st = straight_w(W.st_fq + so, fq, W.st_fp + so, fp, D, lane);
-      else        st = straight_w(fq, W.st_fq + so, fp, W.st_fp + so, D, lane);
+      if (v == 1) st = straight_w(fq_k, lq, fp_k, lp, D, lane);
+      else        st = straight_w(lq, fq_k, lp, fp_k, D, lane);
       sub_s = sub_s && st;
-      vcopy(W.sfq + o, W.st_fq + so, D, lane); vcopy(W.sfp + o, W.st_fp + so, D, lane);
-      __syncwarp();
+      sf = pf;
       sub_n = n_tot;
       sub_alpha = W.st_alpha[ss] + sub_alpha;
       sub_na = W.st_na[ss] + sub_na;
       ++k;
     } else {
       if (sub_s) {
-        vcopy(W.st_fq + so, W.sfq + o, D, lane); vcopy(W.st_fp + so, W.sfp + o, D, lane);
-        vcopy(W.st_cq + so, W.scq + o, D, lane); vcopy(W.st_cg + so, W.scg + o, D, lane);
-        if (lane == 0) { W.st_clp[ss] = sub_clp; W.st_n[ss] = sub_n; W.st_na[ss] = sub_na; W.st_alpha[ss] = sub_alpha; }
+        if (lane == 0) {
+          W.st_f[ss] = sf; W.st_c[ss] = sc;
+          W.st_clp[ss] = sub_clp; W.st_n[ss] = sub_n; W.st_na[ss] = sub_na; W.st_alpha[ss] = sub_alpha;
+        }
         break;
       }
       ++k;
     }
   }
   if (lane == 0) {
+    W.leaf_slot[c] = L;
     if (finished) {
       W.building[c] = 0;
+      W.sub_c[c] = sc;
       W.sclp[c] = sub_clp; W.sub_n[c] = sub_n; W.sub_na[c] = sub_na; W.sub_s[c] = sub_s ? 1 : 0; W.sub_alpha[c] = sub_alpha;
     } else {
       W.leaf[c] = i + 1;
@@ -621,10 +650,10 @@ __device__ __forceinline__ void nuts_doubling_end_dev(const b2m_nuts_args &A, co
   const uint64_t gchain = (uint64_t)(A.chain_offset + c);
   const uint32_t giter = (uint32_t)(A.iter_offset + it);
   const size_t row = (size_t)it * A.n_chains + c;
-  const size_t o = (size_t)c * D;
   const int v = W.v[c];
-  if (v == 1) { vcopy(W.q_hi + o, W.fq + o, D, lane); vcopy(W.p_hi + o, W.fp + o, D, lane); vcopy(W.g_hi + o, W.fg + o, D, lane); }
-  else        { vcopy(W.q_lo + o, W.fq + o, D, lane); vcopy(W.p_lo + o, W.fp + o, D, lane); vcopy(W.g_lo + o, W.fg + o, D, lane); }
+  int lo = W.lo[c], hi = W.hi[c];
+  if (v == 1) hi = W.leaf_slot[c];   // the last leaf is the new edge in direction v
+  else        lo = W.leaf_slot[c];
   const int sub_n = W.sub_n[c], sub_s = W.sub_s[c];
   const int n = W.n[c];
   int took = 0;
@@ -633,16 +662,14 @@ __device__ __forceinline__ void nuts_doubling_end_dev(const b2m_nuts_args &A, co
     if (A.inj_take) ut = A.inj_take[row * A.max_tree_depth + j];
     else ut = u01(Philox::draw(A.seed, gchain, giter, SLOT_NUTS_DOUBLING + j).y);
     const double pr = fmin(1.0, (double)sub_n / fmax((double)n, 1.0));
-    if ((double)ut < pr) {
-      vcopy(W.cq + o, W.scq + o, D, lane); vcopy(W.cg + o, W.scg + o, D, lane);
-      took = 1;
-    }
+    if ((double)ut < pr) took = 1;
   }
-  __syncwarp();
-  const bool st = straight_w(W.q_lo + o, W.q_hi + o, W.p_lo + o, W.p_hi + o, D, lane);
+  const bool st = straight_w(slot_row(W, D, c, lo, 0), slot_row(W, D, c, hi, 0), slot_row(W, D, c, lo, 1),
+                             slot_row(W, D, c, hi, 1), D, lane);
   const int s_new = (sub_s && st) ? 1 : 0;
   if (lane == 0) {
-    if (took) W.clp[c] = W.sclp[c];
+    W.lo[c] = lo; W.hi[c] = hi;
+    if (took) { W.cand[c] = W.sub_c[c]; W.clp[c] = W.sclp[c]; }
     W.n[c] = n + sub_n;
     W.s[c] = s_new;
     W.alpha_sum[c] += W.sub_alpha[c];
@@ -663,12 +690,12 @@ __global__ void __launch_bounds__(32 * WPB) nuts_doubling_end_kernel(b2m_nuts_ar
 __device__ __forceinline__ void nuts_end_dev(const b2m_nuts_args &A, const NutsBufs &W, int D, int64_t c, int lane, int it) {
   const uint32_t giter = (uint32_t)(A.iter_offset + it);
   const size_t row = (size_t)it * A.n_chains + c;
-  const size_t o = (size_t)c * D;
-  vcopy(A.theta + o, W.cq + o, D, lane);
-  vcopy(W.g + o, W.cg + o, D, lane);
+  // the candidate slot stays as it is: the next transition starts from it (nuts_begin_dev)
+  const float *cq = slot_row(W, D, c, W.cand[c], 0);
+  vcopy(A.theta + (size_t)c * D, cq, D, lane);
   if (A.draws) {
-    if (W.tf && !A.draws_unconstrained) write_draw(A.draws + row * D, W.cq + o, D, lane, W.tf);
-    else vcopy(A.draws + row * D, W.cq + o, D, lane);
+    if (W.tf && !A.draws_unconstrained) write_draw(A.draws + row * D, cq, D, lane, W.tf);
+    else vcopy(A.draws + row * D, cq, D, lane);
   }
   if (lane == 0) {
     W.lp[c] = W.clp[c];
@@ -770,15 +797,17 @@ __global__ void __launch_bounds__(1024) nuts_pool_adapt_kernel(b2m_nuts_args A, 
 // carve the NUTS workspace (both schedules) out of the model's arena
 static void nuts_layout(Arena &A, NutsBufs &W, int64_t C, int D, int MD) {
   const size_t cd = (size_t)C * D;
-  float **vecs[] = {&W.g, &W.p0, &W.q_lo, &W.p_lo, &W.g_lo, &W.q_hi, &W.p_hi, &W.g_hi, &W.cq, &W.cg,
-                    &W.fq, &W.fp, &W.fg, &W.sfq, &W.sfp, &W.scq, &W.scg};
+  float **vecs[] = {&W.g, &W.fq, &W.fp, &W.fg};
   for (auto v : vecs) A.take(v, cd);
-  float **stk[] = {&W.st_fq, &W.st_fp, &W.st_cq, &W.st_cg};
-  for (auto v : stk) A.take(v, cd * MD);
+  static_assert(2 * B2M_MAX_TREE_DEPTH + 2 <= 32, "the free-slot search keeps the live slots in a 32-bit mask");
+  W.n_slots = 2 * MD + 2;
+  A.take(&W.slots, cd * 3 * W.n_slots);
   float **fs[] = {&W.lp, &W.clp, &W.h0, &W.log_slice, &W.flp, &W.sclp, &W.feps, &W.heps};
   for (auto v : fs) A.take(v, C);
-  int **is[] = {&W.n, &W.s, &W.v, &W.leaf, &W.building, &W.sub_n, &W.sub_na, &W.sub_s, &W.alpha_cnt, &W.depth};
+  int **is[] = {&W.n, &W.s, &W.v, &W.leaf, &W.building, &W.sub_n, &W.sub_na, &W.sub_s, &W.alpha_cnt, &W.depth,
+                &W.lo, &W.hi, &W.cand, &W.leaf_slot, &W.sub_c};
   for (auto v : is) A.take(v, C);
+  A.take(&W.st_f, (size_t)C * MD); A.take(&W.st_c, (size_t)C * MD);
   A.take(&W.alpha_sum, C); A.take(&W.sub_alpha, C);
   A.take(&W.st_clp, (size_t)C * MD); A.take(&W.st_n, (size_t)C * MD); A.take(&W.st_na, (size_t)C * MD);
   A.take(&W.st_alpha, (size_t)C * MD);
