@@ -275,6 +275,22 @@ int b2m_model_glm_form(const b2m_model *m);
 int b2m_logp_grad(b2m_model *m, const float *theta, int64_t n_chains, float *logp, float *grad,
                   int32_t lanes, void *stream);
 
+/* ---- pointwise log-likelihood statistics over posterior draws (WAIC; DESIGN.md 4.6) ----
+ * For every observation n of the listed observation terms -- terms whose value operand involves no parameter (CONST,
+ * DATA, or LIN without parameter entries) while p0 or p1 does; CONSTANT terms never -- and every draw s:
+ *     ll[s, n] = w log p(x_n | params(theta_s))      (w = the term's weight; theta_s in model coordinates: no transforms,
+ *                                                      no Jacobian)
+ * out[n] = (lppd_n, mean_n, var_n): log((1/S) sum_s exp ll[s, n]), (1/S) sum_s ll[s, n], and the sample variance (ddof 1)
+ * over the S = n_draws draws.  Observations are numbered in term order, by element within a term.
+ *   draws      DEVICE [n_draws, D] (the samplers' [S, C, D] seen as rows)
+ *   obs_terms  HOST [n_obs_terms] term indices into the table given to b2m_model_create, increasing
+ *   out        DEVICE [n_obs, 3] float64; n_obs must be the sum of the listed terms' lengths
+ * The [S, N] matrix is never stored: GLM-class models reduce it inside the B X^T contraction (a statistics epilogue),
+ * other terms in a SIMT kernel; float64 running state, fixed order: repeated calls are bit-identical.  Refused for
+ * observation-sharded models.  Moves the GLM reference point beta0 (every sampler / logp call recentres). */
+int b2m_loglik_stats(b2m_model *m, const float *draws, int64_t n_draws, const int32_t *obs_terms, int32_t n_obs_terms,
+                     double *out, int64_t n_obs, void *stream);
+
 int b2m_hmc_run(b2m_model *m, const b2m_hmc_args *a, void *stream);
 int b2m_mh_run(b2m_model *m, const b2m_mh_args *a, void *stream);
 int b2m_nuts_run(b2m_model *m, const b2m_nuts_args *a, void *stream);

@@ -83,7 +83,8 @@ EXPORTS = ["b2m_last_error", "b2m_abi_version", "b2m_struct_sizes", "b2m_model_c
            "b2m_launch_count", "b2m_comm_unique_id", "b2m_comm_init", "b2m_comm_destroy", "b2m_model_set_comm",
            "b2m_comm_allreduce_f32", "b2m_profile", "b2m_profile_read", "b2m_diag_series", "b2m_diag_params", "b2m_sample",
            "b2m_options_size", "b2m_peer_alloc", "b2m_peer_open", "b2m_peer_close", "b2m_peer_free", "b2m_model_peer_bytes",
-           "b2m_model_peer_attach", "b2m_mass_from_draws", "b2m_quantiles", "b2m_model_attach_module", "b2m_model_has_module", "b2m_profile_read_ex"]
+           "b2m_model_peer_attach", "b2m_mass_from_draws", "b2m_quantiles", "b2m_model_attach_module", "b2m_model_has_module", "b2m_profile_read_ex",
+           "b2m_loglik_stats"]
 
 _lib = None
 
@@ -141,6 +142,7 @@ def load(build_if_missing: bool = True):
     lib.b2m_model_glm_path.argtypes = [c_p]
     lib.b2m_model_glm_form.argtypes = [c_p]
     lib.b2m_logp_grad.argtypes = [c_p, c_p, C.c_int64, c_p, c_p, C.c_int32, c_p]
+    lib.b2m_loglik_stats.argtypes = [c_p, c_p, C.c_int64, C.POINTER(C.c_int32), C.c_int32, c_p, C.c_int64, c_p]
     lib.b2m_hmc_run.argtypes = [c_p, C.POINTER(HmcArgs), c_p]
     lib.b2m_mh_run.argtypes = [c_p, C.POINTER(MhArgs), c_p]
     lib.b2m_nuts_run.argtypes = [c_p, C.POINTER(NutsArgs), c_p]

@@ -18,7 +18,7 @@ INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(CSRC, "libb200mcmc.so")
 STAMP = os.path.join(CSRC, ".build_stamp")
 
-SOURCES = ["capi.cu", "pointwise.cu", "nuts_pointwise.cu", "glm.cu", "glm_samplers.cu", "glm_tc.cu", "comm.cu", "diag.cu", "sample.cu", "jit.cu"]
+SOURCES = ["capi.cu", "pointwise.cu", "nuts_pointwise.cu", "glm.cu", "glm_samplers.cu", "glm_tc.cu", "comm.cu", "diag.cu", "sample.cu", "jit.cu", "loglik.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-I", INCLUDE,

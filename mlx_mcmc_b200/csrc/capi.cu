@@ -40,6 +40,8 @@ int diag_series(const float *draws, int64_t S, int64_t C, int64_t D, int ess_mod
                 float *ess_geyer, cudaStream_t st);
 int diag_params(const float *mean, const float *var, const float *ess_ref, const float *ess_geyer, int64_t S, int64_t C,
                 int64_t D, double *out, cudaStream_t st);
+int loglik_stats(const KModel &km, GlmModel *g, int lik, const std::vector<b2m_term> &terms, const std::vector<int> &obs,
+                 const float *draws, int64_t S, double *out, int64_t n_obs, cudaStream_t st);
 
 }  // namespace b2m
 
@@ -64,6 +66,19 @@ struct b2m_model {
   B2M_REQUIRE(_guard.owns_lock(), "this model handle is in use by another call (handles are not re-entrant: one per thread)")
 
 using b2m::set_error;
+
+// Observation terms (b2m_loglik_stats; the Python tracer's TracedModel.observation_terms makes the same choice): the
+// value operand involves no parameter and at least one of the distribution's parameters does.  Constant terms never.
+static bool op_has_param(const b2m_operand &o, const std::vector<b2m_lin_entry> &lin) {
+  if (o.kind == B2M_OP_PARAM || o.kind == B2M_OP_PARAMVEC || o.kind == B2M_OP_MATVEC) return true;
+  if (o.kind == B2M_OP_LIN)
+    for (int e = o.a; e < o.a + o.b; ++e)
+      if (lin[e].param >= 0) return true;
+  return false;
+}
+static bool is_observation_term(const b2m_term &T, const std::vector<b2m_lin_entry> &lin) {
+  return T.dist != B2M_CONSTANT && !op_has_param(T.x, lin) && (op_has_param(T.p0, lin) || op_has_param(T.p1, lin));
+}
 
 static bool valid_lanes(int l) { return l == 0 || l == 1 || l == 2 || l == 4 || l == 8 || l == 16 || l == 32; }
 
@@ -369,6 +384,51 @@ int b2m_logp_grad(b2m_model *m, const float *theta, int64_t n_chains, float *log
   if (m->model_class == 1)
     return b2m::glm_logp_grad(m->glm, theta, n_chains, logp, grad, static_cast<cudaStream_t>(stream), true);
   return b2m::launch_logp_grad(m->km, theta, n_chains, logp, grad, lanes, static_cast<cudaStream_t>(stream), m->jit);
+}
+
+int b2m_loglik_stats(b2m_model *m, const float *draws, int64_t n_draws, const int32_t *obs_terms, int32_t n_obs_terms,
+                     double *out, int64_t n_obs, void *stream) {
+  B2M_REQUIRE(m && draws && obs_terms && out, "b2m_loglik_stats: NULL argument");
+  B2M_REQUIRE(n_draws > 0, "b2m_loglik_stats: n_draws must be positive");
+  B2M_REQUIRE(n_obs_terms > 0, "b2m_loglik_stats: no observation terms listed");
+  B2M_REQUIRE(m->model_class == 0 || (m->glm.comm == nullptr && m->glm.pw.nranks == 0),
+              "b2m_loglik_stats: the model is observation-sharded (each rank holds only its rows of the observations)");
+  const int n_terms = (int)m->terms.size();
+  std::vector<int> obs(n_obs_terms);
+  int64_t total = 0;
+  for (int i = 0; i < n_obs_terms; ++i) {
+    const int t = obs_terms[i];
+    if (t < 0 || t >= n_terms) {
+      set_error("b2m_loglik_stats: term index " + std::to_string(t) + " out of range (the model has " +
+                std::to_string(n_terms) + " terms)");
+      return 1;
+    }
+    if (i > 0 && t <= obs[i - 1]) {
+      set_error("b2m_loglik_stats: observation terms must be listed in increasing term order, each once");
+      return 1;
+    }
+    if (!is_observation_term(m->terms[t], m->lin)) {
+      set_error("b2m_loglik_stats: term " + std::to_string(t) + " is not an observation term (its value must be data or a "
+                "constant and one of its distribution parameters must depend on the model parameters)");
+      return 1;
+    }
+    obs[i] = t;
+    total += m->terms[t].length;
+  }
+  if (total != n_obs) {
+    set_error("b2m_loglik_stats: n_obs = " + std::to_string(n_obs) + " but the listed terms have " + std::to_string(total) +
+              " observations");
+    return 1;
+  }
+  int lik = -1;
+  if (m->model_class == 1)
+    for (int t = 0; t < n_terms; ++t) {
+      const b2m_term &T = m->terms[t];
+      if (T.x.kind == B2M_OP_MATVEC || T.p0.kind == B2M_OP_MATVEC || T.p1.kind == B2M_OP_MATVEC) lik = t;
+    }
+  B2M_MODEL_GUARD(m);
+  return b2m::loglik_stats(m->km, m->model_class == 1 ? &m->glm : nullptr, lik, m->terms, obs, draws, n_draws, out, n_obs,
+                           static_cast<cudaStream_t>(stream));
 }
 
 struct b2m_comm {

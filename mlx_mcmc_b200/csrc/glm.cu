@@ -600,13 +600,16 @@ PackP make_pack(const GlmModel &g) {
 constexpr int TM = 64, TN = 64, TK = 16;
 
 // RESID && LOGIT: the Bernoulli-logit epilogue; y = labels, eta0 = c + X beta0 (GlmModel::y0)
-template <bool RESID, bool LOGIT = false>
+// STATS: the log-likelihood statistics epilogue of b2m_loglik_stats (Normal, or Bernoulli-logit with LOGIT): per
+// observation and 32 draw rows, (max, sum exp(ll - max), mean, M2) into part [Cp / 32, ldc]; nothing else is written
+template <bool RESID, bool LOGIT = false, bool STATS = false>
 __global__ void __launch_bounds__(256) simt_gemm_kernel(const float *__restrict__ A, const float *__restrict__ Bm,
                                                         int K, int lda, int ldb, float *__restrict__ Cout, int ldc,
                                                         const float *__restrict__ y, const float *__restrict__ inv_var,
                                                         float *__restrict__ ss_part, int64_t Cp, int N_valid,
                                                         float loc_const, float weight,
-                                                        const float *__restrict__ eta0 = nullptr) {
+                                                        const float *__restrict__ eta0 = nullptr,
+                                                        float4 *__restrict__ part = nullptr, int64_t rows_valid = 0) {
   __shared__ float sA[TK][TM + 4], sB[TK][TN + 4];
   const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
   const int m0 = blockIdx.y * TM, n0 = blockIdx.x * TN;
@@ -629,6 +632,54 @@ __global__ void __launch_bounds__(256) simt_gemm_kernel(const float *__restrict_
         for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
     }
     __syncthreads();
+  }
+  if constexpr (STATS) {
+    // ll per element into a [64 rows][64 columns] tile, then 128 threads reduce one column over 32 rows each, with the
+    // arithmetic of the tensor-core statistics epilogue (glm_tc.cu) in the same order
+    __shared__ float sl[TM][TN + 1];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int m = m0 + ty * 4 + i;
+      const float iv = LOGIT ? 1.0f : inv_var[m];
+      const float lbase = LOGIT ? 0.f : 0.5f * logf(iv) - kHalfLog2Pi;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int n = n0 + tx * 4 + j;
+        float ll;
+        if (LOGIT) {
+          float dt;
+          bernoulli_logit(y[n] != 0.f, eta0[n] + acc[i][j], ll, dt);
+        } else {
+          const float z = ((n < N_valid) ? y[n] : 0.f) - acc[i][j];
+          ll = lbase - 0.5f * (iv * (z * z));
+        }
+        sl[ty * 4 + i][tx * 4 + j] = ll * weight;
+      }
+    }
+    __syncthreads();
+    if (tid < 2 * TN) {
+      const int col = tid % TN, rg = tid / TN, n = n0 + col;
+      const int64_t row0 = m0 + rg * 32, left = rows_valid - row0;
+      const int nv = left >= 32 ? 32 : (left > 0 ? (int)left : 0);
+      if (nv > 0 && n < N_valid) {
+        float mx = -INFINITY, s = 0.f;
+        for (int r = 0; r < nv; ++r) {
+          const float v = sl[rg * 32 + r][col];
+          mx = fmaxf(mx, v);
+          s += v;
+        }
+        const float mean = s / (float)nv;
+        float se = 0.f, m2 = 0.f;
+        for (int r = 0; r < nv; ++r) {
+          const float v = sl[rg * 32 + r][col];
+          se += mx == -INFINITY ? 0.f : expf(v - mx);
+          const float d = v - mean;
+          m2 = fmaf(d, d, m2);
+        }
+        part[(row0 >> 5) * ldc + n] = make_float4(mx, se, mean, m2);
+      }
+    }
+    return;
   }
   if (RESID) {
     // epilogue: z = y - c - M ; R = w z / sigma^2 ; per-row partial sum of z^2 over this column tile
@@ -679,6 +730,19 @@ int simt_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   else
     simt_gemm_kernel<true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, g.R, g.Np, g.y0, g.inv_var, g.ss_part, Cp,
                                                   g.N, 0.f, g.weight);
+  ++g_launches;
+  B2M_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int simt_gemm_stats(GlmModel &g, int64_t Cp, int64_t rows_valid, float4 *part, cudaStream_t st) {
+  dim3 grid(g.Np / TN, (unsigned)(Cp / TM));
+  if (g.lik == kLikLogit)
+    simt_gemm_kernel<false, true, true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, nullptr, g.Np, g.y, g.inv_var,
+                                                              nullptr, Cp, g.N, 0.f, g.weight, g.y0, part, rows_valid);
+  else
+    simt_gemm_kernel<false, false, true><<<grid, 256, 0, st>>>(g.B, g.X, g.Dp, g.Dp, g.Dp, nullptr, g.Np, g.y0, g.inv_var,
+                                                               nullptr, Cp, g.N, 0.f, g.weight, nullptr, part, rows_valid);
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -862,6 +926,43 @@ int glm_logp_grad(GlmModel &g, const float *theta, int64_t C, float *logp, float
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
+}
+
+// ---------------------------------------------------------------- pointwise log-likelihood statistics (b2m_loglik_stats)
+// The centring of the samplers around beta0 = the mean of ALL draws of the call: X (theta_s - beta0) is then of the size
+// of the posterior spread (same accuracy argument as for the samplers).  The next sampler or logp call recentres.
+int glm_loglik_center(GlmModel &g, const float *draws, int64_t S, cudaStream_t st) {
+  dim3 gp(g.Dp / 32, kCenterSlices), bp(32, 8);
+  glm_center_partial_kernel<<<gp, bp, 0, st>>>(draws, S, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
+  glm_center_final_kernel<<<(g.Dp + 127) / 128, 128, 0, st>>>(g.center_part, g.Dp, S, g.beta0);
+  cudaMemsetAsync(g.y0max_bits, 0, sizeof(unsigned), st);
+  glm_y0_kernel<<<(g.Np + 7) / 8, 256, sizeof(float) * g.Dp, st>>>(g.X, g.y, g.beta0, g.N, g.Np, g.Dp, g.loc_const, g.y0,
+                                                                   g.y0max_bits, g.lik == kLikLogit);
+  g_launches += 3;
+  B2M_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// One batch of `rows` draws (model coordinates: no transforms) -> partials of the X @ beta term [Cp / 32, Np].  The
+// batch is packed as the samplers pack a lock-step batch (rows past `rows` are zero rows) and contracted with the
+// statistics epilogue of K5.
+int glm_loglik_batch(GlmModel &g, const float *draws, int64_t rows, float4 *part, cudaStream_t st) {
+  if (int rc = glm_reserve(g, rows)) return rc;
+  const int64_t Cp = rows <= 128 ? 128 : (rows + 255) / 256 * 256;
+  if (g.use_tc == 2) {
+    PackP P = make_pack(g);
+    P.tf = nullptr;                           // the draws are already constrained
+    P.r_scale = nullptr; P.r_unscale = nullptr;   // there is no residual operand
+    glm_pack16_kernel<<<(unsigned)((Cp + 3) / 4), 128, 0, st>>>(P, draws, nullptr, rows, Cp);
+  } else {
+    glm_pack_kernel<<<(unsigned)((Cp * g.Dp + 255) / 256), 256, 0, st>>>(draws, g.beta0, nullptr, rows, Cp, g.Dtot, g.beta_off,
+                                                                          g.D, g.Dp, g.sigma_param, g.sigma_const, g.B,
+                                                                          g.Bh, g.Bl, g.inv_var);
+  }
+  ++g_launches;
+  B2M_CHECK_CUDA(cudaGetLastError());
+  if (g.use_tc) return tc_gemm_stats(g, Cp, rows, part, st);
+  return simt_gemm_stats(g, Cp, rows, part, st);
 }
 
 }  // namespace b2m

@@ -155,6 +155,11 @@ int simt_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);    // R -> G
 int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st);     // B -> R, ss_part
 int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st);      // R -> G
 int tc_gemm_gram(GlmModel &g, int64_t Cp, cudaStream_t st);      // B -> G = (beta - beta0) G~  (Gram form)
+// pointwise log-likelihood statistics over posterior draws (b2m_loglik_stats): B -> partials [Cp / 32, Np] of 32 draws
+int simt_gemm_stats(GlmModel &g, int64_t Cp, int64_t rows_valid, float4 *part, cudaStream_t st);
+int tc_gemm_stats(GlmModel &g, int64_t Cp, int64_t rows_valid, float4 *part, cudaStream_t st);
+int glm_loglik_center(GlmModel &g, const float *draws, int64_t S, cudaStream_t st);   // beta0 = mean draw, y0 / eta0
+int glm_loglik_batch(GlmModel &g, const float *draws, int64_t rows, float4 *part, cudaStream_t st);
 bool tc_available();
 void tc_profile(bool enable);
 int tc_profile_read(double *out4);

@@ -27,6 +27,9 @@
 //                 LOGIT: eta = eta0 + acc, per-row sum of y eta - softplus(eta), R = w (y - sigmoid(eta))
 //                        (K5 of the Bernoulli-logit likelihood, same transposition and stores as RESID)
 //                 PLAIN: store the split-K partial of G                                              (K6)
+//                 STATS: per element the pointwise log-likelihood ll of the Normal or Bernoulli-logit kind, reduced
+//                        over the warp's 32 chain rows per observation into (max, sum exp(ll - max), mean, M2)
+//                        partials (b2m_loglik_stats: K5 over posterior draws instead of chains, no R written)
 #include <cuda.h>
 #include <cuda_fp16.h>
 
@@ -226,6 +229,9 @@ struct EpiParams {
   const float *inv_col_scale;   // [Dp]
   // LOGIT (last, so that the parameter offsets of the other modes stay where they were)
   const float *eta0;      // [Np] c + X beta0 (float64-accumulated centring, padding -inf); `y` holds the labels
+  // STATS: [Cp / 32, Np] partials of 32 draw rows each; rows >= rows_valid of the batch are excluded
+  float4 *part;
+  int64_t rows_valid;
 };
 
 template <int BLOCK_N, int NCTA>
@@ -240,7 +246,8 @@ struct Cfg {
 };
 
 // MODE: 0 = PLAIN (split-K partial of G), 1 = RESID (K5 residual epilogue), 2 = PUSH (K6 tile -> owner's window),
-//       3 = LOGIT (K5 with the Bernoulli-logit residual epilogue)
+//       3 = LOGIT (K5 with the Bernoulli-logit residual epilogue), 4 / 5 = STATS (K5 with the log-likelihood statistics
+//       epilogue, Normal / Bernoulli-logit)
 template <int BLOCK_N, int MODE, int NCTA, bool F16>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
@@ -249,8 +256,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
   if (E.skip_flag && *reinterpret_cast<const volatile int *>(E.skip_flag) >= E.skip_target) return;   // uniform over the grid
   using C = Cfg<BLOCK_N, NCTA>;
   constexpr bool LOGIT = MODE == 3, RESID = MODE == 1 || LOGIT, PUSH = MODE == 2;
+  constexpr bool STATS = MODE == 4 || MODE == 5, STATS_LOGIT = MODE == 5;
+  constexpr bool K5 = RESID || STATS;          // the B X^T tile order
   constexpr int BLOCK_K = Enc<F16>::BLOCK_K;   // K elements per k-block (shadows the tf32 constant)
-  constexpr int SCRATCH_BYTES = (RESID || PUSH) ? NUM_EPI_WARPS * 32 * 33 * 4 : 0;   // per-warp transpose scratch of the epilogue
+  constexpr int SCRATCH_BYTES = (RESID || PUSH || STATS) ? NUM_EPI_WARPS * 32 * 33 * 4 : 0;   // per-warp transpose scratch of the epilogue
   extern __shared__ unsigned char smem_raw[];
   unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   float *scratch_base = reinterpret_cast<float *>(smem + C::STAGES * C::STAGE_BYTES);
@@ -272,8 +281,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
   // are set up once; the producer and the MMA issuer run ahead into the next tile while the promotion warps are
   // still in the epilogue of the previous one (both TMEM chunk buffers are free by then).
 #define B2M_DECODE_TILE(t)                                                         \
-  const int mp_ = RESID ? (t) % Tm : ((t) / Tn) % Tm;                              \
-  const int nt = RESID ? ((t) / Tm) % Tn : (t) % Tn;                               \
+  const int mp_ = K5 ? (t) % Tm : ((t) / Tn) % Tm;                                 \
+  const int nt = K5 ? ((t) / Tm) % Tn : (t) % Tn;                                  \
   const int zs = (t) / (Tm * Tn);                                                  \
   const int m0 = (mp_ * NCTA + (int)cta) * BLOCK_M, n0 = nt * BLOCK_N;             \
   const int kb0 = zs * k_blocks_per_split;                                         \
@@ -490,6 +499,66 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__
         __syncwarp();
       }
       E.ss_part[((int64_t)nt * 2 + half) * E.Cp + m] = ss;
+    } else if (STATS) {
+      // Statistics epilogue.  The thread that owns row m (a draw) computes ll for its CW columns and transposes each
+      // 32 x 32 block through the warp's scratch, as the residual epilogue does; afterwards lane l owns observation
+      // nb + 32 b + l over the warp's 32 rows and reduces that column: max and sum exp(ll - max), then the mean and, in
+      // a second pass, M2 = sum (ll - mean)^2 (fp32 sum ll^2 - (sum ll)^2 / n cancels where the variance is small).
+      const float a_un = F16 ? E.a_unscale[m] : 1.0f;
+      const float iv = STATS_LOGIT ? 1.0f : E.inv_var[m];
+      const float lbase = STATS_LOGIT ? 0.f : 0.5f * logf(iv) - kHalfLog2Pi;
+      float *scratch = scratch_base + (warp - 2) * (32 * 33);
+      const int64_t row0 = (int64_t)(m0 + q * 32);
+      const int64_t left = E.rows_valid - row0;
+      const int nv = left >= 32 ? 32 : (left > 0 ? (int)left : 0);   // draw rows of this warp that count (uniform)
+      float yv[CW / 32], ev[STATS_LOGIT ? CW / 32 : 1];
+#pragma unroll
+      for (int b = 0; b < CW / 32; ++b) {
+        const int n = nb + b * 32 + lane;
+        if (STATS_LOGIT) {
+          yv[b] = __ldg(E.y + n);
+          ev[b] = __ldg(E.eta0 + n);
+        } else {
+          yv[b] = (n < E.N_valid) ? __ldg(E.y + n) : 0.f;
+        }
+      }
+#pragma unroll
+      for (int b = 0; b < CW / 32; ++b) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          const float yj = __shfl_sync(0xffffffffu, yv[b], j);
+          const float xd = F16 ? acc[b * 32 + j] * a_un : acc[b * 32 + j];
+          float ll;
+          if (STATS_LOGIT) {
+            float dt;
+            bernoulli_logit(yj != 0.f, __shfl_sync(0xffffffffu, ev[b], j) + xd, ll, dt);
+          } else {
+            const float z = yj - xd;
+            ll = lbase - 0.5f * (iv * (z * z));
+          }
+          scratch[lane * 33 + j] = ll * E.weight;
+        }
+        __syncwarp();
+        const int n = nb + b * 32 + lane;
+        if (nv > 0 && n < E.N_valid) {
+          float mx = -INFINITY, s = 0.f;
+          for (int r = 0; r < nv; ++r) {
+            const float v = scratch[r * 33 + lane];
+            mx = fmaxf(mx, v);
+            s += v;
+          }
+          const float mean = s / (float)nv;
+          float se = 0.f, m2 = 0.f;
+          for (int r = 0; r < nv; ++r) {
+            const float v = scratch[r * 33 + lane];
+            se += mx == -INFINITY ? 0.f : expf(v - mx);
+            const float d = v - mean;
+            m2 = fmaf(d, d, m2);
+          }
+          E.part[(row0 >> 5) * E.Np + n] = make_float4(mx, se, mean, m2);
+        }
+        __syncwarp();
+      }
     } else if (PUSH) {
       // The tile's 128 rows belong to one owner rank (own % 128 == 0).  Each warp transposes its 32 x 32 blocks through
       // the shared-memory scratch so that every store instruction writes one 128-byte row segment into the owner's
@@ -613,7 +682,7 @@ int launch_tc_n(const CUtensorMap &Ah, const CUtensorMap &Al, const CUtensorMap 
                 int kb_total, int kb_per_split, const EpiParams &E, cudaStream_t st, int chunk_kb, int mma_mask,
                 int prof_kind) {
   using C = Cfg<BLOCK_N, NCTA>;
-  constexpr bool RESID = MODE == 1 || MODE == 3;
+  constexpr bool RESID = MODE == 1 || MODE == 3 || MODE == 4 || MODE == 5;
   auto kernel = tc_gemm_kernel<BLOCK_N, MODE, NCTA, F16>;
   constexpr int SMEM = C::SMEM_BYTES + (MODE != 0 ? NUM_EPI_WARPS * 32 * 33 * 4 : 0);
   // per device: the attribute belongs to the function on the current device.  Setting it again is harmless, so a plain
@@ -784,6 +853,32 @@ int tc_gemm_resid(GlmModel &g, int64_t Cp, cudaStream_t st) {
   const int ck = (f16 && g.Dp / bk >= 8) ? 8 : DEFAULT_CHUNK_KB;
   if (logit) return launch_tc<256, 3>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
   return launch_tc<256, 1>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
+}
+
+// K5 over a batch of posterior draws with the statistics epilogue: the operand set-up and tile schedule of
+// tc_gemm_resid, no residual operand, per-observation partials of 32 draws into `part` [Cp / 32, Np].  Timed in the
+// K5 slot of the profile.
+int tc_gemm_stats(GlmModel &g, int64_t Cp, int64_t rows_valid, float4 *part, cudaStream_t st) {
+  const int ncta = pair_mode(Cp);
+  const bool f16 = g.use_tc == 2;
+  const int bk = f16 ? 64 : 32;
+  const void *A_h = f16 ? (const void *)g.B16h : (const void *)g.Bh, *A_l = f16 ? (const void *)g.B16l : (const void *)g.Bl;
+  const void *B_h = f16 ? (const void *)g.X16h : (const void *)g.Xh, *B_l = f16 ? (const void *)g.X16l : (const void *)g.Xl;
+  CUtensorMap Ah, Al, Bh, Bl;
+  if (make_map(&Ah, A_h, Cp, g.Dp, BLOCK_M, f16) || make_map(&Al, A_l, Cp, g.Dp, BLOCK_M, f16) ||
+      make_map(&Bh, B_h, g.Np, g.Dp, 256 / ncta, f16) || make_map(&Bl, B_l, g.Np, g.Dp, 256 / ncta, f16))
+    return 2;
+  EpiParams E{};
+  E.y = g.y0; E.inv_var = g.inv_var; E.Cp = Cp; E.Np = g.Np;
+  E.a_unscale = g.a_unscale;
+  E.N_valid = g.N; E.weight = g.weight;
+  E.part = part; E.rows_valid = rows_valid;
+  const bool logit = g.lik == kLikLogit;
+  if (logit) { E.y = g.y; E.eta0 = g.y0; }
+  dim3 grid((unsigned)(Cp / BLOCK_M), g.Np / 256, 1);
+  const int ck = (f16 && g.Dp / bk >= 8) ? 8 : DEFAULT_CHUNK_KB;   // as tc_gemm_resid
+  if (logit) return launch_tc<256, 5>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
+  return launch_tc<256, 4>(ncta, Ah, Al, Bh, Bl, grid, g.Dp / bk, g.Dp / bk, E, st, ck, 7, f16);
 }
 
 int tc_gemm_grad(GlmModel &g, int64_t Cp, cudaStream_t st) {

@@ -140,3 +140,63 @@ def device_quantiles(x, q):
         _cabi.check(lib.b2m_quantiles(C.c_void_p(x.data_ptr()), x.numel(), qa, len(q), out,
                                       C.c_void_p(torch.cuda.current_stream().cuda_stream)))
     return [float(v) for v in out]
+
+
+# ------------------------------------------------------------------------------------------ model comparison (WAIC)
+def waic_totals(lppd, mean, var, n_draws: int) -> dict:
+    """WAIC from the per-observation statistics of the pointwise log-likelihood ll[s, n] over S draws (Vehtari, Gelman &
+    Gabry 2017): lppd_n = log mean_s exp ll[s, n], mean_n = mean_s ll[s, n], var_n = sample variance (ddof 1).
+        elpd_waic = sum_n (lppd_n - var_n),  p_waic = sum_n var_n,  waic = -2 elpd_waic,
+        se = sqrt(N Var_n(lppd_n - var_n)),  n_warn = #{n : var_n > 0.4}
+    plus ``pointwise`` = {lppd, p_waic, elpd} as [N] float64 arrays (what ``waic_compare`` needs)."""
+    lppd = np.asarray(lppd, dtype=np.float64)
+    mean = np.asarray(mean, dtype=np.float64)
+    var = np.asarray(var, dtype=np.float64)
+    elpd_i = lppd - var
+    n = elpd_i.size
+    elpd = float(np.sum(elpd_i))
+    return {"elpd_waic": elpd, "p_waic": float(np.sum(var)), "waic": -2.0 * elpd,
+            "se": float(np.sqrt(n * np.var(elpd_i))) if n > 0 else 0.0, "lppd": float(np.sum(lppd)),
+            "n_warn": int(np.sum(var > 0.4)), "n_obs": int(n), "n_draws": int(n_draws),
+            "pointwise": {"lppd": lppd, "p_waic": var, "elpd": elpd_i, "mean": mean}}
+
+
+def waic(model, draws) -> dict:
+    """WAIC of `model` (an ``engine.DeviceModel``) over the posterior `draws` [S, C, D] (float32 CUDA tensor in model
+    coordinates, as the samplers write them).  The pointwise log-likelihood of every draw and every observation of the
+    model's observation terms (``TracedModel.observation_terms``) is reduced on the device (b2m_loglik_stats: for the
+    GLM class inside the B X^T contraction); only [N, 3] float64 statistics reach the host.  Returns ``waic_totals``."""
+    import torch
+    from . import _cabi
+    if not (hasattr(draws, "is_cuda") and draws.is_cuda and draws.dtype == torch.float32 and draws.dim() == 3):
+        raise ValueError("waic expects a float32 CUDA tensor of shape [S, C, D]")
+    if draws.shape[2] != model.D:
+        raise ValueError(f"waic: draws have D = {draws.shape[2]}, the model has {model.D} parameters")
+    obs = model.traced.observation_terms()
+    if not obs:
+        raise ValueError("waic: the model has no observation terms (no term's value is data while one of its "
+                         "distribution parameters depends on the model parameters)")
+    if getattr(model, "_comm", None) is not None or getattr(model, "_peer", None) is not None:
+        raise ValueError("waic: observation-sharded models are not supported (each rank holds only its rows)")
+    draws = draws.contiguous()
+    if not bool(torch.isfinite(draws).all()):
+        raise ValueError("waic: the draws contain non-finite values")
+    S = draws.shape[0] * draws.shape[1]
+    n_obs = sum(model.traced.terms[i].length for i in obs)
+    out = torch.empty((n_obs, 3), dtype=torch.float64, device=draws.device)
+    idx = (C.c_int32 * len(obs))(*obs)
+    with torch.cuda.device(draws.device):
+        _cabi.check(model.lib.b2m_loglik_stats(model.handle, C.c_void_p(draws.data_ptr()), S, idx, len(obs),
+                                               C.c_void_p(out.data_ptr()), n_obs,
+                                               C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    h = out.cpu().numpy()
+    return waic_totals(h[:, 0], h[:, 1], h[:, 2], S)
+
+
+def waic_compare(a: dict, b: dict) -> dict:
+    """Difference of two ``waic`` results on the same observations: elpd_diff = elpd_a - elpd_b and its standard error
+    sqrt(N Var_n(elpd_a,n - elpd_b,n)) from the pointwise arrays.  Positive elpd_diff favours `a`."""
+    if a["n_obs"] != b["n_obs"]:
+        raise ValueError(f"waic_compare: the results cover different observations ({a['n_obs']} vs {b['n_obs']})")
+    d = np.asarray(a["pointwise"]["elpd"], dtype=np.float64) - np.asarray(b["pointwise"]["elpd"], dtype=np.float64)
+    return {"elpd_diff": float(np.sum(d)), "se_diff": float(np.sqrt(d.size * np.var(d)))}

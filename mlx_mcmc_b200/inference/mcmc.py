@@ -26,6 +26,7 @@ class MCMC:
         self.acceptance_rate = None
         self.info = None
         self._single_chain = True
+        self._waic_source = None
 
     def run(self, initial_params, num_samples=1000, num_warmup=1000, method='metropolis', proposal_scale=0.1,
             random_seed=0, verbose=True, **kwargs):
@@ -64,6 +65,9 @@ class MCMC:
                 peer = total if kwargs.get("slice_state") in (True, "peer") else None
                 kwargs["model"] = D_.compile_obs_sharded(self.log_prob_fn, initial_params, peer_chains=peer)
         self._single_chain = int(kwargs.get("num_chains", 1)) == 1 and gather is None
+        # what waic() needs to find the same device model again (compile_model's cache) after the run
+        self._waic_source = dict(initial_params=initial_params, shard=shard, model=kwargs.get("model"),
+                                 transforms=kwargs.get("transforms"), cache=kwargs.get("cache", True))
         out = self._run_local(initial_params, num_samples, num_warmup, method, proposal_scale, random_seed, verbose, kwargs)
         if gather is not None:
             D_, count = gather
@@ -165,6 +169,31 @@ class MCMC:
             cols = device_summary(d, None, ess)
             table[name] = {k: (float(v[0]) if x.dim() == 2 else v.copy()) for k, v in cols.items()}
         return table
+
+    def waic(self):
+        """WAIC of the model over the draws of the last ``run`` (numpy or ``return_torch=True``, any number of chains),
+        from the pointwise log-likelihood of every observation of the model's observation terms, reduced on the device
+        (``diagnostics.waic``).  Not in the reference.  Runs with ``shard='obs'`` are refused: each rank holds only its
+        rows of the observations."""
+        import torch
+        from ..diagnostics import waic
+        from ..engine import DeviceModel, compile_model
+        if self.samples is None or self._waic_source is None:
+            raise ValueError("Must run sampling first. Call run() method.")
+        src = self._waic_source
+        if src["shard"] == "obs":
+            raise ValueError("waic() is not supported for observation-sharded runs (shard='obs')")
+        model = src["model"] if isinstance(src["model"], DeviceModel) else compile_model(
+            self.log_prob_fn, src["initial_params"], cache=src["cache"], transforms=src["transforms"])
+        # the inverse of DeviceModel.unpack: {name: (S,) | (S, n) | (C, S) | (C, S, n)} -> [S, C, D] in model coordinates
+        parts = []
+        for name, (off, n, shp) in model.layout.items():
+            x = torch.as_tensor(self.samples[name]).to(device=model.device, dtype=torch.float32)
+            if self._single_chain:
+                x = x[None]
+            parts.append(x.reshape(x.shape[0], x.shape[1], n))
+        draws = torch.cat(parts, dim=2).permute(1, 0, 2).contiguous()
+        return waic(model, draws)
 
     def print_summary(self, credible_interval=0.95):
         table = self.summary(credible_interval)

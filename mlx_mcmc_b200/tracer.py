@@ -532,6 +532,21 @@ class TracedModel:
         codes[clash] = 0
         return codes
 
+    @staticmethod
+    def _involves_param(o: Operand) -> bool:
+        if o.kind in (OP_PARAM, OP_PARAMVEC, OP_MATVEC):
+            return True
+        return o.kind == OP_LIN and any(p >= 0 for p, _, _ in o.lin)
+
+    def observation_terms(self) -> List[int]:
+        """Indices of the observation terms, in term order: the value operand involves no parameter (a constant, data,
+        or an affine expression of data) and p0 or p1 does.  Every element of such a term is one observation, numbered
+        in term order and by element within a term -- the columns of the pointwise log-likelihood that WAIC is
+        computed from (diagnostics.waic, b2m_loglik_stats, which checks this choice).  Constant terms never count."""
+        return [i for i, t in enumerate(self.terms)
+                if t.dist != CONSTANT and not self._involves_param(t.x)
+                and (self._involves_param(t.p0) or self._involves_param(t.p1))]
+
     def describe(self) -> str:
         rows = []
         for t in self.terms:
