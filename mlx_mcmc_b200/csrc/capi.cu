@@ -161,6 +161,8 @@ static int setup_glm(b2m_model *m, int D, int glm_path, int glm_form, const int3
   for (size_t t = 0; t < m->terms.size(); ++t)
     if ((int)t != lik) prior.push_back(m->terms[t]);
   g.has_prior = !prior.empty();
+  for (const b2m_term &T : prior)
+    g.prior_lin = g.prior_lin || T.x.kind == B2M_OP_LIN || T.p0.kind == B2M_OP_LIN || T.p1.kind == B2M_OP_LIN;
   g.prior = m->km;
   g.prior.n_terms = (int)prior.size();
   g.prior.max_len = 1;

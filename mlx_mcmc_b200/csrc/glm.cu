@@ -415,8 +415,12 @@ int glm_build(GlmModel &g, const float *X, const float *y, int N, int D, bool fo
 // beta0 = the mean of the chains' current positions.  X (beta_c - beta0) is then of the size of the
 // posterior spread, and its rounding no longer dominates z.  Same function, different association.
 
-__global__ void __launch_bounds__(256) glm_center_partial_kernel(const float *__restrict__ theta, int64_t C, int Dtot,
-                                                                 int beta_off, int D, int Dp, double *__restrict__ part) {
+// `tf` (sampler coordinates, nullptr otherwise): the centre is the mean of the constrained coefficients T(theta)_beta,
+// the values that pack subtracts beta0 from -- so that delta stays of the size of the posterior spread when beta itself
+// is transformed, and the samplers' centring agrees with that of the draws (glm_loglik_center).
+__global__ void __launch_bounds__(256) glm_center_partial_kernel(const float *__restrict__ theta, const int *__restrict__ tf,
+                                                                 int64_t C, int Dtot, int beta_off, int D, int Dp,
+                                                                 double *__restrict__ part) {
   __shared__ double sh[8][33];
   const int d = blockIdx.x * 32 + threadIdx.x, ty = threadIdx.y;
   const int64_t per = (C + kCenterSlices - 1) / kCenterSlices;
@@ -424,7 +428,8 @@ __global__ void __launch_bounds__(256) glm_center_partial_kernel(const float *__
   double acc = 0.0;
   if (d < D)
     for (int64_t c = c0 + ty; c < c1; c += 8) {
-      const float v = theta[c * Dtot + beta_off + d];
+      float v = theta[c * Dtot + beta_off + d];
+      if (tf) v = tf_constrain(tf[beta_off + d], v);
       if (fabsf(v) <= 3.0e38f) acc += (double)v;   // a diverged / NaN chain must not move the centre
     }
   sh[ty][threadIdx.x] = acc;
@@ -519,7 +524,7 @@ __global__ void __launch_bounds__(256) gram_q_kernel(const double *__restrict__ 
 
 int glm_recenter(GlmModel &g, const float *theta, int64_t C, cudaStream_t st) {
   dim3 gp(g.Dp / 32, kCenterSlices), bp(32, 8);
-  glm_center_partial_kernel<<<gp, bp, 0, st>>>(theta, C, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
+  glm_center_partial_kernel<<<gp, bp, 0, st>>>(theta, g.tf, C, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
   glm_center_final_kernel<<<(g.Dp + 127) / 128, 128, 0, st>>>(g.center_part, g.Dp, C, g.beta0);
   if (g.form == kFormGram) {
     gram_center_kernel<<<(g.Dp + 7) / 8, 256, 0, st>>>(g.G64, g.gvec, g.beta0, g.Dp, g.loc_const, g.gb, g.gterm);
@@ -813,6 +818,7 @@ int glm_set_comm(GlmModel &g, Comm *c, cudaStream_t st) {
 
 // ---------------------------------------------------------------- finish: assemble log p and the full gradient
 // One warp per chain (body: finish_row, glm_rows.cuh).  Rows [row_base, row_end) of the batch.
+template <bool LIN>
 __global__ void __launch_bounds__(128) glm_finish_kernel(KModel prior, FinishP F, const float *__restrict__ theta,
                                                           int64_t row_base, int64_t row_end, float *__restrict__ logp,
                                                           float *__restrict__ grad, const int *__restrict__ idx) {
@@ -824,7 +830,7 @@ __global__ void __launch_bounds__(128) glm_finish_kernel(KModel prior, FinishP F
   const int64_t c = row_base + (int64_t)blockIdx.x * (blockDim.x / 32) + warp;
   if (c >= row_end) return;
   const int64_t src = idx ? idx[c] : c;       // chain served by row c of a compacted batch
-  finish_row(F, sm, theta + src * F.Dtot, c, c, logp + src, grad ? grad + src * F.Dtot : nullptr, lane);
+  finish_row<LIN>(F, sm, theta + src * F.Dtot, c, c, logp + src, grad ? grad + src * F.Dtot : nullptr, lane);
 }
 
 FinishP make_finish(const GlmModel &g, int64_t Cp, bool with_grad) {
@@ -858,7 +864,8 @@ int glm_finish_launch(GlmModel &g, const float *theta, int64_t C, float *logp, f
   if (idx) C = n_rows;
   const int64_t Cp = C <= 128 ? 128 : (C + 255) / 256 * 256;
   const FinishP F = make_finish(g, Cp, grad != nullptr);
-  glm_finish_kernel<<<(unsigned)((C + 3) / 4), 128, finish_smem(g), st>>>(g.prior, F, theta, 0, C, logp, grad, idx);
+  (g.prior_lin ? glm_finish_kernel<true> : glm_finish_kernel<false>)<<<(unsigned)((C + 3) / 4), 128, finish_smem(g), st>>>(
+      g.prior, F, theta, 0, C, logp, grad, idx);
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -921,8 +928,8 @@ int glm_logp_grad(GlmModel &g, const float *theta, int64_t C, float *logp, float
   }
   const int64_t row_base = (g.comm && own_count > 0) ? own_base : 0;
   const int64_t rows = (g.comm && own_count > 0) ? own_count : C;
-  glm_finish_kernel<<<(unsigned)((rows + 3) / 4), 128, finish_smem(g), st>>>(g.prior, F, theta, row_base, row_base + rows,
-                                                                            logp, grad, idx);
+  (g.prior_lin ? glm_finish_kernel<true> : glm_finish_kernel<false>)<<<(unsigned)((rows + 3) / 4), 128, finish_smem(g), st>>>(
+      g.prior, F, theta, row_base, row_base + rows, logp, grad, idx);
   ++g_launches;
   B2M_CHECK_CUDA(cudaGetLastError());
   return 0;
@@ -933,7 +940,7 @@ int glm_logp_grad(GlmModel &g, const float *theta, int64_t C, float *logp, float
 // of the posterior spread (same accuracy argument as for the samplers).  The next sampler or logp call recentres.
 int glm_loglik_center(GlmModel &g, const float *draws, int64_t S, cudaStream_t st) {
   dim3 gp(g.Dp / 32, kCenterSlices), bp(32, 8);
-  glm_center_partial_kernel<<<gp, bp, 0, st>>>(draws, S, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
+  glm_center_partial_kernel<<<gp, bp, 0, st>>>(draws, nullptr, S, g.Dtot, g.beta_off, g.D, g.Dp, g.center_part);
   glm_center_final_kernel<<<(g.Dp + 127) / 128, 128, 0, st>>>(g.center_part, g.Dp, S, g.beta0);
   cudaMemsetAsync(g.y0max_bits, 0, sizeof(unsigned), st);
   glm_y0_kernel<<<(g.Np + 7) / 8, 256, sizeof(float) * g.Dp, st>>>(g.X, g.y, g.beta0, g.N, g.Np, g.Dp, g.loc_const, g.y0,

@@ -98,6 +98,7 @@ struct GlmModel {
   // prior terms (everything except the matvec likelihood) as a pointwise term table
   KModel prior{};
   bool has_prior = false;
+  bool prior_lin = false;   // some prior operand is affine (B2M_OP_LIN): glm_finish_kernel<true> differentiates it
   // workspace sized for `cap` chains (padded to 128)
   int64_t cap = 0;
   float *B = nullptr, *Bh = nullptr, *Bl = nullptr;          // [cap, Dp]

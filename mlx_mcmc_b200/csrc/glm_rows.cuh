@@ -176,10 +176,39 @@ __device__ __forceinline__ float gram_row(const FinishP &F, const float *__restr
   return (float)(F.gb[Dp] + acc);
 }
 
+// Gradient of the affine operands (B2M_OP_LIN) of prior term T, added into gr (constrained coordinates): for every
+// entry coef (* data_n) theta_p of an affine slot, w sum_n df/dslot_n coef (data_n).  The entries of one slot share
+// parameters with other lanes' elements, so each entry is one warp sum in a fixed order (lane-strided partial sums,
+// xor tree, lane 0 adds): deterministic, no atomics.  The element partials are recomputed per entry -- priors are
+// short -- and the helper stays out of line, off the register budget and instruction footprint of the inlined finish.
+static __device__ __noinline__ void lin_prior_grad(const b2m_term &T, const SModel &sm, const float *__restrict__ th,
+                                                   float *__restrict__ gr, int lane) {
+  for (int slot = 0; slot < 3; ++slot) {
+    const b2m_operand &o = slot == 0 ? T.x : (slot == 1 ? T.p0 : T.p1);
+    if (o.kind != B2M_OP_LIN) continue;
+    for (int e = o.a; e < o.a + o.b; ++e) {
+      const b2m_lin_entry le = sm.lin[e];
+      if (le.param < 0) continue;
+      float acc = 0.f;
+      for (int n = lane; n < T.length; n += 32) {
+        const float x = op_fetch(T.x, n, th, 1, sm), p0 = op_fetch(T.p0, n, th, 1, sm), p1 = op_fetch(T.p1, n, th, 1, sm);
+        const Elem el = dist_eval<true>(T.dist, x, p0, p1, T.k0, T.k1, T.k2);
+        const float t = le.array >= 0 ? le.coef * sm.arrays[le.array].ptr[n] : le.coef;
+        acc += (slot == 0 ? el.dx : (slot == 1 ? el.d0 : el.d1)) * t;
+      }
+      for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+      if (lane == 0) gr[le.param] += T.weight * acc;
+      __syncwarp();
+    }
+  }
+}
+
 // Assemble log p and the full gradient of one chain from the contraction outputs.  `c` = row of ss_part / G (and of
 // thc); `th` = the chain's parameter row as the samplers hold it (unconstrained when tf is set); logp / gr = outputs.
 // Likelihood value from the partial sums (fixed summation order => deterministic), gradient of beta from G, gradient
-// of sigma analytically, then the prior terms (generic densities) added on top.
+// of sigma analytically, then the prior terms (generic densities) added on top.  LIN = false: the caller knows that no
+// prior operand is affine (GlmModel::prior_lin) and gets the finish without the out-of-line call and its register cost.
+template <bool LIN = true>
 __device__ __forceinline__ void finish_row(const FinishP &F, const SModel &sm, const float *__restrict__ th, int64_t c,
                                            int64_t c_batch, float *__restrict__ logp_out, float *__restrict__ gr, int lane) {
   B2M_ASSERT(c >= 0 && c < F.Cp && F.g_splits >= 0 && F.n_tiles >= 1);
@@ -305,6 +334,8 @@ __device__ __forceinline__ void finish_row(const FinishP &F, const SModel &sm, c
       if (T.p1.kind == B2M_OP_PARAM) gr[T.p1.a] += T.weight * a1;
     }
     __syncwarp();
+    if (LIN && gr && (T.x.kind == B2M_OP_LIN || T.p0.kind == B2M_OP_LIN || T.p1.kind == B2M_OP_LIN))
+      lin_prior_grad(T, sm, th, gr, lane);
   }
   float lj = 0.f;
   if (F.tf) {   // chain rule through theta = T(u) and the log-Jacobian

@@ -938,6 +938,7 @@ __device__ __forceinline__ void spin_until(const unsigned long long *flag, unsig
   }
 }
 
+template <bool LIN>
 __global__ void __launch_bounds__(32 * WPB, 7) nuts_state_kernel(b2m_nuts_args A, NutsBufs W, int D, KModel prior, StateP S) {
   extern __shared__ __align__(16) unsigned char smem[];
   SModel sm;
@@ -954,7 +955,7 @@ __global__ void __launch_bounds__(32 * WPB, 7) nuts_state_kernel(b2m_nuts_args A
     const int64_t c = S.idx ? S.idx[row] : row;
     B2M_ASSERT(c >= 0 && c < A.n_chains && row >= 0 && (S.peer || row < S.n_pad));
     if (S.do_finish) {
-      finish_row(S.F, sm, W.fq + c * D, S.peer ? r : row, row, W.flp + c, W.fg + c * D, lane);
+      finish_row<LIN>(S.F, sm, W.fq + c * D, S.peer ? r : row, row, W.flp + c, W.fg + c * D, lane);
       __syncwarp();
     }
     if (S.do_tick_pack) {
@@ -1395,7 +1396,7 @@ int glm_nuts_run_fused(GlmModel &gm, const b2m_nuts_args &a, cudaStream_t st) {
   auto launch_state = [&](const StateP &S) {
     const unsigned grid = (unsigned)((S.n_pad + WPB - 1) / WPB);
     prof_mark(2, st);
-    nuts_state_kernel<<<grid, T, finish_smem(gm), st>>>(a, W, D, gm.prior, S);
+    (gm.prior_lin ? nuts_state_kernel<true> : nuts_state_kernel<false>)<<<grid, T, finish_smem(gm), st>>>(a, W, D, gm.prior, S);
     prof_mark(2, st);
     ++g_launches;
   };
